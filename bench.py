@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Throughput benchmark of the ray-marching hot path (contract: see the task brief / DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], "C2"): Part 2 Instant-NeRF -- 16-level hash grid (T = 2^19,
@@ -15,6 +15,18 @@ resident in HBM; ``e2e`` = the same step fed from pinned HOST buffers (H2D of th
 the loss inside the timed region).  ``--impl reference`` times the reference's CPU implementation
 of the same step (the oracle port; the real reference + tcnn shim if /root/reference is present)
 on a bounded ray sample.
+
+``--dump-outputs DIR`` (rank 0): after the timed headline steps, what the last of them computed --
+rendered color / depth / acc, the loss, and every parameter and its (clipped) gradient after the
+optimizer step -- as DIR/<name>.npy in float32.  An array of more than 2^20 elements (the 13 M-entry
+hash table and its gradient) is stored as a fixed seeded sample of 2^20 of its elements, so a dump
+stays under 64 MB.  Seeds fix every input, so two builds run with the same arguments can be
+compared output for output.  The hash-table gradient is summed with atomics and AdamW magnifies
+near-zero gradients, so two runs of ONE build already differ.  Two runs of
+``python bench.py --no-extras --no-cpu-baseline --dump-outputs DIR`` (the default 20 steps after 3
+warm-up steps) on a B200 at its 1000 W power limit differed by relative L2 (||a - b|| / ||b|| per
+file) 4e-3 in the hash table, 7e-4 in its gradient, 4e-4 in the decoder weights and 7e-5 in
+color / depth / acc.
 """
 import argparse
 import json
@@ -53,7 +65,14 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip the sparse-occupancy and render legs")
     ap.add_argument("--only", default=None, help="run only one extra leg (c1_vanilla, c3_dnerf, c4_instant_dnerf, "
                                                  "c5_dualhash) and print its dict -- development aid")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed headline step computed to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b2n" or args.only):
+        ap.error("--dump-outputs applies to the headline step of --impl b2n")
+    return args
 
 
 # --------------------------------------------------------------------------------------- CPU arm
@@ -134,8 +153,7 @@ def cpu_train_rays_per_s(n_rays, steps, warmup, occupancy):
 def run_reference_arm(args, rank, world):
     if rank != 0:
         return
-    # bounded sample: one 2^14-ray step is ~10 s of CPU work on 16 cores
-    steps, warm = max(1, min(args.steps, 5)), max(0, min(args.warmup, 1))
+    steps, warm = args.steps, args.warmup
     r = cpu_train_rays_per_s(args.cpu_rays, steps, warm, args.occupancy)
     line = {
         "impl": "reference", "metric": "train_rays_per_s", "value": r["value"], "unit": "rays/s",
@@ -150,6 +168,22 @@ def run_reference_arm(args, rank, world):
 
 
 # --------------------------------------------------------------------------------------- helpers
+DUMP_MAX_ELEMENTS = 2 ** 20        # per array: C2 dumps 10 arrays, so a dump is at most 40 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """``arrays`` (name -> tensor) as out_dir/<name>.npy in float32.  A tensor of more than DUMP_MAX_ELEMENTS elements is
+    flattened and sampled at the same seeded positions in every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMENTS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def workload_config(args, rays):
     return {
         "workload": "C2 Part-2 Instant-NeRF training step: hash grid L=16 F=2 T=2^19 + 64-wide sigma/color MLPs "
@@ -235,7 +269,7 @@ def _maybe_profile(step):
                                     max_name_column_width=70), file=sys.stderr)
 
 
-def bench_c1(dev):
+def bench_c1(dev, steps):
     """BASELINE.json configs[0] ("C1", Part 2 vanilla NeRF: PosEnc 10/4, 8x256 MLP on tcgen05, 64 samples, batch
     4096) on one GPU -- reported as an extra, the headline stays C2."""
     from b2n import synthetic
@@ -271,7 +305,7 @@ def bench_c1(dev):
         torch.cuda.synchronize()
         return e0.elapsed_time(e1) / n
 
-    ms_train = run(step, 20, 5)
+    ms_train = run(step, steps, 5)
     _maybe_profile(step)
     # the same step captured into ONE CUDA graph (b2n.graphs): no occupancy grid -> every shape is static.  A fresh model
     # and a capturable Adam; per step the new ray batch is copied into the graph's static input buffers.
@@ -292,7 +326,7 @@ def bench_c1(dev):
             return loss
 
         graphed = b2n.graphs.GraphedStep(gstep, pool[0])
-        ms_graph = run(lambda i: graphed(*pool[i % 3]), 20, 5)
+        ms_graph = run(lambda i: graphed(*pool[i % 3]), steps, 5)
         graph = {"train_rays_per_s_cuda_graph": B / ms_graph * 1e3, "train_ms_per_step_cuda_graph": ms_graph,
                  "cuda_graph_note": "whole step (march .. fused Adam) replayed as one graph launch",
                  "loss_after_graph_steps": float(graphed(*pool[0]).detach())}
@@ -300,7 +334,7 @@ def bench_c1(dev):
         graph = {"cuda_graph_error": f"{type(exc).__name__}: {exc}"[:300]}
     model.eval()
     with torch.no_grad():
-        ms_render = run(lambda i: render_rays(model, pool[i % 3][0], pool[i % 3][1], NEAR, FAR, N, False), 20, 5)
+        ms_render = run(lambda i: render_rays(model, pool[i % 3][0], pool[i % 3][1], NEAR, FAR, N, False), steps, 5)
     return {"workload": "C1 Part-2 vanilla NeRF, B=4096 rays x 64 samples, 8x256 MLP (tcgen05 bf16), Adam (b2n.optim.FusedAdamW, weight_decay 0)",
             "train_rays_per_s": B / ms_train * 1e3, "train_ms_per_step": ms_train,
             "train_mlp_tflops_algorithmic": 3 * 2.0 * B * N * 593408 / ms_train / 1e9,
@@ -331,7 +365,7 @@ DYNAMIC = {
 }
 
 
-def bench_dynamic(dev, name, steps=10, warm=4, occupancy="dense", world=1, rank=0, strong=False):
+def bench_dynamic(dev, name, steps, warm=4, occupancy="dense", world=1, rank=0, strong=False):
     """Training step of run.py:1073-1178 / :1804-1949 (autocast + GradScaler, render_rays with times, RGB MSE +
     deformation L2 + table TV, clip, AdamW) for the dynamic configs -- reported as extras.
 
@@ -449,7 +483,7 @@ def bench_dynamic(dev, name, steps=10, warm=4, occupancy="dense", world=1, rank=
         out["fused_optimizer_error"] = f"{type(exc).__name__}: {exc}"[:300]
     if reducer is not None:
         # the collective on its own: the flat gradient buffer all-reduced back to back (what a step pays when nothing overlaps)
-        ms_ar = run(lambda i: reducer.allreduce(), 10, 3)
+        ms_ar = run(lambda i: reducer.allreduce(), steps, 3)
         out.update(allreduce_bytes_per_step=reducer.nbytes, allreduce_ms_alone=ms_ar)
     # ---- (3) the whole step as ONE CUDA graph (static-capacity march + FusedAdamW; constant LR inside the graph).  Under
     # data parallelism the gradient all-reduces (NCCL) are captured with it: at 1024 rays per GPU (C5 strong scaling at 8
@@ -529,7 +563,8 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     B = args.rays
     if args.only:
-        r = bench_c1(dev) if args.only == "c1_vanilla" else bench_dynamic(dev, args.only, occupancy=args.occupancy)
+        r = (bench_c1(dev, args.steps) if args.only == "c1_vanilla"
+             else bench_dynamic(dev, args.only, args.steps, occupancy=args.occupancy))
         print(json.dumps({args.only: r}), flush=True)
         return
 
@@ -556,11 +591,13 @@ def main():
     dev_pool = [tuple(t.to(dev) for t in b) for b in host_pool]
     h2d_bytes = sum(t.numel() * t.element_size() for t in host_pool[0])
 
+    last = {}                                              # what the latest train_step computed (--dump-outputs)
+
     def train_step(batch, grid):
         rays_o, rays_d, rgba = batch
         target = rgba[:, :3] * rgba[:, 3:4] + bg * (1.0 - rgba[:, 3:4])
-        pred, _, _ = render_rays(model=model, rays_o=rays_o, rays_d=rays_d, near=NEAR, far=FAR, n_samples=N_SAMPLES,
-                                 perturb=True, white_bkgd=True, density_grid=grid, bg_color=bg)
+        pred, depth, acc = render_rays(model=model, rays_o=rays_o, rays_d=rays_d, near=NEAR, far=FAR,
+                                       n_samples=N_SAMPLES, perturb=True, white_bkgd=True, density_grid=grid, bg_color=bg)
         loss_rgb = torch.nn.functional.mse_loss(pred, target)
         loss = loss_rgb + torch.mean(torch.abs(table[1:] - table[:-1])) * TV_WEIGHT
         reducer.zero_grad()
@@ -570,6 +607,7 @@ def main():
         torch.nn.utils.clip_grad_norm_(model.decoder.parameters(), max_norm=1.0)
         opt.step()
         sched.step()
+        last.update(color=pred.detach(), depth=depth.detach(), acc=acc.detach(), loss=loss.detach())
         return loss
 
     def barrier():
@@ -613,6 +651,10 @@ def main():
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
     value = world * B * args.steps / (ms * 1e-3)
     summary = prof.summary()
+    if args.dump_outputs and rank == 0:
+        params = list(model.named_parameters())
+        dump_outputs(args.dump_outputs, {**last, **{f"param.{n}": p for n, p in params},
+                                         **{f"grad.{n}": p.grad for n, p in params}})
 
     # ---- e2e: pinned host batch -> H2D -> step -> D2H loss, every step
     def e2e_step(i):
@@ -737,8 +779,8 @@ def main():
     if not args.no_extras and world > 1:
         # BASELINE.json configs[4]: Part 4 Dual-Hash, ray batch sharded over the GPUs, hash-table gradient all-reduce:
         # weak scaling (8192 rays per GPU) and the config's own global batch of 8192 rays split over the GPUs (strong)
-        weak = bench_dynamic(dev, "c5_dualhash", world=world, rank=rank)
-        strong = bench_dynamic(dev, "c5_dualhash", world=world, rank=rank, strong=True)
+        weak = bench_dynamic(dev, "c5_dualhash", args.steps, world=world, rank=rank)
+        strong = bench_dynamic(dev, "c5_dualhash", args.steps, world=world, rank=rank, strong=True)
         extras["c5_dualhash_dp"] = weak
         extras["c5_dualhash_dp_strong"] = strong
         dp_scalars = {"c5_dualhash_dp_weak_rays_per_s": weak.get("train_rays_per_s"),
@@ -750,9 +792,9 @@ def main():
                       "c5_dualhash_dp_allreduce_ms_alone": weak.get("allreduce_ms_alone"),
                       "c5_dualhash_dp_allreduce_bytes": weak.get("allreduce_bytes_per_step")}
     if not args.no_extras and rank == 0:
-        extras["c1_vanilla"] = bench_c1(dev)
+        extras["c1_vanilla"] = bench_c1(dev, args.steps)
         for name in DYNAMIC:
-            extras[name] = bench_dynamic(dev, name)
+            extras[name] = bench_dynamic(dev, name, args.steps)
 
     if rank != 0:
         if world > 1:
@@ -826,7 +868,7 @@ def main():
 
     cpu = None
     if world == 1 and not args.no_cpu_baseline:
-        r = cpu_train_rays_per_s(args.cpu_rays, 3, 1, args.occupancy)          # ~30-40 s of CPU work
+        r = cpu_train_rays_per_s(args.cpu_rays, args.steps, args.warmup, args.occupancy)   # --cpu-rays bounds its cost
         cpu = {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")}
 
     line = {
