@@ -34,8 +34,12 @@ int b2n_debug_instant_bwd_groups(int groups);
 
 /* A/B switch of the F = 2 hash-grid kernels: variant bit 0 = pair-lane forward (default on), bit 1 = pair-lane table
  * gradient (default on); 0 = the (point, level)-per-lane kernels.  merge_res >= 0 sets the coarsest-level run-merging
- * threshold of the pair-lane table gradient (levels with res <= merge_res are reduced across runs of equal cells). */
+ * threshold of the pair-lane table gradient (levels with res <= merge_res are reduced across runs of equal cells).
+ * B2N_EINVAL, and nothing changes, for a variant outside 0..3 or merge_res > 1625 (the merge path's uint32 cell id of a
+ * level holds res^3). */
 int b2n_debug_hash_variant(int variant, int merge_res);
+/* the current variant and merge threshold (host ints), so that a caller can restore what it found */
+int b2n_debug_hash_config(int* variant, int* merge_res);
 
 /* random 8-byte gathers over a float2[n_entries] table (n_entries = 2^k): the L2 gather peak the hash-grid kernels are
  * compared against (tools/kbench.py l2, bench.py hash_vs_l2) */

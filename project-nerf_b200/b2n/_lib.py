@@ -74,6 +74,7 @@ DEBUG_SIGNATURES = {
     "b2n_debug_mlp256_flags": [ctypes.c_int],
     "b2n_debug_mlp256_set_pair": [ctypes.c_int],
     "b2n_debug_hash_variant": [I, I],
+    "b2n_debug_hash_config": [P, P],
     "b2n_debug_instant_bwd_groups": [I],
     "b2n_debug_instant_fwd_slots": [I],
     "b2n_debug_gather_bench": [P, L, I, I, P, P],
@@ -156,12 +157,40 @@ def call(name: str, *args, work=(0.0, 0.0)):
     if prof is not None:
         e1.record()
         prof.records.append((name, float(work[0]), float(work[1]), e0, e1))
+    _raise_on(name, rc)
+    LAUNCHES["count"] += _KERNELS_PER_CALL.get(name, 1)
+
+
+def _raise_on(name, rc):
     if rc != 0:
         msg = lib.b2n_last_error().decode(errors="replace")
         if rc == -1:
             raise ValueError(f"{name}: {msg}")
         raise RuntimeError(f"{name} failed ({rc}): {msg}")
-    LAUNCHES["count"] += _KERNELS_PER_CALL.get(name, 1)
+
+
+def hash_config():
+    """(variant, merge_res) the F = 2 hash-grid kernels currently run with (include/b2nerf_debug.h)"""
+    v, m = ctypes.c_int(), ctypes.c_int()
+    _raise_on("b2n_debug_hash_config", lib.b2n_debug_hash_config(ctypes.byref(v), ctypes.byref(m)))
+    return v.value, m.value
+
+
+class hash_variant:
+    """``with hash_variant(variant, merge_res):`` -- the F = 2 hash-grid kernels run in that A/B configuration
+    (b2n_debug_hash_variant); the configuration found on entry is restored on exit."""
+
+    def __init__(self, variant, merge_res):
+        self.cfg = (variant, merge_res)
+
+    def __enter__(self):
+        self.prev = hash_config()
+        _raise_on("b2n_debug_hash_variant", lib.b2n_debug_hash_variant(*self.cfg))
+        return self
+
+    def __exit__(self, *exc):
+        _raise_on("b2n_debug_hash_variant", lib.b2n_debug_hash_variant(*self.prev))
+        return False
 
 
 # ---- device-side row count (b2n_set_active_rows): see march.march(static=True)

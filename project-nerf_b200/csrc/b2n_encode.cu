@@ -831,7 +831,17 @@ extern "C" int b2n_hash_tri_bwd(const float* x, const float* t, int64_t P, float
 }
 
 extern "C" int b2n_debug_hash_variant(int variant, int merge_res) {
+  B2N_REQUIRE(variant >= 0 && variant <= 3, "variant must be in 0..3");
+  // the run-merging path builds a uint32 cell id gx + gy res + gz res^2 of a level with res <= merge_res: res^3 must fit
+  B2N_REQUIRE(merge_res <= 1625, "merge_res must be <= 1625 (1626^3 overflows the uint32 cell id)");
   g_hash_variant = variant;
   if (merge_res >= 0) g_merge_res = (uint32_t)merge_res;
+  return B2N_OK;
+}
+
+extern "C" int b2n_debug_hash_config(int* variant, int* merge_res) {
+  B2N_REQUIRE(variant && merge_res, "null pointer");
+  *variant = g_hash_variant;
+  *merge_res = (int)g_merge_res;
   return B2N_OK;
 }

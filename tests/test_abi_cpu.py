@@ -48,6 +48,25 @@ def test_error_convention_without_gpu(lib):
     assert lib.lib.b2n_march_scan_scratch(2 ** 18) >= 4 * (128 + 2)
 
 
+def test_hash_variant_switch_reports_and_validates(lib):
+    """b2n_debug_hash_variant / b2n_debug_hash_config are host state: the shipped configuration is readable, a switch
+    restores what it found, and values the kernels cannot run (a merge threshold whose res^3 cell id overflows uint32, an
+    unknown variant) are refused without changing anything"""
+    shipped = lib.hash_config()
+    assert shipped == (3, 128)
+    with lib.hash_variant(1, 1625):
+        assert lib.hash_config() == (1, 1625)
+        with lib.hash_variant(2, 0):
+            assert lib.hash_config() == (2, 0)
+        assert lib.hash_config() == (1, 1625)
+    assert lib.hash_config() == shipped
+    for bad in ((3, 1626), (3, 2 ** 20), (4, 128), (-1, 128)):
+        with pytest.raises(ValueError, match="b2n_debug_hash_variant"):
+            with lib.hash_variant(*bad):
+                pass
+        assert lib.hash_config() == shipped
+
+
 def test_product_has_no_cpu_path(lib):
     import b2n
     with pytest.raises(ValueError, match="no CPU path"):

@@ -245,7 +245,7 @@ def test_hash_index_kat_exact(mods):
         assert ((y[:, li].double() - acc).abs() / (acc.abs() + 1)).max() < 1e-5, li
 
 
-@pytest.mark.parametrize("variant,merge_res", [(3, 64), (3, 0), (3, 200), (0, 64), (1, 64), (2, 24)])
+@pytest.mark.parametrize("variant,merge_res", [(3, 128), (3, 64), (3, 0), (3, 200), (0, 64), (1, 64), (2, 24)])
 @pytest.mark.parametrize("log2T", [19, 20])
 def test_hash_table_grad_on_ray_ordered_samples(mods, variant, merge_res, log2T):
     """Consecutive samples of a ray share coarse cells: the table-gradient kernels merge such runs inside a warp before
@@ -253,7 +253,6 @@ def test_hash_table_grad_on_ray_ordered_samples(mods, variant, merge_res, log2T)
     kernel variant / merge threshold, both canonical geometries (T = 2^20 makes level 4 a dense 81^3 level)."""
     from oracle import nerf_oracle as O
     b2n = mods["b2n"]
-    lib = b2n._lib.lib
     geom = b2n.HashGeometry(16, 16, 1.5, log2T, 2)
     lv = O.hash_level_table(16, 16, 1.5, log2T)
     gen = torch.Generator().manual_seed(9)
@@ -267,13 +266,10 @@ def test_hash_table_grad_on_ray_ordered_samples(mods, variant, merge_res, log2T)
     gy = torch.randn(y_ref.shape, generator=gen)
     gy[::11] = 0.0                                  # samples that receive no gradient
     gt_ref, gx_ref = torch.autograd.grad((y_ref * gy).sum(), [t_ref, x_ref])
-    try:
-        lib.b2n_debug_hash_variant(variant, merge_res)
+    with b2n._lib.hash_variant(variant, merge_res):
         t_cu, x_cu = cu(table).requires_grad_(True), cu(xw).requires_grad_(True)
         y = b2n.hash_encode(x_cu, t_cu, geom, 1.5)
         gt, gx = torch.autograd.grad((y * cu(gy)).sum(), [t_cu, x_cu])
-    finally:
-        lib.b2n_debug_hash_variant(3, 64)
     assert rel_err(y.cpu(), y_ref) < 1e-5
     assert record(f"hash_rays[v{variant},m{merge_res},T{log2T}]:g_table", rel_err(gt.cpu(), gt_ref)) < TOL
     assert rel_err(gx.cpu(), gx_ref) < TOL

@@ -313,7 +313,7 @@ def hash_variants():
     """A/B of the F = 2 hash-grid kernels on the C2 sample set (24 M active points, L = 16, T = 2^19) and the C5 canonical
     geometry (T = 2^20): (point, level)-per-lane kernels against the pair-lane kernels, and the run-merging threshold."""
     from b2n import synthetic, march
-    lib = b2n._lib.lib
+    hash_variant = b2n._lib.hash_variant
     torch.manual_seed(0)
     ro, rd, _ = (t.cuda() for t in synthetic.random_rays(2 ** 18, seed=1))
     u = torch.rand(2 ** 18, 128, device="cuda")
@@ -323,26 +323,25 @@ def hash_variants():
     for log2T in (19, 20):
         geom = b2n.HashGeometry(16, 16, 1.5, log2T, 2)
         table = (torch.randn(geom.n_params, device="cuda") * 0.1).requires_grad_(True)
-        lib.b2n_debug_hash_variant(0, 64)
-        y_ref = b2n.hash_encode(x, table, geom, 1.5)
-        g = torch.randn_like(y_ref)
-        gt_ref, = torch.autograd.grad((y_ref * g).sum(), table)
-        for variant, merge in ((0, 64), (1, 64), (2, 0), (2, 24), (2, 64), (2, 128), (2, 200), (3, 64)):
-            lib.b2n_debug_hash_variant(variant, merge)
-            y = b2n.hash_encode(x, table, geom, 1.5)
-            gt, = torch.autograd.grad((y * g).sum(), table)
-            ey = float((y - y_ref).abs().max() / y_ref.abs().max())
-            eg = float((gt - gt_ref).abs().max() / gt_ref.abs().max())
-            b2n._lib.PROFILER = prof = b2n._lib.Profiler()
-            for _ in range(4):
+        with hash_variant(0, 64):
+            y_ref = b2n.hash_encode(x, table, geom, 1.5)
+            g = torch.randn_like(y_ref)
+            gt_ref, = torch.autograd.grad((y_ref * g).sum(), table)
+        for variant, merge in ((0, 64), (1, 64), (2, 0), (2, 24), (2, 64), (2, 128), (2, 200), (3, 64), (3, 128)):
+            with hash_variant(variant, merge):
                 y = b2n.hash_encode(x, table, geom, 1.5)
-                y.backward(g)
-            torch.cuda.synchronize()
-            b2n._lib.PROFILER = None
+                gt, = torch.autograd.grad((y * g).sum(), table)
+                ey = float((y - y_ref).abs().max() / y_ref.abs().max())
+                eg = float((gt - gt_ref).abs().max() / gt_ref.abs().max())
+                b2n._lib.PROFILER = prof = b2n._lib.Profiler()
+                for _ in range(4):
+                    y = b2n.hash_encode(x, table, geom, 1.5)
+                    y.backward(g)
+                torch.cuda.synchronize()
+                b2n._lib.PROFILER = None
             print(f"T=2^{log2T} variant={variant} merge_res={merge:3d}: " +
                   ", ".join(f"{k} {min(e0.elapsed_time(e1) for n_, _, _, e0, e1 in prof.records if n_ == k):.3f} ms"
                             for k in ("b2n_hash_fwd", "b2n_hash_bwd")) + f"   max rel diff vs variant 0: y {ey:.2e} g_table {eg:.2e}")
-    lib.b2n_debug_hash_variant(3, 64)
 
 
 def red_bench():
