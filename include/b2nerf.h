@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 14
+#define B2N_ABI_VERSION 15
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -163,6 +163,24 @@ int b2n_hash_fwd(const float* x, int64_t P, float bound, const float* table, con
 int b2n_hash_bwd(const float* x, int64_t P, float bound, const float* table, const b2n_hash_level* levels_host,
                  int L, int F, const float* g_out, int ld_g, int col0, float* g_table, float* g_x, int accumulate_x,
                  int level_begin, int level_end, b2n_stream_t stream);
+
+/* Spatial order of the points, so that the 16 points a warp of the pair-lane kernels holds share cells and table lines:
+ * order int32 [P] is a permutation, sorted position -> original row, by the Morton code of the point's cell on a 2^7
+ * lattice over the box (within a cell, in no particular order); x_sorted [P,3] = x[order].  Rows behind the device-side
+ * row count (b2n_set_active_rows) keep their place.  scratch: b2n_hash_order_scratch(P) bytes, 16-byte aligned.  Five
+ * kernels, no host synchronisation. */
+size_t b2n_hash_order_scratch(int64_t P);
+int b2n_hash_order(const float* x, int64_t P, float bound, int* order, float* x_sorted, void* scratch,
+                   b2n_stream_t stream);
+/* b2n_hash_fwd / b2n_hash_bwd (table gradient only) over points in that order: point i is x_sorted[i], its feature row
+ * (gradient row) is row order[i] of out (g_out), so the results are those of the plain entries on x.  F = 2 and the
+ * pair-lane kernels only (b2nerf_debug.h variant 3); anything else is refused. */
+int b2n_hash_fwd_ordered(const float* x_sorted, const int* order, int64_t P, float bound, const float* table,
+                         const b2n_hash_level* levels_host, int L, int F, float* out, int ld_out, int col0,
+                         b2n_stream_t stream);
+int b2n_hash_bwd_ordered(const float* x_sorted, const int* order, int64_t P, float bound, const float* table,
+                         const b2n_hash_level* levels_host, int L, int F, const float* g_out, int ld_g, int col0,
+                         float* g_table, int level_begin, int level_end, b2n_stream_t stream);
 
 /* Tri-grid temporal blend of Part 4 (src/core.py:308-335): out[P, 2L] = sum_i w_i(t) * HashGrid_i(x) for the
  * start / mid / end deformation grids (one shared geometry, F = 2), w_i = clamp(1 - |t - a_i| / 0.5, 0, 1) with

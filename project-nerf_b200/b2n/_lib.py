@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb2nerf.so")
 
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 P, L, I, F = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
 
@@ -36,6 +36,10 @@ SIGNATURES = {
     "b2n_pe_bwd": [P, L, I, P, I, P, I, I, P, I, P],
     "b2n_hash_fwd": [P, L, F, P, P, I, I, P, I, I, P],
     "b2n_hash_bwd": [P, L, F, P, P, I, I, P, I, I, P, P, I, I, I, P],
+    "b2n_hash_order_scratch": [L],
+    "b2n_hash_order": [P, L, F, P, P, P, P],
+    "b2n_hash_fwd_ordered": [P, P, L, F, P, P, I, I, P, I, I, P],
+    "b2n_hash_bwd_ordered": [P, P, L, F, P, P, I, I, P, I, I, P, I, I, P],
     "b2n_hash_tri_fwd": [P, P, L, F, P, P, P, P, I, P, I, P],
     "b2n_hash_tri_bwd": [P, P, L, F, P, I, P, I, P, P, P, P],
     "b2n_linear_fwd": [P, I, P, I, P, P, I, L, I, I, I, P],
@@ -81,7 +85,7 @@ DEBUG_SIGNATURES = {
     "b2n_debug_red_bench": [P, L, I, I, I, P],
     "b2n_debug_mnmajor_probe": [P, P, P, I, I, I, I, P],
 }
-_RESTYPES = {"b2n_last_error": ctypes.c_char_p, "b2n_march_scan_scratch": ctypes.c_size_t,
+_RESTYPES = {"b2n_last_error": ctypes.c_char_p, "b2n_march_scan_scratch": ctypes.c_size_t, "b2n_hash_order_scratch": ctypes.c_size_t,
              "b2n_nerf_mlp_packed_bytes": ctypes.c_size_t, "b2n_nerf_mlp_packed_bwd_bytes": ctypes.c_size_t}
 
 
@@ -112,7 +116,7 @@ lib = _load()
 # launch accounting for bench.py ("gpu_launches"): every successful C-ABI call adds the
 # number of kernels that entry point launches.
 LAUNCHES = {"count": 0}
-_KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
+_KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_hash_order": 5, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
 
 
 def ptr(t):
@@ -145,6 +149,8 @@ class Profiler:
 
 
 PROFILER = None      # set to a Profiler() to time every C-ABI call
+# the ordered hash-grid entries compute what the plain ones compute: timed and counted under the same name
+_PROFILE_AS = {"b2n_hash_fwd_ordered": "b2n_hash_fwd", "b2n_hash_bwd_ordered": "b2n_hash_bwd"}
 
 
 def call(name: str, *args, work=(0.0, 0.0)):
@@ -156,7 +162,7 @@ def call(name: str, *args, work=(0.0, 0.0)):
     rc = getattr(lib, name)(*args)
     if prof is not None:
         e1.record()
-        prof.records.append((name, float(work[0]), float(work[1]), e0, e1))
+        prof.records.append((_PROFILE_AS.get(name, name), float(work[0]), float(work[1]), e0, e1))
     _raise_on(name, rc)
     LAUNCHES["count"] += _KERNELS_PER_CALL.get(name, 1)
 

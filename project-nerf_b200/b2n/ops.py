@@ -23,6 +23,9 @@ import os as _os
 INSTANT_FWD_TC = _os.environ.get("B2N_INSTANT_TC", "1") != "0"
 # backward: weight gradients on tcgen05 (k_instant_bwd_tc) or, when False, everything on mma.sync (k_instant_bwd)
 INSTANT_BWD_TC = _os.environ.get("B2N_INSTANT_BWD_TC", "1") != "0"
+# hash_encode sorts its points into spatial order (b2n_hash_order) from this many points on, when the input needs no
+# gradient and the F = 2 pair-lane kernels run: measured to pay at C2's 24 M points; smaller sets are not sorted
+HASH_ORDER_MIN_POINTS = 1 << 23
 
 
 def call(name, *args, work=(0.0, 0.0)):
@@ -105,9 +108,21 @@ class _HashEncode(torch.autograd.Function):
             raise ValueError(f"hash table has {table.numel()} params, geometry needs {geom.n_params}")
         Pn = x.shape[0]
         out = torch.empty(Pn, geom.out_dim, device=x.device, dtype=torch.float32)
-        call("b2n_hash_fwd", ptr(x), Pn, float(bound), ptr(table), geom.c_levels, geom.n_levels, geom.n_features,
-             ptr(out), geom.out_dim, 0, stream(),
-             work=(Pn * (12 + geom.n_levels * geom.n_features * 4 * 9), 0.0))
+        work = (Pn * (12 + geom.n_levels * geom.n_features * 4 * 9), 0.0)
+        ctx.order = None
+        if Pn >= HASH_ORDER_MIN_POINTS and geom.n_features == 2 and not ctx.needs_input_grad[0] and _lib.hash_config()[0] == 3:
+            # spatial order (b2n_hash_order): the warps of both kernels hold nearby points; features are unchanged
+            order = torch.empty(Pn, device=x.device, dtype=torch.int32)
+            xs = torch.empty_like(x)
+            scratch = torch.empty(_lib.lib.b2n_hash_order_scratch(Pn) // 4, device=x.device, dtype=torch.int32)
+            call("b2n_hash_order", ptr(x), Pn, float(bound), ptr(order), ptr(xs), ptr(scratch), stream(),
+                 work=(Pn * (12 + 4 + 4 + 12 + 4 + 12), 0.0))
+            call("b2n_hash_fwd_ordered", ptr(xs), ptr(order), Pn, float(bound), ptr(table), geom.c_levels, geom.n_levels,
+                 geom.n_features, ptr(out), geom.out_dim, 0, stream(), work=work)
+            x, ctx.order = xs, order
+        else:
+            call("b2n_hash_fwd", ptr(x), Pn, float(bound), ptr(table), geom.c_levels, geom.n_levels, geom.n_features,
+                 ptr(out), geom.out_dim, 0, stream(), work=work)
         ctx.save_for_backward(x, table)
         ctx.geom, ctx.bound = geom, bound
         ctx.sink = sink if (sink is not None and ctx.needs_input_grad[1]) else None
@@ -129,6 +144,10 @@ class _HashEncode(torch.autograd.Function):
         bytes_x = (24 + L * F * 4 * 9) * int(need_x)
 
         def launch(g_table, gx, lo, hi, nbytes):
+            if ctx.order is not None:             # x is in sorted order (forward); no input gradient on this path
+                call("b2n_hash_bwd_ordered", ptr(x), ptr(ctx.order), Pn, float(ctx.bound), ptr(table), geom.c_levels, L,
+                     F, ptr(g), geom.out_dim, 0, ptr(g_table), lo, hi, stream(), work=(Pn * nbytes, 0.0))
+                return
             call("b2n_hash_bwd", ptr(x), Pn, float(ctx.bound), ptr(table), geom.c_levels, L, F, ptr(g), geom.out_dim, 0,
                  ptr(g_table), ptr(gx), 0, lo, hi, stream(), work=(Pn * nbytes, 0.0))
 

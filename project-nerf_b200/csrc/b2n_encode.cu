@@ -5,6 +5,7 @@
 // src/decoders.py:83,159 cost no extra pass.
 #include "b2n_common.cuh"
 #include "b2n_hash.cuh"
+#include <cub/block/block_scan.cuh>
 
 namespace b2n {
 
@@ -302,13 +303,121 @@ k_hash_bwd_table_dense(const float* __restrict__ x, int64_t P, float bound, floa
 // warp holds fall into a handful of cells that share their lines.  Level geometry comes from the constant bank.
 __device__ __forceinline__ float pair_sum(float v) { return v + __shfl_xor_sync(0xffffffffu, v, 1); }
 
+// Spatial order (b2n_hash_order): in ray order the 16 points of a warp are 16 samples of one ray and share cells only at
+// the coarsest levels; in Morton order they share cells and table lines up to the middle levels.  The key is the Morton
+// code of the point's cell on a 2^7 lattice over the box; within a bucket points keep the order in which the counting
+// pass reached them (features do not depend on it, the table gradient is a sum of atomics anyway).
+constexpr int kOrderBits = 7;
+constexpr int kOrderBuckets = 1 << (3 * kOrderBits);      // 2 M counters: 8 MB of L2, beside the 52 MB C2 gradient table
+constexpr int kOrderTile = 2048;                          // buckets per scan block (256 threads x 8)
+constexpr int kOrderTiles = kOrderBuckets / kOrderTile;   // 1024: one block scans the tile sums
+// Ordered input: the blocks resident at one time hold ~150 k consecutive points, a small stretch of the curve, and the
+// coarse-level reductions of every SM would meet at the same few entries (scatter 7.5 -> 11.5 ms at 24 M points).  Block
+// b takes the 128-point chunk (b mod kSpread) * R + b / kSpread of R * kSpread chunks: consecutive blocks sit 1/kSpread of
+// the curve apart.  The ordered grid is padded to a multiple of kSpread blocks.
+constexpr int kSpread = 2048;
+
+__device__ __forceinline__ uint32_t spread3(uint32_t v) {     // 10 bits -> every third bit
+  v = (v | (v << 16)) & 0x030000FFu;
+  v = (v | (v << 8)) & 0x0300F00Fu;
+  v = (v | (v << 4)) & 0x030C30C3u;
+  return (v | (v << 2)) & 0x09249249u;
+}
+
+__device__ __forceinline__ uint32_t order_key(const float* __restrict__ x, int64_t p, float bound, float two_bound) {
+  uint32_t q[3];
+#pragma unroll
+  for (int d = 0; d < 3; ++d) {
+    bool in;
+    const float u = to_unit(__ldg(x + 3 * p + d), bound, two_bound, &in);      // clamped to [0, 1]; NaN -> 0
+    q[d] = min((uint32_t)(u * (float)(1 << kOrderBits)), (uint32_t)((1 << kOrderBits) - 1));
+  }
+  return spread3(q[0]) | (spread3(q[1]) << 1) | (spread3(q[2]) << 2);
+}
+
+// first point of the 128-point chunk this block walks, or -1 (nothing to do)
+__device__ __forceinline__ int64_t block_first_point(int64_t P, bool ordered) {
+  if (!ordered) return (int64_t)blockIdx.x * 128;
+  const int64_t nc = (P + 127) / 128, R = (nc + kSpread - 1) / kSpread, b = blockIdx.x;
+  if (b / kSpread >= R) return -1;                      // padding of the grid: keeps the mapping one-to-one
+  const int64_t c = (b % kSpread) * R + b / kSpread;
+  return c < nc ? c * 128 : -1;
+}
+
+__global__ void __launch_bounds__(256)
+k_order_count(const float* __restrict__ x, int64_t P, float bound, float two_bound, int* __restrict__ counts,
+              int* __restrict__ rank, const int* __restrict__ rows) {
+  P = clamp_rows(P, rows);
+  const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p < P) rank[p] = atomicAdd(counts + order_key(x, p, bound, two_bound), 1);
+}
+
+// exclusive scan of the bucket counts inside each tile of kOrderTile buckets (in place); tile totals to tile_sum
+__global__ void __launch_bounds__(256) k_order_scan_tiles(int* __restrict__ counts, int* __restrict__ tile_sum) {
+  using Scan = cub::BlockScan<int, 256>;
+  __shared__ typename Scan::TempStorage tmp;
+  int4* base = reinterpret_cast<int4*>(counts + (int64_t)blockIdx.x * kOrderTile) + 2 * threadIdx.x;
+  const int4 a = base[0], b = base[1];
+  int v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+  int tot = 0;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) tot += v[i];
+  int pre, all;
+  Scan(tmp).ExclusiveSum(tot, pre, all);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const int t = v[i];
+    v[i] = pre;
+    pre += t;
+  }
+  base[0] = make_int4(v[0], v[1], v[2], v[3]);
+  base[1] = make_int4(v[4], v[5], v[6], v[7]);
+  if (threadIdx.x == 0) tile_sum[blockIdx.x] = all;
+}
+
+__global__ void __launch_bounds__(kOrderTiles) k_order_scan_top(int* __restrict__ tile_sum) {
+  using Scan = cub::BlockScan<int, kOrderTiles>;
+  __shared__ typename Scan::TempStorage tmp;
+  int v = tile_sum[threadIdx.x];
+  Scan(tmp).ExclusiveSum(v, v);
+  tile_sum[threadIdx.x] = v;
+}
+
+// only the 4-byte order entry is stored at the scattered position; x_sorted follows in k_order_gather with contiguous
+// stores (three scattered 4-byte stores per point into the 288 MB x_sorted cost more than the whole sort otherwise)
+__global__ void __launch_bounds__(256)
+k_order_scatter(const float* __restrict__ x, int64_t P_cap, float bound, float two_bound, const int* __restrict__ counts,
+                const int* __restrict__ tile_sum, const int* __restrict__ rank, int* __restrict__ order,
+                const int* __restrict__ rows) {
+  const int64_t P = clamp_rows(P_cap, rows);
+  const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= P_cap) return;
+  int64_t pos = p;                                      // rows behind the device-side count keep their place
+  if (p < P) {
+    const uint32_t k = order_key(x, p, bound, two_bound);
+    pos = (int64_t)__ldg(tile_sum + k / kOrderTile) + __ldg(counts + k) + rank[p];
+  }
+  order[pos] = (int)p;
+}
+
+__global__ void __launch_bounds__(256)
+k_order_gather(const float* __restrict__ x, int64_t P_cap, const int* __restrict__ order, float* __restrict__ xs) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= P_cap) return;
+  const int64_t p = __ldg(order + i);
+#pragma unroll
+  for (int d = 0; d < 3; ++d) xs[3 * i + d] = __ldg(x + 3 * p + d);
+}
+
 __global__ void __launch_bounds__(256)
 k_hash_fwd_pair(const float* __restrict__ x, int64_t P, float bound, float two_bound, const float2* __restrict__ table,
-                const Levels lv, int nl, float* __restrict__ out, int ld, int col0, const int* __restrict__ rows) {
+                const Levels lv, int nl, float* __restrict__ out, int ld, int col0, const int* __restrict__ order,
+                const int* __restrict__ rows) {
+  // order != NULL: x is in sorted order and point i's feature row is row order[i] of out
   P = clamp_rows(P, rows);
-  if ((int64_t)blockIdx.x * (blockDim.x >> 1) >= P) return;      // whole block behind the (device-side) row count
-  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t p = tid >> 1;
+  const int64_t p_block = block_first_point(P, order != nullptr);
+  if (p_block < 0 || p_block >= P) return;                        // whole block behind the (device-side) row count
+  const int64_t p = p_block + (threadIdx.x >> 1);
   const int s = threadIdx.x & 1;
   const bool live = p < P;
   float x01[3] = {0.f, 0.f, 0.f};
@@ -317,7 +426,7 @@ k_hash_fwd_pair(const float* __restrict__ x, int64_t P, float bound, float two_b
 #pragma unroll
     for (int d = 0; d < 3; ++d) x01[d] = to_unit(__ldg(x + 3 * p + d), bound, two_bound, &in);
   }
-  float* orow = out + p * ld + col0;
+  float* orow = out + (order && live ? (int64_t)__ldg(order + p) : p) * ld + col0;
   const bool vec = ((reinterpret_cast<uintptr_t>(out + col0) & 15) == 0) && ((ld & 3) == 0);
   // When the feature rows are contiguous (the plain [P, 2L] output, 2L <= 32) a warp's 16 rows are one contiguous block:
   // the levels are collected in shared memory and leave as fully coalesced 16-byte stores (4 lines per instruction instead
@@ -373,13 +482,15 @@ k_hash_fwd_pair(const float* __restrict__ x, int64_t P, float bound, float two_b
   }
   if (contig) {
     __syncwarp();
-    const int64_t p_warp = ((int64_t)blockIdx.x * blockDim.x + 32 * warp) >> 1;     // first point of this warp
+    const int64_t p_warp = p_block + 16 * warp;                                         // first point of this warp
     const int per_row = ld >> 2;                                                        // float4 per feature row
     const int n4 = 16 * per_row;
-    float4* dst = reinterpret_cast<float4*>(out + p_warp * ld);
     for (int i = lane; i < n4; i += 32) {
       const int row = i / per_row, col = i - row * per_row;
-      if (p_warp + row < P) __stcs(dst + i, stage[warp][row * 10 + col]);
+      const int64_t pr = p_warp + row;
+      // ordered: the rows land at scattered addresses, but each is still one whole 128-byte line
+      if (pr < P) __stcs(reinterpret_cast<float4*>(out + (order ? (int64_t)__ldg(order + pr) : pr) * ld) + col,
+                         stage[warp][row * 10 + col]);
     }
   }
 }
@@ -390,13 +501,14 @@ k_hash_fwd_pair(const float* __restrict__ x, int64_t P, float bound, float two_b
 __global__ void __launch_bounds__(256)
 k_hash_bwd_table_pair(const float* __restrict__ x, int64_t P, float bound, float two_bound, const Levels lv, int lbeg,
                       int nl, const float* __restrict__ g, int ld, int col0, float2* __restrict__ g_table,
-                      uint32_t merge_res, const int* __restrict__ rows) {
+                      uint32_t merge_res, const int* __restrict__ order, const int* __restrict__ rows) {
   P = clamp_rows(P, rows);
   // levels [lbeg, nl) of the table (lbeg a multiple of 4): a caller that overlaps the gradient all-reduce of the fine
-  // levels with the scatter of the coarse ones launches this kernel once per level window
-  if ((int64_t)blockIdx.x * (blockDim.x >> 1) >= P) return;      // whole block behind the (device-side) row count
-  const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t p = tid >> 1;
+  // levels with the scatter of the coarse ones launches this kernel once per level window.  order != NULL: x is in
+  // sorted order and point i's gradient row is row order[i] of g
+  const int64_t p_block = block_first_point(P, order != nullptr);
+  if (p_block < 0 || p_block >= P) return;                        // whole block behind the (device-side) row count
+  const int64_t p = p_block + (threadIdx.x >> 1);
   const int lane = threadIdx.x & 31, s = lane & 1, pi = lane >> 1;     // pi: point index inside the warp (0..15)
   const bool live = p < P;
   float x01[3] = {0.f, 0.f, 0.f};
@@ -405,7 +517,7 @@ k_hash_bwd_table_pair(const float* __restrict__ x, int64_t P, float bound, float
 #pragma unroll
     for (int d = 0; d < 3; ++d) x01[d] = to_unit(__ldg(x + 3 * p + d), bound, two_bound, &in);
   }
-  const float* grow = g + p * ld + col0;
+  const float* grow = g + (order && live ? (int64_t)__ldg(order + p) : p) * ld + col0;
   const bool vec = ((reinterpret_cast<uintptr_t>(g + col0) & 15) == 0) && ((ld & 3) == 0);
   for (int l0 = lbeg; l0 < nl; l0 += 4) {
     float gv[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -444,7 +556,9 @@ k_hash_bwd_table_pair(const float* __restrict__ x, int64_t P, float bound, float
       const uint32_t cell_prev = __shfl_up_sync(0xffffffffu, cell, 2);
       const bool head = (pi == 0) || (cell != cell_prev);
       const uint32_t heads = __ballot_sync(0xffffffffu, head && s == 0);
-      const int steps = L.res <= 24 ? 3 : (L.res <= 64 ? 2 : 1);
+      // merge depth (2^steps points): in ray order runs are about res / 12 samples long; in Morton order a warp's 16
+      // points share a cell at the coarse levels and a few of them still do at res ~ 100 (measured at 24 M points)
+      const int steps = order ? (L.res <= 54 ? 4 : (L.res <= 122 ? 3 : 2)) : (L.res <= 24 ? 3 : (L.res <= 64 ? 2 : 1));
       const int run_start = (31 - __clz((int)(heads & (0xffffffffu >> (31 - 2 * pi))))) >> 1;
       const bool issuer = live && (((pi - run_start) & ((1 << steps) - 1)) == 0);
 #pragma unroll
@@ -455,7 +569,7 @@ k_hash_bwd_table_pair(const float* __restrict__ x, int64_t P, float bound, float
           const int o = 1 << st;
           const float t0 = __shfl_down_sync(0xffffffffu, v0, 2 * o), t1 = __shfl_down_sync(0xffffffffu, v1, 2 * o);
           // points pi+1 .. pi+o all continue this point's run <=> none of them is a head
-          const uint32_t span = (o == 1) ? 0x1u : (o == 2 ? 0x5u : 0x55u);
+          const uint32_t span = ((1u << (2 * o)) - 1u) & 0x55555555u;      // the even (head) bits of points pi+1 .. pi+o
           const bool same_run = (pi + o < 16) && (((heads >> (2 * (pi + 1))) & span) == 0u);
           if (same_run) v0 += t0, v1 += t1;
         }
@@ -729,10 +843,16 @@ extern "C" int b2n_pe_bwd(const float* x, int64_t P, int D, const float* bands, 
   return check_launch("b2n_pe_bwd");
 }
 
-extern "C" int b2n_hash_fwd(const float* x, int64_t P, float bound, const float* table,
-                            const b2n_hash_level* levels_host, int L, int F, float* out, int ld_out, int col0,
-                            b2n_stream_t stream) {
+// grid of the pair-lane kernels: 128 points per block; ordered input pads it to a multiple of kSpread (block_first_point)
+static unsigned pair_grid(int64_t P, const int* order) {
+  const int64_t g = (P + 127) / 128;
+  return (unsigned)(order ? (g + kSpread - 1) / kSpread * kSpread : (g < 1 ? 1 : g));
+}
+
+static int hash_fwd(const float* x, const int* order, int64_t P, float bound, const float* table,
+                    const b2n_hash_level* levels_host, int L, int F, float* out, int ld_out, int col0, b2n_stream_t stream) {
   B2N_REQUIRE(P >= 0 && (F == 1 || F == 2 || F == 4) && bound >= 0.f, "bad shape (F in {1,2,4})");
+  B2N_REQUIRE(!order || (F == 2 && (g_hash_variant & 1)), "an order needs F = 2 and the pair-lane forward");
   Levels lv;
   B2N_REQUIRE(fill_levels(levels_host, L, &lv) == 0, "bad level table");
   if (P == 0) return B2N_OK;
@@ -743,18 +863,17 @@ extern "C" int b2n_hash_fwd(const float* x, int64_t P, float bound, const float*
   const float tb = 2.0f * bound;
   cudaStream_t st = (cudaStream_t)stream;
   if (F == 2 && (g_hash_variant & 1))
-    k_hash_fwd_pair<<<grid_for(2 * P, 256), 256, 0, st>>>(x, P, bound, tb, reinterpret_cast<const float2*>(table), lv, L, out,
-                                                        ld_out, col0, g_active_rows);
+    k_hash_fwd_pair<<<pair_grid(P, order), 256, 0, st>>>(x, P, bound, tb, reinterpret_cast<const float2*>(table), lv, L, out,
+                                                       ld_out, col0, order, g_active_rows);
   else if (F == 2) k_hash_fwd<2><<<grid, 256, 0, st>>>(x, P, bound, tb, table, lv, L, out, ld_out, col0, g_active_rows);
   else if (F == 4) k_hash_fwd<4><<<grid, 256, 0, st>>>(x, P, bound, tb, table, lv, L, out, ld_out, col0, g_active_rows);
   else k_hash_fwd<1><<<grid, 256, 0, st>>>(x, P, bound, tb, table, lv, L, out, ld_out, col0, g_active_rows);
   return check_launch("b2n_hash_fwd");
 }
 
-extern "C" int b2n_hash_bwd(const float* x, int64_t P, float bound, const float* table,
-                            const b2n_hash_level* levels_host, int L, int F, const float* g_out, int ld_g, int col0,
-                            float* g_table, float* g_x, int accumulate_x, int level_begin, int level_end,
-                            b2n_stream_t stream) {
+static int hash_bwd(const float* x, const int* order, int64_t P, float bound, const float* table,
+                    const b2n_hash_level* levels_host, int L, int F, const float* g_out, int ld_g, int col0,
+                    float* g_table, float* g_x, int accumulate_x, int level_begin, int level_end, b2n_stream_t stream) {
   B2N_REQUIRE(P >= 0 && (F == 1 || F == 2 || F == 4) && bound >= 0.f, "bad shape (F in {1,2,4})");
   if (level_end < 0) level_end = L;
   B2N_REQUIRE(level_begin >= 0 && level_begin <= level_end && level_end <= L, "bad level window");
@@ -768,12 +887,15 @@ extern "C" int b2n_hash_bwd(const float* x, int64_t P, float bound, const float*
   B2N_REQUIRE(!g_x || table, "input gradient needs the table");
   B2N_REQUIRE((reinterpret_cast<uintptr_t>(g_table) & 15) == 0 && (reinterpret_cast<uintptr_t>(table) & 15) == 0,
               "table / g_table must be 16-byte aligned (vector reductions)");
+  B2N_REQUIRE(!order || (!g_x && F == 2 && ((g_hash_variant & 2) || windowed)),
+              "an order needs F = 2, the pair-lane table gradient and no input gradient");
   const float tb = 2.0f * bound;
   cudaStream_t st = (cudaStream_t)stream;
   if (g_table && F == 2 && ((g_hash_variant & 2) || windowed)) {
     if (level_begin < level_end)
-      k_hash_bwd_table_pair<<<grid_for(2 * P, 256), 256, 0, st>>>(x, P, bound, tb, lv, level_begin, level_end, g_out, ld_g,
-                                                                col0, reinterpret_cast<float2*>(g_table), g_merge_res, g_active_rows);
+      k_hash_bwd_table_pair<<<pair_grid(P, order), 256, 0, st>>>(x, P, bound, tb, lv, level_begin, level_end, g_out, ld_g,
+                                                               col0, reinterpret_cast<float2*>(g_table), g_merge_res, order,
+                                                               g_active_rows);
   } else if (g_table) {
     int n_dense = 0;                      // leading run of un-hashed levels
     while (n_dense < L && !lv.l[n_dense].hashed) ++n_dense;
@@ -800,6 +922,59 @@ extern "C" int b2n_hash_bwd(const float* x, int64_t P, float bound, const float*
     else k_hash_bwd_input<1><<<grid, 256, 0, st>>>(x, P, bound, tb, table, lv, L, g_out, ld_g, col0, g_x, accumulate_x, g_active_rows);
   }
   return check_launch("b2n_hash_bwd");
+}
+
+extern "C" int b2n_hash_fwd(const float* x, int64_t P, float bound, const float* table,
+                            const b2n_hash_level* levels_host, int L, int F, float* out, int ld_out, int col0,
+                            b2n_stream_t stream) {
+  return hash_fwd(x, nullptr, P, bound, table, levels_host, L, F, out, ld_out, col0, stream);
+}
+
+extern "C" int b2n_hash_fwd_ordered(const float* x_sorted, const int* order, int64_t P, float bound, const float* table,
+                                    const b2n_hash_level* levels_host, int L, int F, float* out, int ld_out, int col0,
+                                    b2n_stream_t stream) {
+  B2N_REQUIRE(order, "null order");
+  return hash_fwd(x_sorted, order, P, bound, table, levels_host, L, F, out, ld_out, col0, stream);
+}
+
+extern "C" int b2n_hash_bwd(const float* x, int64_t P, float bound, const float* table,
+                            const b2n_hash_level* levels_host, int L, int F, const float* g_out, int ld_g, int col0,
+                            float* g_table, float* g_x, int accumulate_x, int level_begin, int level_end,
+                            b2n_stream_t stream) {
+  return hash_bwd(x, nullptr, P, bound, table, levels_host, L, F, g_out, ld_g, col0, g_table, g_x, accumulate_x,
+                  level_begin, level_end, stream);
+}
+
+extern "C" int b2n_hash_bwd_ordered(const float* x_sorted, const int* order, int64_t P, float bound, const float* table,
+                                    const b2n_hash_level* levels_host, int L, int F, const float* g_out, int ld_g,
+                                    int col0, float* g_table, int level_begin, int level_end, b2n_stream_t stream) {
+  B2N_REQUIRE(order, "null order");
+  return hash_bwd(x_sorted, order, P, bound, table, levels_host, L, F, g_out, ld_g, col0, g_table, nullptr, 0,
+                  level_begin, level_end, stream);
+}
+
+extern "C" size_t b2n_hash_order_scratch(int64_t P) {
+  return sizeof(int) * ((size_t)kOrderBuckets + kOrderTiles + (size_t)(P > 0 ? P : 0));
+}
+
+extern "C" int b2n_hash_order(const float* x, int64_t P, float bound, int* order, float* x_sorted, void* scratch,
+                              b2n_stream_t stream) {
+  B2N_REQUIRE(P >= 0 && P < (1LL << 31) && bound >= 0.f, "bad shape (P < 2^31 rows)");
+  if (P == 0) return B2N_OK;
+  B2N_REQUIRE(x && order && x_sorted && scratch, "null pointer");
+  B2N_REQUIRE((reinterpret_cast<uintptr_t>(scratch) & 15) == 0, "scratch must be 16-byte aligned");
+  int* counts = static_cast<int*>(scratch);
+  int* tile_sum = counts + kOrderBuckets;
+  int* rank = tile_sum + kOrderTiles;
+  cudaStream_t st = (cudaStream_t)stream;
+  const float tb = 2.0f * bound;
+  if (cudaMemsetAsync(counts, 0, sizeof(int) * kOrderBuckets, st) != cudaSuccess) return check_launch("b2n_hash_order");
+  k_order_count<<<grid_for(P, 256), 256, 0, st>>>(x, P, bound, tb, counts, rank, g_active_rows);
+  k_order_scan_tiles<<<kOrderTiles, 256, 0, st>>>(counts, tile_sum);
+  k_order_scan_top<<<1, kOrderTiles, 0, st>>>(tile_sum);
+  k_order_scatter<<<grid_for(P, 256), 256, 0, st>>>(x, P, bound, tb, counts, tile_sum, rank, order, g_active_rows);
+  k_order_gather<<<grid_for(P, 256), 256, 0, st>>>(x, P, order, x_sorted);
+  return check_launch("b2n_hash_order");
 }
 
 extern "C" int b2n_hash_tri_fwd(const float* x, const float* t, int64_t P, float bound, const float* table_start,

@@ -270,15 +270,19 @@ def hash_levels(P=24_000_000):
 
 
 def hash_sorted():
-    """What spatial order buys the hash-grid kernels AS THEY ARE (lanes = the 16 levels of a point): the C2 sample set in
-    ray order against the same points sorted by a 30-bit Morton key (torch argsort; sort cost reported separately)."""
+    """What spatial order buys the shipped pair-lane hash-grid kernels (variant 3) on the C2 sample set (dense occupancy,
+    2^18 rays x 128 samples, L = 16, T = 2^19): ray order against the same points ordered by a Morton key of their cell on
+    a 2^k lattice over the box (torch.argsort, stable, so a cell keeps its points in ray order), and against the k = 10 order
+    with its 128-point blocks interleaved over the curve, with the run-merging threshold merge_res swept.  Per entry: median
+    and best of 10 calls (CUDA events of b2n._lib.Profiler).  Result: profiles/hashsort_b200.txt, DESIGN.md section 7b."""
     from b2n import synthetic, march
+    hash_variant = b2n._lib.hash_variant
     torch.manual_seed(0)
     ro, rd, _ = (t.cuda() for t in synthetic.random_rays(2 ** 18, seed=1))
     u = torch.rand(2 ** 18, 128, device="cuda")
     occ = torch.ones(128, 128, 128, dtype=torch.bool, device="cuda")
     x = march.march(ro, rd, 2.0, 6.0, 128, u, bits=march.pack_occupancy(occ), R=128, bound=1.5).pts
-    print("points", x.shape[0])
+    print("points", x.shape[0], "|", torch.cuda.get_device_name())
 
     def spread(v):                                   # 10 bits -> every third bit
         v = (v | (v << 16)) & 0x030000FF
@@ -286,27 +290,41 @@ def hash_sorted():
         v = (v | (v << 4)) & 0x030C30C3
         return (v | (v << 2)) & 0x09249249
 
-    def morton(p):
-        q = ((p + 1.5) / 3.0 * 1023.0).clamp(0, 1023).to(torch.int64)
+    def morton(p, k):
+        q = ((p + 1.5) / 3.0 * (1 << k)).clamp(0, (1 << k) - 1).to(torch.int64)
         return spread(q[:, 0]) | (spread(q[:, 1]) << 1) | (spread(q[:, 2]) << 2)
 
-    t_sort, _ = timeit(lambda: torch.argsort(morton(x)), n=3, warm=1)
-    order = torch.argsort(morton(x))
-    xs = x[order].contiguous()
-    print(f"morton key + torch.argsort: {t_sort:.3f} ms (a radix sort of 30-bit keys would be the product path)")
+    def interleave(xs, S=2048):
+        # the sorted set in chunks of 128 points (one block of the pair-lane kernels), chunk i of a group of S at curve
+        # position i * (n_chunks / S): consecutive blocks -- the ones resident at the same time -- sit far apart on the curve
+        nc = xs.shape[0] // 128 // S * S
+        head = xs[: nc * 128].view(S, nc // S, 128, 3).transpose(0, 1).reshape(-1, 3)
+        return torch.cat([head, xs[nc * 128:]]).contiguous()
+
+    sets = [("ray order", x)]
+    for k in (8, 10):
+        t_sort, _ = timeit(lambda: x[torch.argsort(morton(x, k), stable=True)], n=5, warm=2)
+        sets.append((f"morton k={k}", x[torch.argsort(morton(x, k), stable=True)].contiguous()))
+        print(f"morton key (k={k}) + torch.argsort + gather: {t_sort:.3f} ms")
+    sets.append(("morton k=10, blocks interleaved", interleave(sets[-1][1])))
     geom = b2n.HashGeometry(16, 16, 1.5, 19, 2)
     table = (torch.randn(geom.n_params, device="cuda") * 0.1).requires_grad_(True)
-    for name, pts in (("ray order", x), ("morton order", xs)):
-        y = b2n.hash_encode(pts, table, geom, 1.5)
-        g = torch.randn_like(y)
-        b2n._lib.PROFILER = prof = b2n._lib.Profiler()
-        for _ in range(4):
-            y = b2n.hash_encode(pts, table, geom, 1.5)
-            y.backward(g)
-        torch.cuda.synchronize()
-        b2n._lib.PROFILER = None
-        print(f"{name:13s}: " + ", ".join(f"{k} {min(e0.elapsed_time(e1) for n_, _, _, e0, e1 in prof.records if n_ == k):.3f} ms"
-                                           for k in ("b2n_hash_fwd", "b2n_hash_bwd")))
+    keys = ("b2n_hash_fwd", "b2n_hash_bwd")
+    for name, pts in sets:
+        for merge in (128, 200, 300, 400):
+            with hash_variant(3, merge):
+                y = b2n.hash_encode(pts, table, geom, 1.5)
+                g = torch.randn_like(y)
+                b2n._lib.PROFILER = prof = b2n._lib.Profiler()
+                for _ in range(10):
+                    y = b2n.hash_encode(pts, table, geom, 1.5)
+                    y.backward(g)
+                torch.cuda.synchronize()
+                b2n._lib.PROFILER = None
+            ts = {k: sorted(e0.elapsed_time(e1) for n_, _, _, e0, e1 in prof.records if n_ == k) for k in keys}
+            med = {k: v[len(v) // 2] for k, v in ts.items()}
+            print(f"{name:31s} merge_res={merge:3d}: " + ", ".join(f"{k} {med[k]:.3f} (best {ts[k][0]:.3f}) ms" for k in keys)
+                  + f", fwd+bwd {sum(med.values()):.3f} ms")
 
 
 def hash_variants():
