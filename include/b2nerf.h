@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 15
+#define B2N_ABI_VERSION 16
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -417,6 +417,36 @@ int b2n_opt_prepare(const b2n_opt_tensor* tensors, int n_tensors, const float* g
 int b2n_opt_adamw(const b2n_opt_tensor* tensors, int n_tensors, const float* grad_scale, int already_unscaled,
                   const float* found_inf, const float* step_dev, const float* norm2, const float* max_norm_host,
                   b2n_stream_t stream);
+
+/* ------------------------------------------------------------------------
+ * Surface extraction (marching tetrahedra) from a density lattice: the closed triangle mesh of the region sigma > tau,
+ * e.g. of the lattice that DensityGrid.update sweeps (src/renderer.py:49-116), at any resolution 2 <= R <= 1024.
+ *   sigma [R,R,R] fp32, index [ix,iy,iz] (x slowest) = the point (axis[ix], axis[iy], axis[iz]) of a 1-D axis (torch's
+ *     linspace(-bound, bound, R) in the Python API).  A point is INSIDE when sigma > tau (strict, as `grid > threshold`);
+ *     tau > 0 and finite.
+ *   The lattice is padded with a virtual ring of points where sigma = 0, so every surface is closed: the EXTENDED axis
+ *     axis_ext [R+2] = {axis[0] - h, axis[0..R-1], axis[R-1] + h}, h = axis[1] - axis[0] (fp32), is what the vertex
+ *     coordinates come from.  Points of the extended lattice are numbered p = (i*(R+2) + j)*(R+2) + k.
+ *   Every cell is split into the 6 Kuhn tetrahedra {0, e_a, e_a+e_b, e_a+e_b+e_c} for the permutations (a,b,c) of the
+ *     axes in lexicographic order xyz, xzy, yxz, yzx, zxy, zyx.  Their edges run from a point p to p + d, d one of 7
+ *     direction classes in the order x, y, z, xy, xz, yz, xyz.  Each edge whose ends lie on different sides of tau
+ *     carries ONE vertex shared by every face around it: a = p, b = p + d, t = (tau - sigma_a) / (sigma_b - sigma_a),
+ *     vertex = a + t*(b - a) per coordinate, each operation rounded separately (fp32, no fused multiply-add).
+ *   A tetrahedron with 1 or 3 corners inside gives one triangle, with 2 inside a quad (ik, il, jl, jk) (i < j inside,
+ *     k, l outside ordered so that (i,j,k,l) is an even permutation of the corners 0..3), split along ik - jl.  Every
+ *     triangle is wound so that its normal points from inside to outside (derived from the case and the tetrahedron's
+ *     parity, never from coordinates).
+ *   Order (deterministic, no atomics): vertices by point p, then direction class; faces by cell (= its lowest point p),
+ *     then tetrahedron, then triangle.
+ * b2n_mesh_count: sigma -> totals (device int64 [2]: number of vertices V, faces F; exact, even when they exceed int32)
+ *   and the per-point counts in scratch (b2n_mesh_scratch(R) bytes, 256-byte aligned; 0 for an unsupported R).
+ * b2n_mesh_emit: with the same sigma, tau and scratch, and V / F read back from totals -> verts [V,3] fp32 (world
+ *   coordinates), faces [F,3] int32 vertex ids.  Refuses V or F >= 2^31.  Two kernels; V == 0 is a no-op.
+ * The host read of the totals between the two calls is the only synchronisation of an extraction. */
+size_t b2n_mesh_scratch(int R);
+int b2n_mesh_count(const float* sigma, int R, float threshold, void* scratch, int64_t* totals, b2n_stream_t stream);
+int b2n_mesh_emit(const float* sigma, const float* axis_ext, int R, float threshold, void* scratch, int64_t n_verts,
+                  int64_t n_faces, float* verts, int32_t* faces, b2n_stream_t stream);
 
 #ifdef __cplusplus
 }

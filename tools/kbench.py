@@ -207,6 +207,45 @@ def occ_update():
                   f"three calls in a row (run.py pattern) median {med3:.3f} ms")
 
 
+def mesh(sizes=(128, 256, 512)):
+    """b2n.mesh: the sigma sweep of the C2 model (part2_instant, scene_bound 1.5, bf16 mode, density branch) on an R^3
+    lattice, and surface extraction alone on an analytic field (a ball of radius 0.6 in [-1, 1]^3, sigma = 1 + 4 * signed
+    distance, tau = 1; count / emit split from per-entry CUDA events).  Medians over 10 runs after 3 warm-ups."""
+    import subprocess
+    from b2n import mesh as bm
+    try:
+        smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,power.max_limit", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=60).stdout.strip().splitlines()[0]
+    except Exception as e:                                # noqa: BLE001 -- the measurement stands without it
+        smi = f"nvidia-smi unavailable ({e})"
+    print(f"device: {torch.cuda.get_device_name()} | nvidia-smi name, power.limit, power.max_limit: {smi}")
+    b2n.set_mlp_precision("bf16")
+    torch.manual_seed(0)
+    model = NeuralField(dict(mode="part2_instant", scene_bound=1.5)).cuda().eval()
+    for R in sizes:
+        med, best = timeit(lambda: bm.density_lattice(model, R, 1.5), n=10, warm=3)
+        print(f"sweep C2 part2_instant R={R}: {R ** 3 / 1e6:.1f} M points, median {med:.3f} ms (best {best:.3f}), "
+              f"{R ** 3 / med / 1e6:.2f} G points/s")
+    for R in sizes:
+        ax = bm.lattice_axis(R, 1.0, "cuda").double()
+        x, y, z = torch.meshgrid(ax, ax, ax, indexing="ij")
+        sigma = (1.0 + 4.0 * (0.6 - torch.sqrt(x * x + y * y + z * z))).float().contiguous()
+        del x, y, z
+        verts, faces = bm.extract(sigma, 1.0, 1.0)
+        med, best = timeit(lambda: bm.extract(sigma, 1.0, 1.0), n=10, warm=3)
+        _lib.PROFILER = _lib.Profiler()
+        for _ in range(10):
+            bm.extract(sigma, 1.0, 1.0)
+        torch.cuda.synchronize()
+        summ = _lib.PROFILER.summary()
+        _lib.PROFILER = None
+        split = ", ".join(f"{k[len('b2n_mesh_'):]} {v['ms'] / v['calls']:.3f} ms" for k, v in summ.items())
+        print(f"extract ball R={R}: {verts.shape[0]} vertices, {faces.shape[0]} triangles, median {med:.3f} ms "
+              f"(best {best:.3f}; {split}; the rest is the host read of the totals and the allocations)")
+        del sigma, verts, faces
+        torch.cuda.empty_cache()
+
+
 def c1_step(P_rays=4096, N=64):
     """C1: vanilla NeRF training step (render_rays + MSE + backward + Adam), B=4096, N=64."""
     from b2n import synthetic
@@ -519,6 +558,8 @@ if __name__ == "__main__":
         c1_step()
     elif what == "occ":
         occ_update()
+    elif what == "mesh":
+        mesh()
     elif what == "hashsort":
         hash_sorted()
     elif what == "hash":
