@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 16
+#define B2N_ABI_VERSION 17
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -241,23 +241,16 @@ int b2n_sigma_head_bwd(const float* h, int ldh, int64_t P, const float* g_sigma,
 /* in_pad_value: what the PADDED input columns of the two FullyFusedMLPs hold (pos_dim .. pad16(pos_dim) of sigma_net,
  * 16 + dir_dim .. pad16(16 + dir_dim) of color_net): 0 (this package, the oracle) or 1 (checkpoints of an upstream
  * tiny-cuda-nn whose Network pads its inputs with ones, which makes those weight columns a bias: b2n.checkpoint). */
-int b2n_instant_mlp_fwd(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
-                        int L_dir, const float* sigma_params, const float* color_params, int64_t P, float* rgb,
-                        float* sigma, float in_pad_value, b2n_stream_t stream);
-/* The same forward (same arguments, same fp16 split arithmetic) with the layer products on tcgen05: a CTA owns 128
- * points = the 128 TMEM lanes, activations round-trip TMEM -> registers -> shared memory between layers.  err_flag: a
- * device int the kernel sets non-zero if it had to abort a stalled mbarrier wait (outputs are then invalid); it is never
- * cleared by the kernel. */
+/* Forward: the layer products run on tcgen05; a CTA owns 128 points = the 128 TMEM lanes, activations round-trip
+ * TMEM -> registers -> shared memory between layers.  rgb == NULL computes sigma alone (dirs, dir_bands and
+ * color_params are then not read and may be NULL).  err_flag: a device int the kernel sets non-zero if it had to abort
+ * a stalled mbarrier wait (outputs are then invalid); it is never cleared by the kernel. */
 int b2n_instant_mlp_fwd_tc(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
                            int L_dir, const float* sigma_params, const float* color_params, int64_t P, float* rgb,
                            float* sigma, float in_pad_value, int* err_flag, b2n_stream_t stream);
-int b2n_instant_mlp_bwd(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
-                        int L_dir, const float* sigma_params, const float* color_params, int64_t P,
-                        const float* g_rgb, const float* g_sigma, float* g_x_enc, int ldg, float* g_sigma_params,
-                        float* g_color_params, void* work4, float in_pad_value, b2n_stream_t stream);
-/* The same backward (same arguments and arithmetic) with the five weight gradients dW = dZ^T In on tcgen05: the staged
- * 64-point tiles are MN-major SWIZZLE_128B operands, the fp32 accumulators live in TMEM for the whole persistent loop.
- * err_flag as in b2n_instant_mlp_fwd_tc. */
+/* Backward: the forward recompute and the data-gradient chain run on mma.sync, the five weight gradients dW = dZ^T In
+ * on tcgen05: the staged 64-point tiles are MN-major SWIZZLE_128B operands, the fp32 accumulators live in TMEM for the
+ * whole persistent loop.  err_flag as in b2n_instant_mlp_fwd_tc. */
 int b2n_instant_mlp_bwd_tc(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
                            int L_dir, const float* sigma_params, const float* color_params, int64_t P,
                            const float* g_rgb, const float* g_sigma, float* g_x_enc, int ldg, float* g_sigma_params,

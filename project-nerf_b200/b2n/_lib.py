@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb2nerf.so")
 
-ABI_VERSION = 16
+ABI_VERSION = 17
 
 P, L, I, F = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
 
@@ -48,9 +48,7 @@ SIGNATURES = {
     "b2n_act_bwd": [P, I, P, I, L, I, I, P],
     "b2n_sigma_head_fwd": [P, I, L, P, P],
     "b2n_sigma_head_bwd": [P, I, L, P, P, I, P],
-    "b2n_instant_mlp_fwd": [P, I, I, P, P, I, P, P, L, P, P, F, P],
     "b2n_instant_mlp_fwd_tc": [P, I, I, P, P, I, P, P, L, P, P, F, P, P],
-    "b2n_instant_mlp_bwd": [P, I, I, P, P, I, P, P, L, P, P, P, I, P, P, P, F, P],
     "b2n_instant_mlp_bwd_tc": [P, I, I, P, P, I, P, P, L, P, P, P, I, P, P, P, F, P, P],
     "b2n_fmlp_in_pad": [I],
     "b2n_fmlp_out_pad": [I],
@@ -120,7 +118,7 @@ lib = _load()
 # launch accounting for bench.py ("gpu_launches"): every successful C-ABI call adds the
 # number of kernels that entry point launches.
 LAUNCHES = {"count": 0}
-_KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_hash_order": 5, "b2n_mesh_count": 2, "b2n_mesh_emit": 2, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
+_KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_hash_order": 5, "b2n_mesh_count": 2, "b2n_mesh_emit": 2, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
 
 
 def ptr(t):

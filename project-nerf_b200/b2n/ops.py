@@ -17,12 +17,6 @@ from torch.amp import custom_bwd, custom_fwd
 from . import _lib
 from ._lib import HashLevelC, current_rows, ptr, require_cuda, stream, with_ctx_rows
 
-# forward of the fused Instant decoder: the tcgen05 kernel (b2n_mlp64tc.cu) or, when False, the mma.sync one
-# (b2n_mlp64.cu); same arithmetic (environment B2N_INSTANT_TC=0 selects the latter for A/B timing)
-import os as _os
-INSTANT_FWD_TC = _os.environ.get("B2N_INSTANT_TC", "1") != "0"
-# backward: weight gradients on tcgen05 (k_instant_bwd_tc) or, when False, everything on mma.sync (k_instant_bwd)
-INSTANT_BWD_TC = _os.environ.get("B2N_INSTANT_BWD_TC", "1") != "0"
 # hash_encode sorts its points into spatial order (b2n_hash_order) from this many points on, when the input needs no
 # gradient and the F = 2 pair-lane kernels run: measured to pay at C2's 24 M points; smaller sets are not sorted
 HASH_ORDER_MIN_POINTS = 1 << 23
@@ -456,13 +450,9 @@ class _InstantMLP(torch.autograd.Function):
         rgb = _narrow_out(Pn, 3, device=x_enc.device)
         sigma = _narrow_out(Pn, 1, device=x_enc.device)
         flops = 2.0 * Pn * (64 * pos_dim + 16 * 64 + 64 * 43 + 64 * 64 + 3 * 64)
-        if INSTANT_FWD_TC:
-            call("b2n_instant_mlp_fwd_tc", ptr(x_enc), pos_dim, pos_dim, ptr(dirs), ptr(bands), bands.numel(), ptr(sp),
-                 ptr(cp), Pn, ptr(rgb), ptr(sigma), ctx.pad_value, ptr(_sticky_err(x_enc.device)), stream(),
-                 work=(Pn * (4.0 * pos_dim + 12 + 16), flops))
-        else:
-            call("b2n_instant_mlp_fwd", ptr(x_enc), pos_dim, pos_dim, ptr(dirs), ptr(bands), bands.numel(), ptr(sp),
-                 ptr(cp), Pn, ptr(rgb), ptr(sigma), ctx.pad_value, stream(), work=(Pn * (4.0 * pos_dim + 12 + 16), flops))
+        call("b2n_instant_mlp_fwd_tc", ptr(x_enc), pos_dim, pos_dim, ptr(dirs), ptr(bands), bands.numel(), ptr(sp),
+             ptr(cp), Pn, ptr(rgb), ptr(sigma), ctx.pad_value, ptr(_sticky_err(x_enc.device)), stream(),
+             work=(Pn * (4.0 * pos_dim + 12 + 16), flops))
         ctx.save_for_backward(x_enc, dirs, bands, sp, cp)
         return rgb, sigma
 
@@ -476,22 +466,16 @@ class _InstantMLP(torch.autograd.Function):
         g_sp, g_cp = torch.zeros_like(sp), torch.zeros_like(cp)
         work = torch.empty(1, device=x_enc.device, dtype=torch.int32)        # |g|-max of the gradient pre-pass
         flops = 6.0 * Pn * (64 * pos_dim + 16 * 64 + 64 * 43 + 64 * 64 + 3 * 64)
-        if INSTANT_BWD_TC:
-            call("b2n_instant_mlp_bwd_tc", ptr(x_enc), pos_dim, pos_dim, ptr(dirs), ptr(bands), bands.numel(), ptr(sp),
-                 ptr(cp), Pn, ptr(_c(g_rgb)), ptr(_c(g_sigma)), ptr(g_x), pos_dim, ptr(g_sp), ptr(g_cp), ptr(work),
-                 ctx.pad_value, ptr(_sticky_err(x_enc.device)), stream(),
-                 work=(Pn * (8.0 * pos_dim + 12 + 16), flops))
-        else:
-            call("b2n_instant_mlp_bwd", ptr(x_enc), pos_dim, pos_dim, ptr(dirs), ptr(bands), bands.numel(), ptr(sp),
-                 ptr(cp), Pn, ptr(_c(g_rgb)), ptr(_c(g_sigma)), ptr(g_x), pos_dim, ptr(g_sp), ptr(g_cp), ptr(work),
-                 ctx.pad_value, stream(),
-                 work=(Pn * (8.0 * pos_dim + 12 + 16), flops))
+        call("b2n_instant_mlp_bwd_tc", ptr(x_enc), pos_dim, pos_dim, ptr(dirs), ptr(bands), bands.numel(), ptr(sp),
+             ptr(cp), Pn, ptr(_c(g_rgb)), ptr(_c(g_sigma)), ptr(g_x), pos_dim, ptr(g_sp), ptr(g_cp), ptr(work),
+             ctx.pad_value, ptr(_sticky_err(x_enc.device)), stream(),
+             work=(Pn * (8.0 * pos_dim + 12 + 16), flops))
         return g_x, None, None, g_sp, g_cp, None
 
 
 @torch.no_grad()
 def instant_sigma(x_enc, sigma_params, pad_value: float = 0.0):
-    """sigma [P,1] of the fused Instant decoder alone: b2n_instant_mlp_fwd with the colour network switched off (no view
+    """sigma [P,1] of the fused Instant decoder alone: b2n_instant_mlp_fwd_tc with the colour network switched off (no view
     directions, no colour layers).  Same sigma_net arithmetic as ``instant_mlp`` -- bit-identical sigma -- at ~40 % of its
     time; no gradient (occupancy sweeps: DensityGrid.update, SURVEY 8f-3)."""
     require_cuda(x_enc, sigma_params)
@@ -499,12 +483,8 @@ def instant_sigma(x_enc, sigma_params, pad_value: float = 0.0):
     Pn, pos_dim = x_enc.shape
     sigma = _narrow_out(Pn, 1, device=x_enc.device)
     work = (Pn * (4.0 * pos_dim + 4), 2.0 * Pn * (64 * pos_dim + 16 * 64))
-    if INSTANT_FWD_TC:
-        call("b2n_instant_mlp_fwd_tc", ptr(x_enc), pos_dim, pos_dim, None, None, 0, ptr(sp), None, Pn, None, ptr(sigma),
-             float(pad_value), ptr(_sticky_err(x_enc.device)), stream(), work=work)
-    else:
-        call("b2n_instant_mlp_fwd", ptr(x_enc), pos_dim, pos_dim, None, None, 0, ptr(sp), None, Pn, None, ptr(sigma),
-             float(pad_value), stream(), work=work)
+    call("b2n_instant_mlp_fwd_tc", ptr(x_enc), pos_dim, pos_dim, None, None, 0, ptr(sp), None, Pn, None, ptr(sigma),
+         float(pad_value), ptr(_sticky_err(x_enc.device)), stream(), work=work)
     return sigma
 
 

@@ -222,7 +222,7 @@ __device__ __forceinline__ void apply_gate(float (&c)[NT][4], const uint32_t (&g
 
 __device__ __forceinline__ float sigm(float v) { return 1.f / (1.f + expf(-v)); }
 
-// max |g_y| as float bits (see k_instant_bwd's pre-pass: same convention, NaN sorts above everything)
+// max |g_y| as float bits (see k_grad_absmax in b2n_mlp64.cu: same convention, NaN sorts above everything)
 __global__ void __launch_bounds__(256) k_fmlp_absmax(const float* __restrict__ g, int ld, int cols, int64_t P,
                                                      unsigned int* __restrict__ out, const int* __restrict__ rows) {
   P = clamp_rows(P, rows);

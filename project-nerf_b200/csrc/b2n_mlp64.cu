@@ -1,29 +1,22 @@
-// Fused 64-wide decoder of the hash-grid configs: InstantNeRFDecoder.forward
-// (src/decoders.py:136-162), i.e. the two tinycudann FullyFusedMLPs of the reference plus the
-// direction Fourier features (src/embeddings.py:22-32 on view dirs), the softplus(h0-5) density
-// head, the concat and the sigmoid -- one kernel forward, one kernel backward.
+// Backward of the fused 64-wide decoder of the hash-grid configs: InstantNeRFDecoder.forward (src/decoders.py:136-162),
+// i.e. the two tinycudann FullyFusedMLPs of the reference plus the direction Fourier features (src/embeddings.py:22-32 on
+// view dirs), the softplus(h0-5) density head, the concat and the sigmoid.  The forward is k_instant_fwd_tc
+// (b2n_mlp64tc.cu); the arithmetic both must compute identically is in b2n_mlp64.cuh.
 //
 //   sigma_net : x[pos] -> 64 (ReLU) -> 16            (no biases, widths padded to 16)
 //   sigma     = softplus(h[0] - 5)
 //   color_net : cat[h(16), gamma(d)(27 -> 32)] -> 64 (ReLU) -> 64 (ReLU) -> 3 (sigmoid)
 //
 // Arithmetic: IEEE fp16 operands (what the reference's tinycudann FullyFusedMLP uses), fp32 accumulation on the tensor
-// cores (mma.sync m16n8k16).  Two departures from plain fp16, both measured on the CPU error budget
+// cores.  Two departures from plain fp16, both measured on the CPU error budget
 // (tools/bf16_error_budget.py) as what decides the distance of the parameter gradients from an fp32 evaluation:
 //   * sigma_net's FIRST layer -- the product with the hash-grid features, whose pre-activations decide 64 ReLU masks and
 //     the density -- is a split product x_hi W_hi + x_lo W_hi + x_hi W_lo (x = x_hi + x_lo in fp16): ~21 significant bits;
 //   * the gradient chain runs on S * dL/dy with S a power of two that puts the largest incoming gradient at 2^7..2^8
-//     (found by a one-pass |.|-max reduction), so fp16's narrow exponent range never clips it; outputs are divided by S.
-// Activations never leave the SM:
-//   forward : each warp owns 32 points; layer outputs (C fragments) are re-packed in registers
-//             as the next layer's A fragments; weights are bf16 in shared memory (ldmatrix).
-//   backward: each warp owns 16 points of a 64-point block tile; the forward is recomputed, the
-//             data-gradient chain runs in registers (ldmatrix.trans on the same weights), every
-//             layer input / pre-activation gradient is staged once in shared memory as bf16 and
-//             the weight gradients dW = dZ^T * In are accumulated by tensor cores in registers
-//             over the whole persistent loop, then flushed with one atomicAdd per weight per CTA.
+//     (found by a one-pass |.|-max reduction, k_grad_absmax), so fp16's narrow exponent range never clips it; outputs are
+//     divided by S.
 #define B2N_OP_F16
-#include "b2n_mma.cuh"
+#include "b2n_mlp64.cuh"
 #include "b2n_tc.cuh"
 
 namespace b2n {
@@ -33,105 +26,14 @@ constexpr int GEO = 16;      // sigma_net output width
 constexpr int CIN = 48;      // color_net padded input width (16 + 27 -> 48)
 constexpr int MLP_THREADS = 128;
 
-
-// view-direction Fourier features of one point -> 32 bf16 (27 valid, zero padded) at dst
-// (load and use are split so that the load can be issued long before the features are needed: ncu showed
-// long-scoreboard stalls on the small per-tile loads as the top stall reason of both decoder kernels)
+// view direction of point p (zeros beyond P): loaded long before dir_features needs it (ncu showed long-scoreboard stalls
+// on the small per-tile loads as the top stall reason of the decoder kernels)
 __device__ __forceinline__ void load_dir(const float* __restrict__ dirs, int64_t p, int64_t P, float (&d)[3]) {
   d[0] = d[1] = d[2] = 0.f;
   if (dirs && p < P) d[0] = __ldg(dirs + 3 * p), d[1] = __ldg(dirs + 3 * p + 1), d[2] = __ldg(dirs + 3 * p + 2);
 }
-// chunk0 / xr: 16-byte chunk i of the 32 features goes to dst + 8 * ((chunk0 + i) ^ xr) -- the XOR-swizzled rows of the
-// tcgen05 operand tiles (k_instant_bwd_tc); 0 / 0 = contiguous
-__device__ __forceinline__ void dir_features(const float (&d)[3], const float* __restrict__ bands, int L, op16* dst,
-                                             float pad, int chunk0 = 0, int xr = 0) {
-  // columns [3 + 6 L, pad16(16 + 3 + 6 L) - 16) are the INPUT PADDING of color_net (43 -> 48 at L = 4): they hold `pad`
-  // (0, or 1 for checkpoints of an upstream build whose padded inputs are ones: b2n.checkpoint), the rest zeros
-  const int dd = 3 + 6 * L, dpad = ((16 + dd + 15) & ~15) - 16;
-  float f[32];
-#pragma unroll
-  for (int i = 0; i < 32; ++i) f[i] = (i >= dd && i < dpad) ? pad : 0.f;
-  f[0] = d[0], f[1] = d[1], f[2] = d[2];
-  // band k+1 = 2 * band k (the reference's 2^k bands): double-angle recurrence instead of a fresh
-  // sincosf (error grows ~2x per band from 1e-7: far below the bf16 rounding applied next)
-  float ps[3], pc[3], prev = 0.f;
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    if (k < L) {
-      const float fr = __ldg(bands + k);
-      const bool dbl = (k > 0) && (fr == 2.f * prev);
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        float s, c;
-        if (dbl) {
-          s = 2.f * ps[j] * pc[j];
-          c = 1.f - 2.f * ps[j] * ps[j];
-        } else {
-          // view directions are unit vectors and the first band is 1: |arg| <= pi, where the MUFU sin/cos (abs.
-          // error ~1e-6) is far inside the bf16 rounding applied below; larger arguments take the accurate path
-          const float arg = __fmul_rn(__fmul_rn(d[j], fr), 3.14159274101257324f);
-          // beyond +-pi (non-unit directions, custom bands): one fp32 reduction step to [-pi, pi] instead of libm's
-          // Payne-Hanek path (hundreds of instructions and local memory in a kernel whose code must stay cache-resident)
-          const float red = fabsf(arg) <= 3.2f ? arg : __fmaf_rn(-6.28318530717958648f, rintf(arg * 0.159154943091895336f), arg);
-          __sincosf(red, &s, &c);
-        }
-        ps[j] = s, pc[j] = c;
-        f[3 + 6 * k + j] = s;
-        f[3 + 6 * k + 3 + j] = c;
-      }
-      prev = fr;
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-    *reinterpret_cast<uint4*>(dst + 8 * ((chunk0 + i) ^ xr)) =
-        make_uint4(pack2(f[8 * i], f[8 * i + 1]), pack2(f[8 * i + 2], f[8 * i + 3]), pack2(f[8 * i + 4], f[8 * i + 5]),
-                   pack2(f[8 * i + 6], f[8 * i + 7]));
-}
-
-// A fragments of 16 rows of x_enc [P, pos_dim] fp32 (zero beyond pos_dim / P)
-template <int KT>
-__device__ __forceinline__ void load_x(const float* __restrict__ x, int ldx, int pos_dim, int64_t p0, int64_t P,
-                                       uint32_t (&a)[KT][4], int lane) {
-  const int g = lane >> 2, t = lane & 3;
-  const bool vec = ((ldx & 1) == 0) && ((reinterpret_cast<uintptr_t>(x) & 7) == 0);
-#pragma unroll
-  for (int k = 0; k < KT; ++k) {
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {      // h: column half (+0 / +8)
-#pragma unroll
-      for (int r = 0; r < 2; ++r) {    // r: row g / g + 8
-        const int64_t p = p0 + g + 8 * r;
-        const int c = 16 * k + 8 * h + 2 * t;
-        float v0 = 0.f, v1 = 0.f;
-        if (p < P) {
-          const float* src = x + p * ldx + c;
-          if (vec && c + 1 < pos_dim) {
-            const float2 v = __ldcs(reinterpret_cast<const float2*>(src));
-            v0 = v.x, v1 = v.y;
-          } else {
-            if (c < pos_dim) v0 = __ldcs(src);
-            if (c + 1 < pos_dim) v1 = __ldcs(src + 1);
-          }
-        }
-        a[k][2 * h + r] = pack2(v0, v1);
-      }
-    }
-  }
-}
-
-// pull the lines of a future tile towards L2 (no registers held): rows [p0, p0+rows) of x and dirs
-__device__ __forceinline__ void prefetch_rows(const float* __restrict__ x, int ldx, const float* __restrict__ dirs,
-                                              int64_t p0, int rows, int64_t P, int lane) {
-  if (lane < rows && p0 + lane < P) {
-    const char* a = reinterpret_cast<const char*>(x + (p0 + lane) * ldx);
-    asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
-    if (ldx > 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(a + 128));
-    if (dirs && (lane & 7) == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(reinterpret_cast<const char*>(dirs + 3 * (p0 + lane))));
-  }
-}
-
-// split version of load_x for software pipelining: issue the loads now, pack (and stall) later
+// A-fragment elements of 16 rows of x_enc [P, pos_dim] as fp32 pairs (`pad` in the input padding, zero beyond it and
+// beyond P), for software pipelining: issue the loads now, split into hi / lo (and stall) later
 template <int KT>
 __device__ __forceinline__ void load_x_raw(const float* __restrict__ x, int ldx, int pos_dim, int64_t p0, int64_t P,
                                            float2 (&raw)[KT][4], int lane, float pad = 0.f) {
@@ -175,14 +77,6 @@ __device__ __forceinline__ void load_x_raw_full(const float* __restrict__ x, int
       raw[k][2 * h + 1] = __ldcs(reinterpret_cast<const float2*>(r1 + 16 * k + 8 * h));
     }
 }
-template <int KT>
-__device__ __forceinline__ void pack_x(const float2 (&raw)[KT][4], uint32_t (&a)[KT][4]) {
-#pragma unroll
-  for (int k = 0; k < KT; ++k)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) a[k][i] = pack2(raw[k][i].x, raw[k][i].y);
-}
-
 // x = hi + lo with hi = fp16(x), lo = fp16(x - hi): the operands of the split first-layer product
 __device__ __forceinline__ void pack_hl(float v0, float v1, uint32_t& hi, uint32_t& lo) {
   hi = pack2(v0, v1);
@@ -196,17 +90,6 @@ __device__ __forceinline__ void pack_x_hl(const float2 (&raw)[KT][4], uint32_t (
 #pragma unroll
     for (int i = 0; i < 4; ++i) pack_hl(raw[k][i].x, raw[k][i].y, hi[k][i], lo[k][i]);
 }
-
-// softplus(h0 - 5) and the logistic function on the MUFU units (ex2 / lg2 / rcp: ~1e-6 relative, two orders below the fp16
-// operands around them) instead of libm's expf / log1pf and an IEEE division -- 110 of the ~1300 instructions a thread spent
-// per forward tile.  Small e = exp(v): the series of log1p (relative error < e^3 / 4 < 8e-6 below 1/32)
-__device__ __forceinline__ float softplus_m5(float h0) {
-  const float v = h0 - 5.0f;
-  const float e = __expf(fminf(v, 20.f));
-  const float sp = e < 0.03125f ? e * (1.f - e * (0.5f - e * 0.33333334f)) : __logf(1.f + e);
-  return v > 20.f ? v : sp;
-}
-__device__ __forceinline__ float sigmoidf(float v) { return __fdividef(1.f, 1.f + __expf(-v)); }
 
 struct MlpSmem {
   // offsets (in bf16 elements) of the weight matrices inside dynamic shared memory
@@ -244,191 +127,6 @@ __device__ __forceinline__ void load_all_weights(const float* __restrict__ sp, c
   load_weights(cp, HID, CIN, CIN, sm + L.v1);
   load_weights(cp + HID * CIN, HID, HID, HID, sm + L.v2);
   load_weights(cp + HID * CIN + HID * HID, 16, HID, HID, sm + L.v3);
-}
-
-// ------------------------------------------------------------------------------ forward
-template <int POS_K>
-__global__ void __launch_bounds__(MLP_THREADS, 2)
-k_instant_fwd(const float* __restrict__ x, int ldx, int pos_dim, const float* __restrict__ dirs,
-              const float* __restrict__ bands, int L_dir, const float* __restrict__ sp, const float* __restrict__ cp,
-              int64_t P, float* __restrict__ rgb, float* __restrict__ sigma, const int* __restrict__ rows,
-              float in_pad_value) {
-  P = clamp_rows(P, rows);
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  op16* sm = reinterpret_cast<op16*>(smem_raw);
-  constexpr MlpSmem L = weight_layout<POS_K>();
-  constexpr int KT1 = POS_K / 16;
-  constexpr int DS = 32 + PAD;                 // direction-feature staging row stride
-  op16* dstage = sm + L.end + (threadIdx.x >> 5) * 32 * DS;
-  const int in_pad = (pos_dim + 15) & ~15;
-  load_all_weights<POS_K>(sp, cp, in_pad, sm);
-  __syncthreads();
-  const int lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-  const int64_t n_tiles = (P + 31) / 32;
-  const int64_t wstride = (int64_t)gridDim.x * (MLP_THREADS / 32);
-  // POS_K == 32: the next tile's inputs (x_enc rows, view direction) are fetched into registers one tile ahead,
-  // right after the current ones have been packed, and land during the ~10 us of layer work; the 64-wide
-  // variant (Part 3/4: pos_dim 53) has no registers to spare and only pulls the lines towards L2
-  constexpr bool PF = (POS_K == 32);
-  constexpr int KTP = PF ? KT1 : 1;
-  float2 xraw[2][KTP][4];
-  float dnext[3] = {0.f, 0.f, 0.f};
-  const int64_t tile0 = (int64_t)blockIdx.x * (MLP_THREADS / 32) + (threadIdx.x >> 5);
-  if (PF) {
-    load_x_raw<KTP>(x, ldx, pos_dim, tile0 * 32, P, xraw[0], lane, in_pad_value);
-    load_x_raw<KTP>(x, ldx, pos_dim, tile0 * 32 + 16, P, xraw[1], lane, in_pad_value);
-    load_dir(dirs, tile0 * 32 + lane, P, dnext);
-  }
-  for (int64_t tile = tile0; tile < n_tiles; tile += wstride) {
-    const int64_t p0 = tile * 32;
-    uint32_t ax[2][KT1][4], axl[2][KT1][4];
-    float dcur[3];
-    if (PF) {
-#pragma unroll
-      for (int m = 0; m < 2; ++m)
-#pragma unroll
-        for (int k = 0; k < KT1; ++k)
-#pragma unroll
-          for (int i = 0; i < 4; ++i) pack_hl(xraw[m][k % KTP][i].x, xraw[m][k % KTP][i].y, ax[m][k][i], axl[m][k][i]);
-      dcur[0] = dnext[0], dcur[1] = dnext[1], dcur[2] = dnext[2];
-      const int64_t pn = (tile + wstride) * 32;
-      load_x_raw<KTP>(x, ldx, pos_dim, pn, P, xraw[0], lane, in_pad_value);
-      load_x_raw<KTP>(x, ldx, pos_dim, pn + 16, P, xraw[1], lane, in_pad_value);
-      load_dir(dirs, pn + lane, P, dnext);
-    } else {
-      prefetch_rows(x, ldx, dirs, (tile + wstride) * 32, 32, P, lane);
-      load_dir(dirs, p0 + lane, P, dcur);
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-        float2 raw[KT1][4];
-        load_x_raw<KT1>(x, ldx, pos_dim, p0 + 16 * m, P, raw, lane, in_pad_value);
-        pack_x_hl<KT1>(raw, ax[m], axl[m]);
-      }
-    }
-    // sigma_net layer 1
-    uint32_t ah[2][4][4];
-    {
-      float c[2][8][4] = {};
-      gemm_fwd<2, 8, KT1>(c, axl, sm + L.w1, POS_K + PAD, lane);          // split product: the small terms first
-      gemm_fwd<2, 8, KT1>(c, ax, sm + L.w1lo, POS_K + PAD, lane);
-      gemm_fwd<2, 8, KT1>(c, ax, sm + L.w1, POS_K + PAD, lane);
-      c_to_a<8, true>(c[0], ah[0]);
-      c_to_a<8, true>(c[1], ah[1]);
-    }
-    // sigma_net layer 2 -> h (16 wide), density head
-    uint32_t ac[2][3][4];
-    {
-      float c[2][2][4] = {};
-      gemm_fwd<2, 2, 4>(c, ah, sm + L.w2, HID + PAD, lane);
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-        if (t == 0) {
-          const int64_t pa = p0 + 16 * m + g, pb = pa + 8;
-          if (pa < P) __stcs(sigma + pa, softplus_m5(c[m][0][0]));
-          if (pb < P) __stcs(sigma + pb, softplus_m5(c[m][0][2]));
-        }
-        uint32_t tmp[1][4];
-        c_to_a<2, false>(c[m], tmp);
-        ac[m][0][0] = tmp[0][0], ac[m][0][1] = tmp[0][1], ac[m][0][2] = tmp[0][2], ac[m][0][3] = tmp[0][3];
-      }
-    }
-    if (!rgb) continue;      // density sweep (DensityGrid.update, SURVEY 8f-3): sigma is out, the colour network is skipped
-    dir_features(dcur, bands, L_dir, dstage + lane * DS, in_pad_value);     // needed only now: the direction load had two layers to land
-    __syncwarp();
-#pragma unroll
-    for (int m = 0; m < 2; ++m) {
-      ldsm_x4(ac[m][1], dstage + (16 * m + (lane & 7) + 8 * ((lane >> 3) & 1)) * DS + 8 * (lane >> 4));
-      ldsm_x4(ac[m][2], dstage + (16 * m + (lane & 7) + 8 * ((lane >> 3) & 1)) * DS + 16 + 8 * (lane >> 4));
-    }
-    __syncwarp();
-    // color_net
-    uint32_t a1[2][4][4];
-    {
-      float c[2][8][4] = {};
-      gemm_fwd<2, 8, 3>(c, ac, sm + L.v1, CIN + PAD, lane);
-      c_to_a<8, true>(c[0], a1[0]);
-      c_to_a<8, true>(c[1], a1[1]);
-    }
-    {
-      float c[2][8][4] = {};
-      gemm_fwd<2, 8, 4>(c, a1, sm + L.v2, HID + PAD, lane);
-      c_to_a<8, true>(c[0], ah[0]);
-      c_to_a<8, true>(c[1], ah[1]);
-    }
-    {
-      float c[2][1][4] = {};
-      gemm_fwd<2, 1, 4>(c, ah, sm + L.v3, HID + PAD, lane);
-#pragma unroll
-      for (int m = 0; m < 2; ++m) {
-        const int64_t pa = p0 + 16 * m + g, pb = pa + 8;
-        const int col = 2 * t;
-        if (col < 3) {
-          if (pa < P) {
-            rgb[3 * pa + col] = sigmoidf(c[m][0][0]);
-            if (col + 1 < 3) rgb[3 * pa + col + 1] = sigmoidf(c[m][0][1]);
-          }
-          if (pb < P) {
-            rgb[3 * pb + col] = sigmoidf(c[m][0][2]);
-            if (col + 1 < 3) rgb[3 * pb + col + 1] = sigmoidf(c[m][0][3]);
-          }
-        }
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------ backward
-template <int POS_K>
-struct BwdLayout {
-  static constexpr MlpSmem W = weight_layout<POS_K>();
-  static constexpr int SX = POS_K + PAD, SH = HID + PAD, SC = CIN + PAD, SG = 16 + PAD;
-  // staged layer inputs (64 points each)
-  static constexpr int in_x = W.end;
-  static constexpr int in_h1 = in_x + 64 * SX;
-  static constexpr int in_c = in_h1 + 64 * SH;
-  static constexpr int in_c1 = in_c + 64 * SC;
-  static constexpr int in_c2 = in_c1 + 64 * SH;
-  // staged pre-activation gradients
-  static constexpr int dz1 = in_c2 + 64 * SH;
-  static constexpr int dz2 = dz1 + 64 * SH;
-  static constexpr int dz3 = dz2 + 64 * SG;
-  static constexpr int dz4 = dz3 + 64 * SH;
-  static constexpr int dz5 = dz4 + 64 * SH;
-  static constexpr int end = dz5 + 64 * SG;
-};
-
-// ReLU mask from the staged activation tile (the thread re-reads exactly what it wrote)
-template <int NT>
-__device__ __forceinline__ void relu_mask(float (&c)[NT][4], const op16* tile, int S, int row0, int lane) {
-  const int g = lane >> 2, t = lane & 3;
-#pragma unroll
-  for (int j = 0; j < NT; ++j) {
-    const float2 lo = unpack2(*reinterpret_cast<const uint32_t*>(tile + (row0 + g) * S + 8 * j + 2 * t));
-    const float2 hi = unpack2(*reinterpret_cast<const uint32_t*>(tile + (row0 + g + 8) * S + 8 * j + 2 * t));
-    if (!(lo.x > 0.f)) c[j][0] = 0.f;
-    if (!(lo.y > 0.f)) c[j][1] = 0.f;
-    if (!(hi.x > 0.f)) c[j][2] = 0.f;
-    if (!(hi.y > 0.f)) c[j][3] = 0.f;
-  }
-}
-
-template <int NTk>
-__device__ __forceinline__ void flush_acc(const float (&acc)[NTk][4], float* __restrict__ gW, int ldw, int n0, int k0,
-                                          int n_valid, int lane, float inv_s) {
-  const int g = lane >> 2, t = lane & 3;
-#pragma unroll
-  for (int j = 0; j < NTk; ++j) {
-    const int k = k0 + 8 * j + 2 * t;
-    if (k >= ldw) continue;  // columns beyond the stored (padded) input width
-    if (n0 + g < n_valid) {
-      atomicAdd(gW + (size_t)(n0 + g) * ldw + k, acc[j][0] * inv_s);
-      atomicAdd(gW + (size_t)(n0 + g) * ldw + k + 1, acc[j][1] * inv_s);
-    }
-    if (n0 + g + 8 < n_valid) {
-      atomicAdd(gW + (size_t)(n0 + g + 8) * ldw + k, acc[j][2] * inv_s);
-      atomicAdd(gW + (size_t)(n0 + g + 8) * ldw + k + 1, acc[j][3] * inv_s);
-    }
-  }
 }
 
 // max |g| over the incoming gradients as float bits (non-negative floats order like unsigned integers; a NaN has the
@@ -471,216 +169,11 @@ __device__ __forceinline__ float grad_scale_from(unsigned int bits) {
   return __uint_as_float((unsigned int)(se + 127) << 23);
 }
 
-template <int POS_K>
-__global__ void __launch_bounds__(MLP_THREADS)
-k_instant_bwd(const float* __restrict__ x, int ldx, int pos_dim, const float* __restrict__ dirs,
-              const float* __restrict__ bands, int L_dir, const float* __restrict__ sp, const float* __restrict__ cp,
-              int64_t P, const float* __restrict__ g_rgb, const float* __restrict__ g_sigma, float* __restrict__ g_x,
-              int ldg, float* __restrict__ g_sp, float* __restrict__ g_cp, const unsigned int* __restrict__ absmax,
-              const int* __restrict__ rows, float in_pad_value) {
-  P = clamp_rows(P, rows);
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const float gscale = grad_scale_from(__ldg(absmax));
-  const float inv_s = 1.f / gscale;
-  op16* sm = reinterpret_cast<op16*>(smem_raw);
-  using LY = BwdLayout<POS_K>;
-  constexpr MlpSmem L = LY::W;
-  constexpr int KT1 = POS_K / 16;
-  const int in_pad = (pos_dim + 15) & ~15;
-  load_all_weights<POS_K>(sp, cp, in_pad, sm);
-  __syncthreads();
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, g = lane >> 2, t = lane & 3;
-  const int row0 = 16 * warp;  // this warp's slab inside the 64-point tile
-
-  // persistent weight-gradient accumulators (this warp's share of every matrix)
-  float acc1[POS_K / 8][4] = {};  // dW1 rows 16*warp.., all POS_K columns
-  float acc2[2][4] = {};          // dW2 (16 x 64): columns 16*warp..
-  float acc3[6][4] = {};          // dV1 rows 16*warp.., 48 columns
-  float acc4[8][4] = {};          // dV2 rows 16*warp.., 64 columns
-  float acc5[2][4] = {};          // dV3 (16 x 64, 3 valid rows): columns 16*warp..
-
-  const int64_t n_tiles = (P + 63) / 64;
-  float2 xraw[KT1][4];       // this tile's x_enc rows as fp32: fetched one tile ahead, split into hi / lo at the top of the tile
-  load_x_raw<KT1>(x, ldx, pos_dim, (int64_t)blockIdx.x * 64 + row0, P, xraw, lane, in_pad_value);
-  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const int64_t p0 = tile * 64 + row0;
-    // ---------------- forward recompute (staging every layer input)
-    uint32_t ax[1][KT1][4], axl[1][KT1][4];
-    pack_x_hl<KT1>(xraw, ax[0], axl[0]);
-    store_a<KT1>(ax[0], sm + LY::in_x, LY::SX, row0, 0, lane);
-    // small per-tile loads issued now, consumed several layers later (view direction -> colour net input,
-    // incoming gradients -> output layer / density head)
-    float dcur[3];
-    load_dir(dirs, p0 + (lane & 15), P, dcur);
-    float grgb[4] = {0.f, 0.f, 0.f, 0.f}, gsig[2] = {0.f, 0.f};
-    {
-      const int64_t pa = p0 + g, pb = pa + 8;
-      const int col = 2 * t;
-      if (col < 3) {
-        if (pa < P) {
-          grgb[0] = __ldcs(g_rgb + 3 * pa + col);
-          if (col + 1 < 3) grgb[1] = __ldcs(g_rgb + 3 * pa + col + 1);
-        }
-        if (pb < P) {
-          grgb[2] = __ldcs(g_rgb + 3 * pb + col);
-          if (col + 1 < 3) grgb[3] = __ldcs(g_rgb + 3 * pb + col + 1);
-        }
-      }
-      if (t == 0) {
-        if (pa < P) gsig[0] = __ldcs(g_sigma + pa);
-        if (pb < P) gsig[1] = __ldcs(g_sigma + pb);
-      }
-#pragma unroll
-      for (int i = 0; i < 4; ++i) grgb[i] *= gscale;      // the whole gradient chain runs on S * dL/dy
-      gsig[0] *= gscale, gsig[1] *= gscale;
-    }
-    uint32_t ah[1][4][4];
-    {
-      float c[1][8][4] = {};
-      gemm_fwd<1, 8, KT1>(c, axl, sm + L.w1, LY::SX, lane);              // split product (see k_instant_fwd)
-      gemm_fwd<1, 8, KT1>(c, ax, sm + L.w1lo, LY::SX, lane);
-      gemm_fwd<1, 8, KT1>(c, ax, sm + L.w1, LY::SX, lane);
-      c_to_a<8, true>(c[0], ah[0]);
-      store_a<4>(ah[0], sm + LY::in_h1, LY::SH, row0, 0, lane);
-    }
-    // next tile's inputs: the fragments are dead from here on, so the global loads are issued now and have the whole
-    // rest of the tile to land (ncu: the first use of a prefetch issued only before the wgrad phase was the hottest stall)
-    load_x_raw<KT1>(x, ldx, pos_dim, (tile + gridDim.x) * 64 + row0, P, xraw, lane, in_pad_value);
-    float hs0 = 0.f, hs1 = 0.f;  // h[.,0] of rows g and g+8 (threads with t == 0)
-    uint32_t ac[1][3][4];
-    {
-      float c[1][2][4] = {};
-      gemm_fwd<1, 2, 4>(c, ah, sm + L.w2, LY::SH, lane);
-      hs0 = c[0][0][0], hs1 = c[0][0][2];
-      uint32_t tmp[1][4];
-      c_to_a<2, false>(c[0], tmp);
-      ac[0][0][0] = tmp[0][0], ac[0][0][1] = tmp[0][1], ac[0][0][2] = tmp[0][2], ac[0][0][3] = tmp[0][3];
-      store_a<1>(tmp, sm + LY::in_c, LY::SC, row0, 0, lane);
-    }
-    if (lane < 16) dir_features(dcur, bands, L_dir, sm + LY::in_c + (row0 + lane) * LY::SC + 16, in_pad_value);
-    __syncwarp();
-    ldsm_x4(ac[0][1], sm + LY::in_c + (row0 + (lane & 7) + 8 * ((lane >> 3) & 1)) * LY::SC + 16 + 8 * (lane >> 4));
-    ldsm_x4(ac[0][2], sm + LY::in_c + (row0 + (lane & 7) + 8 * ((lane >> 3) & 1)) * LY::SC + 32 + 8 * (lane >> 4));
-    uint32_t a1[1][4][4], a2[1][4][4];
-    {
-      float c[1][8][4] = {};
-      gemm_fwd<1, 8, 3>(c, ac, sm + L.v1, LY::SC, lane);
-      c_to_a<8, true>(c[0], a1[0]);
-      store_a<4>(a1[0], sm + LY::in_c1, LY::SH, row0, 0, lane);
-    }
-    {
-      float c[1][8][4] = {};
-      gemm_fwd<1, 8, 4>(c, a1, sm + L.v2, LY::SH, lane);
-      c_to_a<8, true>(c[0], a2[0]);
-      store_a<4>(a2[0], sm + LY::in_c2, LY::SH, row0, 0, lane);
-    }
-    // ---------------- output layer + its gradient
-    uint32_t dz5[1][4];
-    {
-      float c[1][1][4] = {};
-      gemm_fwd<1, 1, 4>(c, a2, sm + L.v3, LY::SH, lane);
-      float d[4] = {0.f, 0.f, 0.f, 0.f};
-      const int64_t pa = p0 + g, pb = pa + 8;
-      const int col = 2 * t;
-      if (col < 3) {
-        if (pa < P) {
-          const float y = sigmoidf(c[0][0][0]);
-          d[0] = grgb[0] * y * (1.f - y);
-          if (col + 1 < 3) {
-            const float y1 = sigmoidf(c[0][0][1]);
-            d[1] = grgb[1] * y1 * (1.f - y1);
-          }
-        }
-        if (pb < P) {
-          const float y = sigmoidf(c[0][0][2]);
-          d[2] = grgb[2] * y * (1.f - y);
-          if (col + 1 < 3) {
-            const float y1 = sigmoidf(c[0][0][3]);
-            d[3] = grgb[3] * y1 * (1.f - y1);
-          }
-        }
-      }
-      dz5[0][0] = pack2(d[0], d[1]), dz5[0][1] = pack2(d[2], d[3]), dz5[0][2] = 0u, dz5[0][3] = 0u;
-      store_a<1>(dz5, sm + LY::dz5, LY::SG, row0, 0, lane);
-    }
-    // ---------------- data-gradient chain
-    uint32_t dz[1][4][4];
-    {
-      float c[8][4] = {};
-      gemm_dgrad<8, 1>(c, dz5, sm + L.v3, LY::SH, lane);          // d c2
-      relu_mask<8>(c, sm + LY::in_c2, LY::SH, row0, lane);
-      c_to_a<8, false>(c, dz[0]);
-      store_a<4>(dz[0], sm + LY::dz4, LY::SH, row0, 0, lane);
-    }
-    {
-      float c[8][4] = {};
-      gemm_dgrad<8, 4>(c, dz[0], sm + L.v2, LY::SH, lane);        // d c1
-      relu_mask<8>(c, sm + LY::in_c1, LY::SH, row0, lane);
-      c_to_a<8, false>(c, dz[0]);
-      store_a<4>(dz[0], sm + LY::dz3, LY::SH, row0, 0, lane);
-    }
-    uint32_t dz2[1][4];
-    {
-      float c[2][4] = {};
-      gemm_dgrad<2, 4>(c, dz[0], sm + L.v1, LY::SC, lane);        // d h (first 16 inputs of color_net)
-      if (t == 0) {                                               // density head: softplus'(h0 - 5)
-        const int64_t pa = p0 + g, pb = pa + 8;
-        if (pa < P) {
-          const float v = hs0 - 5.f;
-          c[0][0] += gsig[0] * (v > 20.f ? 1.f : sigmoidf(v));
-        }
-        if (pb < P) {
-          const float v = hs1 - 5.f;
-          c[0][2] += gsig[1] * (v > 20.f ? 1.f : sigmoidf(v));
-        }
-      }
-      c_to_a<2, false>(c, dz2);
-      store_a<1>(dz2, sm + LY::dz2, LY::SG, row0, 0, lane);
-    }
-    {
-      float c[8][4] = {};
-      gemm_dgrad<8, 1>(c, dz2, sm + L.w2, LY::SH, lane);          // d hidden1
-      relu_mask<8>(c, sm + LY::in_h1, LY::SH, row0, lane);
-      c_to_a<8, false>(c, dz[0]);
-      store_a<4>(dz[0], sm + LY::dz1, LY::SH, row0, 0, lane);
-    }
-    if (g_x) {
-      float c[POS_K / 8][4] = {};
-      gemm_dgrad<POS_K / 8, 4>(c, dz[0], sm + L.w1, LY::SX, lane);  // d x_enc
-      const int64_t pa = p0 + g, pb = pa + 8;
-#pragma unroll
-      for (int j = 0; j < POS_K / 8; ++j) {
-        const int col = 8 * j + 2 * t;
-        if (pa < P) {
-          if (col < pos_dim) g_x[pa * ldg + col] = c[j][0] * inv_s;
-          if (col + 1 < pos_dim) g_x[pa * ldg + col + 1] = c[j][1] * inv_s;
-        }
-        if (pb < P) {
-          if (col < pos_dim) g_x[pb * ldg + col] = c[j][2] * inv_s;
-          if (col + 1 < pos_dim) g_x[pb * ldg + col + 1] = c[j][3] * inv_s;
-        }
-      }
-    }
-    __syncthreads();
-    // ---------------- weight gradients over the 64 staged points
-    wgrad_tile<POS_K / 8>(acc1, sm + LY::dz1, LY::SH, 16 * warp, sm + LY::in_x, LY::SX, 0, lane);
-    wgrad_tile<2>(acc2, sm + LY::dz2, LY::SG, 0, sm + LY::in_h1, LY::SH, 16 * warp, lane);
-    wgrad_tile<6>(acc3, sm + LY::dz3, LY::SH, 16 * warp, sm + LY::in_c, LY::SC, 0, lane);
-    wgrad_tile<8>(acc4, sm + LY::dz4, LY::SH, 16 * warp, sm + LY::in_c1, LY::SH, 0, lane);
-    wgrad_tile<2>(acc5, sm + LY::dz5, LY::SG, 0, sm + LY::in_c2, LY::SH, 16 * warp, lane);
-    __syncthreads();
-  }
-  // ---------------- flush: one atomicAdd per weight per CTA
-  flush_acc<POS_K / 8>(acc1, g_sp, in_pad, 16 * warp, 0, HID, lane, inv_s);
-  flush_acc<2>(acc2, g_sp + HID * in_pad, HID, 0, 16 * warp, GEO, lane, inv_s);
-  flush_acc<6>(acc3, g_cp, CIN, 16 * warp, 0, HID, lane, inv_s);
-  flush_acc<8>(acc4, g_cp + HID * CIN, HID, 16 * warp, 0, HID, lane, inv_s);
-  flush_acc<2>(acc5, g_cp + HID * CIN + HID * HID, HID, 0, 16 * warp, 3, lane, inv_s);
-}
-
 // ------------------------------------------------------------------------------ backward, weight gradients on tcgen05
-// Same recompute + data-gradient chain as k_instant_bwd (mma.sync, a warp owns 16 points of a 64-point tile), but the
-// five weight gradients dW = dZ^T In -- a third of the kernel's tensor work, the part that needs BOTH operands from
+// A warp owns 16 points of a 64-point tile.  It recomputes the forward (split first layer) and runs the data-gradient
+// chain on mma.sync: activations and gradients as fragments in registers, weights in padded shared-memory rows read with
+// ldmatrix / ldmatrix.trans.  Every layer input and pre-activation gradient is staged in shared memory, and the five
+// weight gradients dW = dZ^T In -- a third of the kernel's tensor work, the part that would need BOTH operands from
 // shared memory through ldmatrix.trans, and 88 accumulator registers per thread -- go to the 5th-generation tensor cores:
 // the staged tiles are written in the SWIZZLE_128B layout (64 points x 128 B, 16-byte chunk c of row r at c ^ (r & 7)),
 // which read with the point as the contraction index is exactly tcgen05's MN-major operand form (b2n_wgrad256.cu), and
@@ -914,7 +407,12 @@ k_instant_bwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
         ac[0][0][0] = tmp[0][0], ac[0][0][1] = tmp[0][1], ac[0][0][2] = tmp[0][2], ac[0][0][3] = tmp[0][3];
         store_a_sw<1>(tmp, T(SL::C), row0, 0, lane);
       }
-      if (lane < 16) dir_features(dcur, bands, L_dir, T(SL::C) + (row0 + lane) * 64, in_pad_value, 2, (row0 + lane) & 7);
+      if (lane < 16) {             // chunks 2..5 (columns 16..47) of swizzled row row0 + lane: the colour net's direction input
+        op16* row = T(SL::C) + (row0 + lane) * 64;
+        const int xr = (row0 + lane) & 7;
+        dir_features(dcur, bands, L_dir, in_pad_value,
+                     [&](int i, uint4 v) { *reinterpret_cast<uint4*>(row + 8 * ((2 + i) ^ xr)) = v; });
+      }
       __syncwarp();
       {
         const int r = row0 + (lane & 7) + 8 * ((lane >> 3) & 1);
@@ -1093,25 +591,6 @@ k_instant_bwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
   if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
 }
 
-template <int POS_K>
-constexpr size_t fwd_smem_bytes() {
-  return (size_t)(weight_layout<POS_K>().end + (MLP_THREADS / 32) * 32 * (32 + PAD)) * sizeof(op16);
-}
-template <int POS_K>
-constexpr size_t bwd_smem_bytes() {
-  return (size_t)BwdLayout<POS_K>::end * sizeof(op16);
-}
-
-static int persistent_grid(const void* kernel, int threads, size_t smem, int64_t work_tiles) {
-  int per_sm = 1;
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem);
-  if (per_sm < 1) per_sm = 1;
-  int64_t g = (int64_t)kSMs * per_sm;
-  if (g > work_tiles) g = work_tiles;
-  if (g < 1) g = 1;
-  return (int)g;
-}
-
 }  // namespace b2n
 
 using namespace b2n;
@@ -1124,78 +603,10 @@ static int check_mlp_args(const float* x, int ldx, int pos_dim, const float* dir
   return B2N_OK;
 }
 
-extern "C" int b2n_instant_mlp_fwd(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
-                                   int L_dir, const float* sigma_params, const float* color_params, int64_t P,
-                                   float* rgb, float* sigma, float in_pad_value, b2n_stream_t stream) {
-  B2N_REQUIRE(P >= 0, "negative size");
-  if (P == 0) return B2N_OK;
-  // rgb == NULL: density only -- dirs / dir_bands / color_params are not read and may be NULL
-  int rc = rgb ? check_mlp_args(x_enc, ldx, pos_dim, dirs, dir_bands, L_dir, sigma_params, color_params)
-               : check_mlp_args(x_enc, ldx, pos_dim, x_enc, nullptr, 0, sigma_params, sigma_params);
-  if (rc) return rc;
-  if (!rgb) dirs = nullptr, dir_bands = nullptr, L_dir = 0, color_params = nullptr;
-  B2N_REQUIRE(sigma, "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int64_t warp_tiles = (P + 31) / 32;
-  const int64_t block_tiles = (warp_tiles + 3) / 4;
-  if (pos_dim <= 32) {
-    constexpr size_t smem = fwd_smem_bytes<32>();
-    cudaFuncSetAttribute(k_instant_fwd<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    const int grid = persistent_grid((const void*)k_instant_fwd<32>, MLP_THREADS, smem, block_tiles);
-    k_instant_fwd<32><<<grid, MLP_THREADS, smem, st>>>(x_enc, ldx, pos_dim, dirs, dir_bands, L_dir, sigma_params,
-                                                       color_params, P, rgb, sigma, g_active_rows, in_pad_value);
-  } else {
-    constexpr size_t smem = fwd_smem_bytes<64>();
-    cudaFuncSetAttribute(k_instant_fwd<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    const int grid = persistent_grid((const void*)k_instant_fwd<64>, MLP_THREADS, smem, block_tiles);
-    k_instant_fwd<64><<<grid, MLP_THREADS, smem, st>>>(x_enc, ldx, pos_dim, dirs, dir_bands, L_dir, sigma_params,
-                                                       color_params, P, rgb, sigma, g_active_rows, in_pad_value);
-  }
-  return check_launch("b2n_instant_mlp_fwd");
-}
-
-extern "C" int b2n_instant_mlp_bwd(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
-                                   int L_dir, const float* sigma_params, const float* color_params, int64_t P,
-                                   const float* g_rgb, const float* g_sigma, float* g_x_enc, int ldg,
-                                   float* g_sigma_params, float* g_color_params, void* work4, float in_pad_value,
-                                   b2n_stream_t stream) {
-  B2N_REQUIRE(P >= 0, "negative size");
-  if (P == 0) return B2N_OK;
-  int rc = check_mlp_args(x_enc, ldx, pos_dim, dirs, dir_bands, L_dir, sigma_params, color_params);
-  if (rc) return rc;
-  B2N_REQUIRE(g_rgb && g_sigma && g_sigma_params && g_color_params && work4, "null pointer");
-  B2N_REQUIRE(!g_x_enc || ldg >= pos_dim, "gradient row too narrow");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int64_t tiles = (P + 63) / 64;
-  unsigned int* absmax = (unsigned int*)work4;
-  if (cudaMemsetAsync(absmax, 0, 4, st) != cudaSuccess) return check_launch("b2n_instant_mlp_bwd (memset)");
-  {
-    const int64_t n = 4 * P;
-    const unsigned grid = (unsigned)((n + 1023) / 1024 < (int64_t)kSMs * 8 ? (n + 1023) / 1024 : (int64_t)kSMs * 8);
-    k_grad_absmax<<<grid, 256, 0, st>>>(g_rgb, g_sigma, P, absmax, g_active_rows);
-  }
-  if (pos_dim <= 32) {
-    constexpr size_t smem = bwd_smem_bytes<32>();
-    cudaFuncSetAttribute(k_instant_bwd<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    const int grid = persistent_grid((const void*)k_instant_bwd<32>, MLP_THREADS, smem, tiles);
-    k_instant_bwd<32><<<grid, MLP_THREADS, smem, st>>>(x_enc, ldx, pos_dim, dirs, dir_bands, L_dir, sigma_params,
-                                                       color_params, P, g_rgb, g_sigma, g_x_enc, ldg, g_sigma_params,
-                                                       g_color_params, absmax, g_active_rows, in_pad_value);
-  } else {
-    constexpr size_t smem = bwd_smem_bytes<64>();
-    cudaFuncSetAttribute(k_instant_bwd<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    const int grid = persistent_grid((const void*)k_instant_bwd<64>, MLP_THREADS, smem, tiles);
-    k_instant_bwd<64><<<grid, MLP_THREADS, smem, st>>>(x_enc, ldx, pos_dim, dirs, dir_bands, L_dir, sigma_params,
-                                                       color_params, P, g_rgb, g_sigma, g_x_enc, ldg, g_sigma_params,
-                                                       g_color_params, absmax, g_active_rows, in_pad_value);
-  }
-  return check_launch("b2n_instant_mlp_bwd");
-}
-
 // groups per CTA of k_instant_bwd_tc at pos_dim <= 32: 3 (default: one CTA per SM with 12 worker warps + the issuer) or
-// 1 (two 4-warp CTAs per SM).  Measured at 4.2 M points (tools/kbench.py mlp64): 1.37 ms against 1.44 ms, the mma.sync
-// kernel 1.70 ms.  The 12-warp schedule only paid off once the d x_enc stores were vectorised (the LSU was the shared
-// limit: 1.55 ms both before); ncu: `wait` (fixed-latency dependencies) is the top stall of both schedules
+// 1 (two 4-warp CTAs per SM).  Measured at 4.2 M points (tools/kbench.py mlp64): 1.37 ms against 1.44 ms (a former
+// all-mma.sync backward: 1.70 ms).  The 12-warp schedule only paid off once the d x_enc stores were vectorised (the LSU
+// was the shared limit: 1.55 ms both before); ncu: `wait` (fixed-latency dependencies) is the top stall of both schedules
 static int g_bwd_groups = 3;
 extern "C" int b2n_debug_instant_bwd_groups(int groups) {
   const int prev = g_bwd_groups;
@@ -1203,7 +614,7 @@ extern "C" int b2n_debug_instant_bwd_groups(int groups) {
   return prev;
 }
 
-// The same backward with the weight gradients on tcgen05 (k_instant_bwd_tc); err_flag as in b2n_instant_mlp_fwd_tc.
+// |g|-max pre-pass + k_instant_bwd_tc; err_flag as in b2n_instant_mlp_fwd_tc.
 extern "C" int b2n_instant_mlp_bwd_tc(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
                                       int L_dir, const float* sigma_params, const float* color_params, int64_t P,
                                       const float* g_rgb, const float* g_sigma, float* g_x_enc, int ldg,

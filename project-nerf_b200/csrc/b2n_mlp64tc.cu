@@ -1,9 +1,9 @@
-// Fused 64-wide Instant decoder on tcgen05 (forward): the same network and arithmetic as k_instant_fwd (b2n_mlp64.cu:
-// InstantNeRFDecoder.forward, src/decoders.py:136-162 -- fp16 operands, fp32 accumulation, sigma_net's first layer as a
-// split hi/lo product) with the layer products on the 5th-generation tensor cores instead of mma.sync.
+// Forward of the fused 64-wide Instant decoder on tcgen05: InstantNeRFDecoder.forward (src/decoders.py:136-162; network
+// and arithmetic in b2n_mlp64.cu's header -- fp16 operands, fp32 accumulation, sigma_net's first layer as a split hi/lo
+// product) with the layer products on the 5th-generation tensor cores.
 //
-// Why: the mma.sync kernel keeps activations in registers (C fragments re-packed as A fragments) and pays ~1500 warp
-// instructions per 32 points for fragment bookkeeping; at 255 registers it runs 8 warps per SM and is latency-bound
+// Why: an earlier mma.sync forward kept activations in registers (C fragments re-packed as A fragments) and paid ~1500
+// warp instructions per 32 points for fragment bookkeeping; at 255 registers it ran 8 warps per SM and was latency-bound
 // (tensor pipe 40 %, IPC 0.29 per scheduler: profiles/r2a_kernels.md).  Here a CTA owns a 128-point tile = the 128 TMEM
 // lanes: thread t owns point t.  Per layer ONE elected thread issues the K/16 tcgen05.mma (A = the activation tile in shared
 // memory, K-major SWIZZLE_128B; B = the layer's weight tile, staged once per CTA; D = 128 x N fp32 in TMEM), commits to an
@@ -13,11 +13,11 @@
 // One layer step is a latency chain (issue -> MMA -> commit -> mbarrier -> tcgen05.ld -> pack -> st.shared ->
 // fence.proxy.async -> bar.sync, ~1800 cycles measured with one CTA per SM), so throughput comes from co-resident CTAs:
 // 52 KB of shared memory at pos_dim <= 32 (x_hi and x_lo share ONE 64-column tile) -> 4 CTAs per SM, 68 KB above -> 3.
-// Measured, 4.2 M points (tools/kbench.py mlp64): 0.42 ms against 0.62 ms for the mma.sync kernel (pos_dim 32), 0.66
+// Measured, 4.2 M points (tools/kbench.py mlp64): 0.42 ms against 0.62 ms for that mma.sync kernel (pos_dim 32), 0.66
 // against 0.86 ms (pos_dim 53); 1 / 2 / 3 / 4 CTAs per SM: 1.05 / 0.66 / 0.50 / 0.42 ms.
 // cudaOccupancyMaxActiveBlocksPerMultiprocessor answers 1 for this kernel; the grid is sized from shared memory instead.
-#include <cuda_fp16.h>
-#include "b2n_common.cuh"
+#define B2N_OP_F16
+#include "b2n_mlp64.cuh"
 #include "b2n_tc.cuh"
 
 namespace b2n {
@@ -58,12 +58,6 @@ __device__ __forceinline__ float4 ldg_stream(const float* p) {      // read-once
   asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p));
   return v;
 }
-__device__ __forceinline__ uint32_t pack2(float lo, float hi) {
-  uint32_t r;
-  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
-  return r;
-}
-__device__ __forceinline__ float2 unpack2(uint32_t v) { return __half22float2(*reinterpret_cast<__half2*>(&v)); }
 
 // fp32 matrix [rows_valid][src_cols] (row stride src_cols) -> fp16 K-major SWIZZLE_128B tile [rows][64]; lo = the low half of the
 // hi/lo split (w - fp16(w)); columns >= src_cols and rows >= rows_valid are zero
@@ -83,56 +77,6 @@ __device__ __forceinline__ void stage_weight(const float* __restrict__ W, int ro
     }
     *reinterpret_cast<uint4*>(dst + swz(r, c)) = make_uint4(pack2(f[0], f[1]), pack2(f[2], f[3]), pack2(f[4], f[5]), pack2(f[6], f[7]));
   }
-}
-
-// softplus(h0 - 5) and the logistic function on the MUFU units (ex2 / lg2 / rcp: ~1e-6 relative, two orders below the fp16
-// operands around them) instead of libm's expf / log1pf and an IEEE division -- 110 of the ~1300 instructions a thread spent
-// per forward tile.  Small e = exp(v): the series of log1p (relative error < e^3 / 4 < 8e-6 below 1/32)
-__device__ __forceinline__ float softplus_m5(float h0) {
-  const float v = h0 - 5.0f;
-  const float e = __expf(fminf(v, 20.f));
-  const float sp = e < 0.03125f ? e * (1.f - e * (0.5f - e * 0.33333334f)) : __logf(1.f + e);
-  return v > 20.f ? v : sp;
-}
-__device__ __forceinline__ float sigmoidf(float v) { return __fdividef(1.f, 1.f + __expf(-v)); }
-
-// 32 view-direction features (3 + 6 L valid, then `pad` up to the colour net's padded input width, then zeros) as 4 chunks
-__device__ __forceinline__ void dir_features(const float (&d)[3], const float* __restrict__ bands, int L, float pad, uint4 (&o)[4]) {
-  const int dd = 3 + 6 * L, dpad = ((16 + dd + 15) & ~15) - 16;
-  float f[32];
-#pragma unroll
-  for (int i = 0; i < 32; ++i) f[i] = (i >= dd && i < dpad) ? pad : 0.f;
-  f[0] = d[0], f[1] = d[1], f[2] = d[2];
-  float ps[3], pc[3], prev = 0.f;
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    if (k < L) {
-      const float fr = __ldg(bands + k);
-      const bool dbl = (k > 0) && (fr == 2.f * prev);
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        float s, c;
-        if (dbl) {
-          s = 2.f * ps[j] * pc[j];
-          c = 1.f - 2.f * ps[j] * ps[j];
-        } else {
-          const float arg = __fmul_rn(__fmul_rn(d[j], fr), 3.14159274101257324f);
-          // beyond +-pi (non-unit directions, custom bands): one fp32 reduction step to [-pi, pi] instead of libm's
-          // Payne-Hanek path (hundreds of instructions and local memory in a kernel whose code must stay cache-resident)
-          const float red = fabsf(arg) <= 3.2f ? arg : __fmaf_rn(-6.28318530717958648f, rintf(arg * 0.159154943091895336f), arg);
-          __sincosf(red, &s, &c);
-        }
-        ps[j] = s, pc[j] = c;
-        f[3 + 6 * k + j] = s;
-        f[3 + 6 * k + 3 + j] = c;
-      }
-      prev = fr;
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-    o[i] = make_uint4(pack2(f[8 * i], f[8 * i + 1]), pack2(f[8 * i + 2], f[8 * i + 3]), pack2(f[8 * i + 4], f[8 * i + 5]),
-                      pack2(f[8 * i + 6], f[8 * i + 7]));
 }
 
 // drain 16 * NCH accumulator columns of this thread's TMEM lane (all loads in flight, one wait), ReLU, pack to fp16 and write
@@ -337,8 +281,8 @@ k_instant_fwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
         for (int j = 0; j < 8; ++j) q[j] = pack2(__uint_as_float(v[2 * j]), __uint_as_float(v[2 * j + 1]));
         sts128(a0 + swz(tid, 0), q[0], q[1], q[2], q[3]);
         sts128(a0 + swz(tid, 1), q[4], q[5], q[6], q[7]);
-        uint4 df[4];
-        dir_features(d[s], bands, L_dir, in_pad_value, df);
+        uint4 df[4];             // all four chunks first, then the stores (storing each chunk as it is packed reschedules NS = 2)
+        dir_features(d[s], bands, L_dir, in_pad_value, [&](int i, uint4 v) { df[i] = v; });
 #pragma unroll
         for (int i = 0; i < 4; ++i) sts128(a0 + swz(tid, 2 + i), df[i].x, df[i].y, df[i].z, df[i].w);      // layer 1 of color_net reads K = 48 only
         proxy_fence();
@@ -401,8 +345,8 @@ extern "C" int b2n_debug_instant_fwd_slots(int slots) {
   return prev;
 }
 
-// Same contract as b2n_instant_mlp_fwd (b2n_mlp64.cu dispatches here unless the mma.sync variant is selected through
-// b2n_debug_instant_variant); err_flag: device int, set non-zero if a stalled barrier aborted a tile.
+// rgb == NULL: density only -- dirs / dir_bands / color_params are not read and may be NULL; err_flag: device int, set
+// non-zero if a stalled barrier aborted a tile.
 extern "C" int b2n_instant_mlp_fwd_tc(const float* x_enc, int ldx, int pos_dim, const float* dirs, const float* dir_bands,
                                       int L_dir, const float* sigma_params, const float* color_params, int64_t P,
                                       float* rgb, float* sigma, float in_pad_value, int* err_flag, b2n_stream_t stream) {

@@ -6,7 +6,7 @@
 // the CPU error budget in tools/bf16_error_budget.py shows the 8-bit forward rounding, not the gradient rounding, is
 // what puts the parameter gradients 3e-2 away from fp32).  fp16 conversions saturate (cvt.rn.satfinite) so that a
 // large activation clamps to +-65504 instead of becoming inf; gradients are range-managed by the caller (a power-of-two
-// scale on the incoming gradient, see k_instant_bwd).
+// scale on the incoming gradient, see k_instant_bwd_tc).
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>

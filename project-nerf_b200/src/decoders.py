@@ -168,7 +168,7 @@ class InstantNeRFDecoder(BaseDecoder):
 
     def forward_fused(self, x_enc, dirs, dir_encoder):
         """Whole decoder (+ direction Fourier features) as ONE tensor-core kernel each way
-        (b2n_instant_mlp_fwd / _bwd); NeuralField.forward takes this path in bf16 mode."""
+        (b2n_instant_mlp_fwd_tc / _bwd_tc); NeuralField.forward takes this path in bf16 mode."""
         if self.sigma_net.input_pad_value != self.color_net.input_pad_value:
             raise ValueError("sigma_net and color_net must share one input_pad_value")
         return b2n.instant_mlp(x_enc, dirs, dir_encoder.freq_bands, self.sigma_net.params, self.color_net.params,

@@ -535,13 +535,20 @@ def test_amp_autocast_compatible(mods):
 BF16_TOL = 1e-2
 
 
-@pytest.mark.parametrize("pos_dim,Pn", [(32, 1000), (32, 64 * 37), (53, 777), (32, 5), (64, 130), (32, 40000)])
+_INSTANT_CASES = [(32, 1000, 0.0), (32, 64 * 37, 0.0), (53, 777, 0.0), (32, 5, 0.0), (64, 130, 0.0), (32, 40000, 0.0),
+                  (20, 1000, 1.0), (32, 300000, 0.0)]
+
+
+@pytest.mark.parametrize("pos_dim,Pn,pad", _INSTANT_CASES,
+                         ids=[f"{p}-{n}" + ("-pad1" if v else "") for p, n, v in _INSTANT_CASES])
 @pytest.mark.parametrize("gscale", [1.0, 65536.0, 2.0 ** -22])
-def test_instant_mlp_fp16_vs_oracle(mods, pos_dim, Pn, gscale):
+def test_instant_mlp_fp16_vs_oracle(mods, pos_dim, Pn, pad, gscale):
     """Fused Instant decoder (fp16 operands, split first layer, power-of-two scaled gradient chain) against
     (a) the oracle evaluated in the kernel's arithmetic model -- tight, forward and backward -- and
     (b) the plain fp32 oracle -- the north star's 1e-2 bar for the 16-bit MLP, outputs and gradients.
-    gscale multiplies the incoming gradient (GradScaler-sized and underflow-sized): the result must scale with it."""
+    gscale multiplies the incoming gradient (GradScaler-sized and underflow-sized): the result must scale with it.
+    pad: what the padded input columns of both networks hold (1.0: checkpoints of an upstream build, b2n.checkpoint).
+    P = 300 000 runs several waves of the persistent loops of both kernels."""
     from oracle import nerf_oracle as O
     torch.manual_seed(7)
     gen = torch.Generator().manual_seed(7)
@@ -552,16 +559,16 @@ def test_instant_mlp_fp16_vs_oracle(mods, pos_dim, Pn, gscale):
     d = d / d.norm(dim=-1, keepdim=True)
     bands = O.fourier_bands(4)
     wrt = [x, sd["d.sigma_net.params"], sd["d.color_net.params"]]
-    rgb, sigma = O.instant_decoder(sd, "d", x, O.fourier_encode(d, bands), 64)
-    rgb_q, sigma_q = O.instant_decoder(sd, "d", x, O.fourier_encode(d, bands), 64, emulate_bf16="kernel")
+    rgb, sigma = O.instant_decoder(sd, "d", x, O.fourier_encode(d, bands), 64, pad_value=pad)
+    rgb_q, sigma_q = O.instant_decoder(sd, "d", x, O.fourier_encode(d, bands), 64, emulate_bf16="kernel", pad_value=pad)
     g_rgb, g_sigma = torch.randn_like(rgb) * gscale, torch.randn_like(sigma) * gscale
     ref32 = torch.autograd.grad((rgb * g_rgb).sum() + (sigma * g_sigma).sum(), wrt)
     ref_q = torch.autograd.grad((rgb_q * g_rgb).sum() + (sigma_q * g_sigma).sum(), wrt)
     x2 = cu(x.detach()).requires_grad_(True)
     sp, cp = (cu(sd[k].detach()).requires_grad_(True) for k in ("d.sigma_net.params", "d.color_net.params"))
-    rgb2, sigma2 = mods["b2n"].instant_mlp(x2, cu(d), cu(bands), sp, cp)
+    rgb2, sigma2 = mods["b2n"].instant_mlp(x2, cu(d), cu(bands), sp, cp, pad_value=pad)
     assert rgb2.shape == (Pn, 3) and sigma2.shape == (Pn, 1)
-    tag = f"instant_mlp[{pos_dim},{Pn}]"
+    tag = f"instant_mlp[{pos_dim},{Pn}" + (",pad1]" if pad else "]")
     assert record(f"{tag}:rgb_vs_fp32", rel_err(rgb2.cpu(), rgb)) < BF16_TOL
     assert record(f"{tag}:sigma_vs_fp32", rel_err(sigma2.cpu(), sigma)) < BF16_TOL
     assert record(f"{tag}:rgb_vs_kernel_model", rel_err(rgb2.cpu(), rgb_q)) < 1e-3
@@ -585,12 +592,12 @@ def test_instant_mlp_fp16_vs_oracle(mods, pos_dim, Pn, gscale):
 
 @pytest.mark.parametrize("pos_dim,Pn,pad", [(32, 128 * 11 + 3, 0.0), (53, 777, 0.0), (64, 130, 0.0), (32, 5, 0.0),
                                             (20, 1000, 1.0), (32, 300000, 0.0)])
-def test_instant_fwd_tcgen05_matches_mma_sync(mods, pos_dim, Pn, pad):
-    """The two forward kernels of the fused Instant decoder (tcgen05: b2n_mlp64tc.cu, mma.sync: b2n_mlp64.cu) implement
-    the same arithmetic (fp16 operands, fp32 accumulation, split first layer): they may differ by accumulation order
-    only.  Also the density-only mode and the ones-padded inputs of upstream checkpoints."""
+def test_instant_fwd_tcgen05_schedules_agree(mods, pos_dim, Pn, pad):
+    """The forward of the fused Instant decoder with one or two point tiles in flight per CTA (b2nerf_debug.h) issues the
+    same MMAs on the same operands: bitwise equal outputs.  The density-only mode (instant_sigma) runs the same sigma_net
+    arithmetic: bitwise equal sigma.  Above pos_dim 32 there is one schedule only, so (53, 777) and (64, 130) compare
+    the kernel with itself; test_instant_mlp_fp16_vs_oracle checks those widths against the oracle."""
     from oracle import nerf_oracle as O
-    ops = mods["b2n"].ops
     gen = torch.Generator().manual_seed(11)
     sp = cu(O._fused_init(pos_dim, 16, 64, 1, gen))
     cp = cu(O._fused_init(43, 3, 64, 2, gen))
@@ -599,33 +606,28 @@ def test_instant_fwd_tcgen05_matches_mma_sync(mods, pos_dim, Pn, pad):
     bands = cu(O.fourier_bands(4))
     lib = mods["b2n"]._lib.lib
     out = {}
-    prev = ops.INSTANT_FWD_TC
     prev_slots = lib.b2n_debug_instant_fwd_slots(1)
     try:
-        for key, tc, slots in (("mma", False, 1), ("tc1", True, 1), ("tc2", True, 2)):       # slots: see b2nerf_debug.h
-            ops.INSTANT_FWD_TC = tc
+        for slots in (1, 2):
             lib.b2n_debug_instant_fwd_slots(slots)
             rgb, sigma = mods["b2n"].instant_mlp(x, d, bands, sp, cp, pad_value=pad)
-            out[key] = (rgb.clone(), sigma.clone(), mods["b2n"].instant_sigma(x, sp, pad_value=pad).clone())
+            out[slots] = (rgb.clone(), sigma.clone(), mods["b2n"].instant_sigma(x, sp, pad_value=pad).clone())
     finally:
-        ops.INSTANT_FWD_TC = prev
         lib.b2n_debug_instant_fwd_slots(prev_slots)
     mods["b2n"].check_errors()
-    for key in ("tc1", "tc2"):
-        tag = f"instant_fwd_{key}[{pos_dim},{Pn}]"
-        assert record(f"{tag}:rgb", rel_err(out[key][0], out["mma"][0])) < 2e-5
-        assert record(f"{tag}:sigma", rel_err(out[key][1], out["mma"][1])) < 2e-5
-        assert torch.equal(out[key][2], out[key][1])            # density-only mode: the same sigma_net arithmetic
-    assert torch.equal(out["tc2"][0], out["tc1"][0]) and torch.equal(out["tc2"][1], out["tc1"][1])      # same MMAs, other schedule
+    for slots in (1, 2):
+        assert torch.equal(out[slots][2], out[slots][1])
+    assert torch.equal(out[2][0], out[1][0]) and torch.equal(out[2][1], out[1][1])
 
 
 @pytest.mark.parametrize("pos_dim,Pn", [(32, 64 * 37 + 5), (53, 777), (64, 130), (32, 5), (32, 200000), (20, 64 * 148 * 3 + 1),
                                         (32, 1500000)])
-def test_instant_bwd_tcgen05_wgrad_matches_mma_sync(mods, pos_dim, Pn):
-    """The two backward kernels of the fused Instant decoder differ only in where the weight gradients are accumulated
-    (tcgen05 + TMEM vs mma.sync + registers): same operands, fp32 accumulation in a different order."""
+def test_instant_bwd_tcgen05_schedules_agree(mods, pos_dim, Pn):
+    """The backward of the fused Instant decoder with one or three 4-warp groups per CTA (b2nerf_debug.h) runs the same
+    mma.sync chain (bitwise equal g_x) and the same weight-gradient MMAs, accumulated over the tiles in another order.
+    Above pos_dim 32 there is one schedule only, so (53, 777) and (64, 130) compare the kernel with itself;
+    test_instant_mlp_fp16_vs_oracle checks those widths against the oracle."""
     from oracle import nerf_oracle as O
-    ops = mods["b2n"].ops
     gen = torch.Generator().manual_seed(13)
     sp = cu(O._fused_init(pos_dim, 16, 64, 1, gen)).requires_grad_(True)
     cp = cu(O._fused_init(43, 3, 64, 2, gen)).requires_grad_(True)
@@ -636,23 +638,20 @@ def test_instant_bwd_tcgen05_wgrad_matches_mma_sync(mods, pos_dim, Pn):
     g1, g2 = torch.randn_like(rgb), torch.randn_like(sigma)
     lib = mods["b2n"]._lib.lib
     out = {}
-    prev = ops.INSTANT_BWD_TC
     prev_groups = lib.b2n_debug_instant_bwd_groups(1)
     try:
-        for key, tc, groups in (("mma", False, 1), ("tc1", True, 1), ("tc3", True, 3)):      # groups: see b2nerf_debug.h
-            ops.INSTANT_BWD_TC = tc
+        for groups in (1, 3):
             lib.b2n_debug_instant_bwd_groups(groups)
-            out[key] = torch.autograd.grad([rgb, sigma], [x, sp, cp], [g1, g2], retain_graph=True)
+            out[groups] = torch.autograd.grad([rgb, sigma], [x, sp, cp], [g1, g2], retain_graph=True)
     finally:
-        ops.INSTANT_BWD_TC = prev
         lib.b2n_debug_instant_bwd_groups(prev_groups)
     mods["b2n"].check_errors()
-    for key in ("tc1", "tc3"):
-        tag = f"instant_bwd_{key}[{pos_dim},{Pn}]"
-        assert torch.equal(out[key][0], out["mma"][0])                 # g_x: the same mma.sync chain
-        for a_, b_, name in zip(out[key][1:], out["mma"][1:], ("g_sigma_params", "g_color_params")):
-            assert record(f"{tag}:{name}", rel_err(a_, b_)) < 2e-5, name
-        V3 = out[key][2][64 * 48 + 64 * 64:].view(16, 64)
+    tag = f"instant_bwd_tc3[{pos_dim},{Pn}]"
+    assert torch.equal(out[3][0], out[1][0])
+    for a_, b_, name in zip(out[3][1:], out[1][1:], ("g_sigma_params", "g_color_params")):
+        assert record(f"{tag}:{name}", rel_err(a_, b_)) < 2e-5, name
+    for groups in (1, 3):          # padded rows of the output layer never receive gradient
+        V3 = out[groups][2][64 * 48 + 64 * 64:].view(16, 64)
         assert float(V3[3:].abs().max()) == 0.0
 
 

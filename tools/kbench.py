@@ -470,7 +470,8 @@ def composite(B=2 ** 18, N=128):
 
 
 def mlp64(P=1 << 22):
-    """fused Instant decoder: forward (mma.sync vs tcgen05) and backward, C2-sized (4.2 M points) and Part-3 width"""
+    """fused Instant decoder: forward (1 or 2 point tiles in flight per CTA) and backward (1 or 3 warp groups per CTA),
+    C2-sized (4.2 M points) and Part-3 width"""
     from oracle import nerf_oracle as O
     for pos_dim in (32, 53):
         gen = torch.Generator().manual_seed(0)
@@ -479,21 +480,19 @@ def mlp64(P=1 << 22):
         x = (torch.randn(P, pos_dim, device="cuda") * 0.5).requires_grad_(True)
         d = torch.nn.functional.normalize(torch.randn(P, 3, device="cuda"), dim=-1)
         bands = O.fourier_bands(4).cuda()
-        for tc, slots in ((False, 1), (True, 1), (True, 2)):
-            ops.INSTANT_FWD_TC = tc
+        for slots in (1, 2):
             _lib.lib.b2n_debug_instant_fwd_slots(slots)
             with torch.no_grad():
                 med, best = timeit(lambda: b2n.instant_mlp(x, d, bands, sp, cp))
                 meds, bests = timeit(lambda: b2n.instant_sigma(x, sp))
-            print(f"instant fwd pos_dim={pos_dim} P={P} tc={tc} slots={slots}: {med:.3f} ms (best {best:.3f}); sigma-only {meds:.3f} ms")
+            print(f"instant fwd pos_dim={pos_dim} P={P} slots={slots}: {med:.3f} ms (best {best:.3f}); sigma-only {meds:.3f} ms")
         b2n.check_errors()
         rgb, sigma = b2n.instant_mlp(x, d, bands, sp, cp)
         g1, g2 = torch.randn_like(rgb), torch.randn_like(sigma)
-        for tc, groups in ((False, 1), (True, 1), (True, 3)):
-            ops.INSTANT_BWD_TC = tc
+        for groups in (1, 3):
             _lib.lib.b2n_debug_instant_bwd_groups(groups)
             med, best = timeit(lambda: torch.autograd.grad([rgb, sigma], [x, sp, cp], [g1, g2], retain_graph=True))
-            print(f"instant bwd pos_dim={pos_dim} P={P} tc={tc} groups={groups}: {med:.3f} ms (best {best:.3f})")
+            print(f"instant bwd pos_dim={pos_dim} P={P} groups={groups}: {med:.3f} ms (best {best:.3f})")
         b2n.check_errors()
 
 
