@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 17
+#define B2N_ABI_VERSION 18
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -80,7 +80,8 @@ int b2n_occ_update(const float* cur_sigma, float* grid, int64_t n_voxels, int dy
  *   u [B,N] or NULL       the U[0,1) jitter (torch.rand) -- NULL = no perturb;
  *   bits or NULL          occupancy bitfield; NULL = every sample active;
  * outputs
- *   z [B,N]               z = lo + (hi - lo) * u   (or z_base)
+ *   z [B,N]               z = lo + (hi - lo) * u   (or z_base); may be NULL
+ *                         when u is NULL (the depths are then z_base itself)
  *   mask_words [B,W]      W = (N+31)/32, bit s%32 of word s/32 = sample active
  *   ray_count [B]         active samples of the ray (int32)                  */
 int b2n_march_mask(const float* rays_o, const float* rays_d, const float* z_base, const float* z_lo,
@@ -440,6 +441,50 @@ size_t b2n_mesh_scratch(int R);
 int b2n_mesh_count(const float* sigma, int R, float threshold, void* scratch, int64_t* totals, b2n_stream_t stream);
 int b2n_mesh_emit(const float* sigma, const float* axis_ext, int R, float threshold, void* scratch, int64_t n_verts,
                   int64_t n_faces, float* verts, int32_t* faces, b2n_stream_t stream);
+
+/* ------------------------------------------------------------------------
+ * Inference rendering with early ray termination (b2n.render; DESIGN.md §5g).  Not the reference's render_rays: a
+ * separate contract that equals the masked render_rays(perturb=False, density_grid) at eps = 0.
+ *   Samples: depth z_s = z_base[s] (s < N <= 1024), point o + d*z_s with separately rounded fp32 operations (bitwise
+ *     the points of b2n_march_compact), active iff bit s of the ray's mask_words (b2n_march_mask with u = z = NULL,
+ *     then b2n_march_scan when a grid is used, which keeps the forced sample 0 of ray 0 of an all-empty mask).
+ *   Compositing: the active samples of a ray, front to back, one at a time, with the per-sample arithmetic of
+ *     b2n_composite_fwd: delta_s = (z_base[s+1] - z_base[s]) * |d| (1e10 * |d| for s = N-1; z_base[s+1] is the next
+ *     depth of the full grid, active or not), alpha = 1 - expf(-sigma * delta), w = alpha * T, T <- T * (1 - alpha +
+ *     1e-10), color += w * rgb, depth += w * z_s, acc += w, each operation rounded separately.  After a sample, T < eps
+ *     ends the ray: none of its later samples count (eps = 0: never).  N == 1 composites nothing (pure background).
+ *   Only the order of the transmittance product differs from b2n_composite_fwd (a sequential chain instead of a warp
+ *   scan).  The per-ray state lives in fp32 across waves, so the result does not depend on how the samples of a ray
+ *   are grouped into waves.  For eps > 0 and colours, bg in [0, 1], color and acc lie within T_stop <= eps of the
+ *   eps = 0 result and depth within eps * far (plus fp32 rounding).
+ * A render is a loop of waves over the ALIVE rays (int32 ray ids, ascending):
+ *   b2n_render_begin: state [B] (32 bytes per ray: T, colour, depth, acc, cursor) initialised, alive = the rays with at
+ *     least one active sample, *n_alive (device int32) = their number.  3 kernels.
+ *   b2n_render_emit: for alive[0..n_alive), the next (up to) K active samples after each ray's cursor, compacted in
+ *     (alive slot, sample) order: sample_idx (s), pts [P,3], dirs [P,3] (d/|d|, as b2n_march_compact), t_out [P]
+ *     (the ray's time; NULL when times is NULL), and *total (device int32) = P.  3 kernels (count, scan, write).
+ *   b2n_render_composite: rgb [P,3], sigma [P] of those samples (the model's output) folded into the state of every
+ *     alive ray; the rays that are not done (T >= eps and an active sample left) go, in order, to alive_next, and
+ *     *n_alive_next (device int32) = their number.  Takes the alive list, n_alive and scratch of the emit before it;
+ *     alive_next must not alias alive.  3 kernels (fold, scan, write).
+ *   b2n_render_finish: color [B,3] = colour + (1 - acc) * bg, depth [B], acc [B] of every ray; bg [3] (bg_per_ray = 0)
+ *     or [B,3] (bg_per_ray = 1).
+ * scratch: b2n_render_scratch(B) bytes, shared by begin / emit / composite.  The host reads *n_alive (to size the next
+ * wave) and *total (to size the model call): two 4-byte reads per wave and no other synchronisation.  Those reads make
+ * a render impossible to capture in a CUDA graph, by design.  B * N < 2^31 and n_alive * K < 2^31. */
+size_t b2n_render_scratch(int64_t B);
+int b2n_render_begin(const uint32_t* mask_words, int64_t B, int N, void* state, int32_t* alive, int32_t* n_alive,
+                     void* scratch, b2n_stream_t stream);
+int b2n_render_emit(const float* rays_o, const float* rays_d, const float* times, const float* z_base,
+                    const uint32_t* mask_words, int64_t B, int N, const void* state, const int32_t* alive,
+                    int64_t n_alive, int K, int32_t* sample_idx, float* pts, float* dirs, float* t_out, int32_t* total,
+                    void* scratch, b2n_stream_t stream);
+int b2n_render_composite(const float* rgb, const float* sigma, const float* z_base, const float* rays_d, int64_t B,
+                         int N, float eps, void* state, const int32_t* alive, int64_t n_alive,
+                         const int32_t* sample_idx, int32_t* alive_next, int32_t* n_alive_next, void* scratch,
+                         b2n_stream_t stream);
+int b2n_render_finish(const void* state, int64_t B, const float* bg, int bg_per_ray, float* color, float* depth,
+                      float* acc, b2n_stream_t stream);
 
 #ifdef __cplusplus
 }

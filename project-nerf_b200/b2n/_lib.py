@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb2nerf.so")
 
-ABI_VERSION = 17
+ABI_VERSION = 18
 
 P, L, I, F = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
 
@@ -72,6 +72,11 @@ SIGNATURES = {
     "b2n_mesh_scratch": [I],
     "b2n_mesh_count": [P, I, F, P, P, P],
     "b2n_mesh_emit": [P, P, I, F, P, L, L, P, P, P],
+    "b2n_render_scratch": [L],
+    "b2n_render_begin": [P, L, I, P, P, P, P, P],
+    "b2n_render_emit": [P, P, P, P, P, L, I, P, P, L, I, P, P, P, P, P, P, P],
+    "b2n_render_composite": [P, P, P, P, L, I, F, P, P, L, P, P, P, P, P],
+    "b2n_render_finish": [P, L, P, I, P, P, P, P],
 }
 # development / measurement entry points (include/b2nerf_debug.h): bound like the rest, never called by a product path
 DEBUG_SIGNATURES = {
@@ -87,7 +92,7 @@ DEBUG_SIGNATURES = {
     "b2n_debug_mnmajor_probe": [P, P, P, I, I, I, I, P],
 }
 _RESTYPES = {"b2n_last_error": ctypes.c_char_p, "b2n_march_scan_scratch": ctypes.c_size_t, "b2n_hash_order_scratch": ctypes.c_size_t,
-             "b2n_mesh_scratch": ctypes.c_size_t,
+             "b2n_mesh_scratch": ctypes.c_size_t, "b2n_render_scratch": ctypes.c_size_t,
              "b2n_nerf_mlp_packed_bytes": ctypes.c_size_t, "b2n_nerf_mlp_packed_bwd_bytes": ctypes.c_size_t}
 
 
@@ -118,7 +123,7 @@ lib = _load()
 # launch accounting for bench.py ("gpu_launches"): every successful C-ABI call adds the
 # number of kernels that entry point launches.
 LAUNCHES = {"count": 0}
-_KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_hash_order": 5, "b2n_mesh_count": 2, "b2n_mesh_emit": 2, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
+_KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_hash_order": 5, "b2n_mesh_count": 2, "b2n_mesh_emit": 2, "b2n_render_begin": 3, "b2n_render_emit": 3, "b2n_render_composite": 3, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
 
 
 def ptr(t):

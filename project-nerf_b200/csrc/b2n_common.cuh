@@ -50,6 +50,36 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// Exclusive scan of one int per thread over the block; *total (shared) gets the block sum.  Every thread of the block
+// must call it (it synchronises).
+__device__ __forceinline__ int block_exclusive_scan(int v, int* total) {
+  __shared__ int warp_tot[32];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  int inc = v;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    int t = __shfl_up_sync(0xffffffffu, inc, o);
+    if (lane >= o) inc += t;
+  }
+  if (lane == 31) warp_tot[wid] = inc;
+  __syncthreads();
+  if (wid == 0) {
+    int t = lane < nw ? warp_tot[lane] : 0;
+    int ti = t;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      int q = __shfl_up_sync(0xffffffffu, ti, o);
+      if (lane >= o) ti += q;
+    }
+    warp_tot[lane] = ti - t;  // exclusive prefix of the warp totals
+    if (lane == 31) *total = ti;
+  }
+  __syncthreads();
+  int res = inc - v + warp_tot[wid];
+  __syncthreads();
+  return res;
+}
+
 // streaming (read-once) loads/stores: keep L2 for the hash tables
 __device__ __forceinline__ float ld_stream(const float* p) { return __ldcs(p); }
 __device__ __forceinline__ void st_stream(float* p, float v) { __stcs(p, v); }

@@ -83,7 +83,7 @@ k_march_mask(const float* __restrict__ rays_o, const float* __restrict__ rays_d,
         } else {
           z = __ldg(z_base + s);
         }
-        __stcs(z_out + r * N + s, z);
+        if (z_out) __stcs(z_out + r * N + s, z);
         if (bits) {
           const float px = __fadd_rn(ox, __fmul_rn(dx, z));
           const float py = __fadd_rn(oy, __fmul_rn(dy, z));
@@ -139,7 +139,7 @@ k_march_mask_u(const float* __restrict__ rays_o, const float* __restrict__ rays_
       act[k] = false;
       if (s < N) {
         const float z = u ? __fadd_rn(lo[k], __fmul_rn(__fsub_rn(hi[k], lo[k]), uu[k])) : lo[k];
-        __stcs(z_out + r * N + s, z);
+        if (z_out) __stcs(z_out + r * N + s, z);
         if (bits) {
           const float px = __fadd_rn(ox, __fmul_rn(dx, z));
           const float py = __fadd_rn(oy, __fmul_rn(dy, z));
@@ -167,34 +167,6 @@ k_march_mask_u(const float* __restrict__ rays_o, const float* __restrict__ rays_
 constexpr int kScanThreads = 256;
 constexpr int kScanPerThread = 8;
 constexpr int kScanChunk = kScanThreads * kScanPerThread;  // 2048 rays per block
-
-__device__ __forceinline__ int block_exclusive_scan(int v, int* total) {
-  __shared__ int warp_tot[32];
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  int inc = v;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    int t = __shfl_up_sync(0xffffffffu, inc, o);
-    if (lane >= o) inc += t;
-  }
-  if (lane == 31) warp_tot[wid] = inc;
-  __syncthreads();
-  if (wid == 0) {
-    int t = lane < nw ? warp_tot[lane] : 0;
-    int ti = t;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      int q = __shfl_up_sync(0xffffffffu, ti, o);
-      if (lane >= o) ti += q;
-    }
-    warp_tot[lane] = ti - t;  // exclusive prefix of the warp totals
-    if (lane == 31) *total = ti;
-  }
-  __syncthreads();
-  int res = inc - v + warp_tot[wid];
-  __syncthreads();
-  return res;
-}
 
 __global__ void __launch_bounds__(kScanThreads) k_scan_block_sums(const int32_t* __restrict__ cnt, int64_t B,
                                                                   int32_t* __restrict__ block_sums) {
@@ -346,8 +318,8 @@ extern "C" int b2n_march_mask(const float* rays_o, const float* rays_d, const fl
                               b2n_stream_t stream) {
   B2N_REQUIRE(B >= 0 && N > 0 && N <= 4096, "bad B or N");
   if (B == 0) return B2N_OK;
-  B2N_REQUIRE(rays_o && rays_d && z_base && z && mask_words && ray_count, "null pointer");
-  B2N_REQUIRE(!u || (z_lo && z_hi), "jitter needs the stratum bounds");
+  B2N_REQUIRE(rays_o && rays_d && z_base && mask_words && ray_count, "null pointer");
+  B2N_REQUIRE(!u || (z_lo && z_hi && z), "jitter needs the stratum bounds and z");
   B2N_REQUIRE(!bits || (R > 0 && R <= 1024), "bad grid resolution");
   B2N_REQUIRE(B * (int64_t)N < (int64_t)1 << 31, "B*N must fit int32");
   if (N <= 64)

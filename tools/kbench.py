@@ -246,6 +246,109 @@ def mesh(sizes=(128, 256, 512)):
         torch.cuda.empty_cache()
 
 
+def render(H=800, N=128, chunk=2 ** 16, checkpoints=(300, 2000)):
+    """One 800 x 800 view at N = 128 of the C2 model (bench.py's configuration, bf16, eval mode) trained on an analytic
+    sphere of radius 1 (white background) with its 128^3 occupancy grid, measured after each number of steps in
+    `checkpoints` (the longer the training, the more opaque the surface): reference-semantics render_image, chunked
+    render_rays with the grid, and b2n.render_image_fast at t_min = 0 and 1e-4.  Medians over 10 runs after 3 warm-ups.
+    After the last checkpoint the wave budget (b2n.render.WAVE_POINTS) is swept at t_min = 1e-4."""
+    import subprocess
+    from b2n import render as br
+    from b2n import synthetic
+    from src.renderer import DensityGrid, render_image, render_rays
+    try:
+        smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,power.max_limit", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=60).stdout.strip().splitlines()[0]
+    except Exception as e:                                # noqa: BLE001 -- the measurement stands without it
+        smi = f"nvidia-smi unavailable ({e})"
+    print(f"device: {torch.cuda.get_device_name()} | nvidia-smi name, power.limit, power.max_limit: {smi}")
+    sys.path.insert(0, ROOT)
+    from bench import C2, GRID_R, GRID_THR
+    near, far, radius = 2.0, 6.0, 1.0
+    b2n.set_mlp_precision("bf16")
+    torch.manual_seed(0)
+    model = NeuralField(C2).cuda().train()
+    grid = DensityGrid(resolution=GRID_R, bound=C2["scene_bound"], threshold=GRID_THR).cuda()
+    opt = torch.optim.AdamW(model.parameters(), lr=1e-2, weight_decay=1e-5)
+    bg = torch.ones(3, device="cuda")
+    ro, rd = synthetic.image_rays(synthetic.hemisphere_poses(1, seed=123)[0], H=H, W=H)
+    ro, rd = ro.cuda(), rd.cuda()
+    rays = H * H
+
+    def sphere(o, d):
+        b = (o * d).sum(-1)
+        disc = b * b - ((o * o).sum(-1) - radius ** 2)
+        p = o + d * (-b - torch.sqrt(disc.clamp_min(0)))[:, None]
+        col = torch.stack([0.5 + 0.5 * p[:, 2], 0.2 + 0.3 * p[:, 0], 0.5 - 0.5 * p[:, 2]], -1).clamp(0, 1)
+        return torch.where((disc > 0)[:, None], col, torch.ones_like(col))
+
+    def image():
+        return render_image(model, ro.view(H, H, 3), rd.view(H, H, 3), near, far, N, chunk, True)
+
+    def masked():
+        outs = [render_rays(model, ro[i:i + chunk], rd[i:i + chunk], near, far, N, False, density_grid=grid)
+                for i in range(0, rays, chunk)]
+        return [torch.cat(x) for x in zip(*outs)]
+
+    def fast(t_min):
+        return br.render_image_fast(model, ro.view(H, H, 3), rd.view(H, H, 3), near, far, N, density_grid=grid,
+                                    t_min=t_min)
+
+    step = 0
+    for stop in checkpoints:
+        model.train()
+        for step in range(step + 1, stop + 1):
+            o, d, _ = (t.cuda() for t in synthetic.random_rays(2 ** 16, seed=step))
+            pred, _, _ = render_rays(model, o, d, near, far, 64, True, density_grid=grid, bg_color=bg)
+            loss = torch.nn.functional.mse_loss(pred, sphere(o, d))
+            opt.zero_grad()
+            loss.backward()
+            opt.step()
+            if step >= 50 and step % 16 == 0:
+                model.eval()
+                grid.update(model, device="cuda")
+                model.train()
+        model.eval()
+        occ = grid.update(model, device="cuda")
+        with torch.no_grad():
+            psnr = -10 * torch.log10(((image().view(-1, 3) - sphere(ro, rd)) ** 2).mean())
+            ref = masked()
+            n_masked = b2n.march.march(ro, rd, near, far, N, None, bits=grid.bits(), R=grid.resolution,
+                                       bound=grid.bound).n_active
+            print(f"\nC2 trained {stop} steps on a sphere of radius {radius}: loss {loss.item():.5f}, grid occupancy "
+                  f"{occ:.3f}, test-view PSNR {psnr.item():.2f} dB; view {H}x{H}, N={N}, wave budget 2^"
+                  f"{br.WAVE_POINTS.bit_length() - 1}")
+            legs = [("render_image (reference semantics, every sample)", image, rays * N, None),
+                    ("render_rays with the grid, chunks of 2^16 rays", masked, n_masked, None),
+                    ("render_image_fast t_min=0", lambda: fast(0.0), None, 0.0),
+                    ("render_image_fast t_min=1e-4", lambda: fast(1e-4), None, 1e-4)]
+            for name, fn, n_eval, t_min in legs:
+                med, best = timeit(fn, n=10, warm=3)
+                extra = ""
+                if t_min is not None:
+                    out = fast(t_min)
+                    n_eval = out.n_evaluated
+                    err = [float((a.reshape(b.shape) - b).abs().max()) for a, b in zip(out[:3], ref)]
+                    extra = (f", {out.n_waves} waves, max |diff| to the masked path: color {err[0]:.2e} "
+                             f"depth {err[1]:.2e} acc {err[2]:.2e}")
+                print(f"{name}: median {med:.3f} ms (best {best:.3f}), {n_eval / rays:.2f} evaluated samples per ray"
+                      f"{extra}")
+            out = br.render_image_fast(model, ro.view(H, H, 3), rd.view(H, H, 3), near, far, N, density_grid=grid,
+                                       t_min=1e-4, _samples_per_wave=1)
+            print(f"composited samples per ray at t_min=1e-4 (one sample per wave): {out.n_evaluated / rays:.2f}")
+    default = br.WAVE_POINTS
+    try:
+        with torch.no_grad():
+            for wp in (2 ** 18, 2 ** 19, 2 ** 20, 2 ** 21, 2 ** 22, 2 ** 23, 2 ** 24):
+                br.WAVE_POINTS = wp
+                med, best = timeit(lambda: fast(1e-4), n=10, warm=3)
+                out = fast(1e-4)
+                print(f"wave budget 2^{wp.bit_length() - 1}: t_min=1e-4 median {med:.3f} ms (best {best:.3f}), "
+                      f"{out.n_waves} waves, {out.n_evaluated / rays:.2f} evaluated samples per ray")
+    finally:
+        br.WAVE_POINTS = default
+
+
 def c1_step(P_rays=4096, N=64):
     """C1: vanilla NeRF training step (render_rays + MSE + backward + Adam), B=4096, N=64."""
     from b2n import synthetic
@@ -559,6 +662,8 @@ if __name__ == "__main__":
         occ_update()
     elif what == "mesh":
         mesh()
+    elif what == "render":
+        render()
     elif what == "hashsort":
         hash_sorted()
     elif what == "hash":
