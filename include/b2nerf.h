@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 18
+#define B2N_ABI_VERSION 19
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -485,6 +485,32 @@ int b2n_render_composite(const float* rgb, const float* sigma, const float* z_ba
                          b2n_stream_t stream);
 int b2n_render_finish(const void* state, int64_t B, const float* bg, int bg_per_ray, float* color, float* depth,
                       float* acc, b2n_stream_t stream);
+
+/* ------------------------------------------------------------------------
+ * Hierarchical importance sampling (b2n.importance; DESIGN.md §5h): NeRF's sample_pdf (Mildenhall et al. 2020) on the
+ * GPU.  Not part of the reference, which samples one stratified pass; an extension that is off unless asked for.
+ * Per ray r < B, with sorted coarse depths z [B,Nc] (jittered or not) and coarse densities sigma [B,Nc]:
+ *   Weights, with the arithmetic of b2n_composite_fwd: delta_s = (z_{s+1} - z_s) * |d| (1e10 * |d| for s = Nc-1),
+ *     alpha_s = 1 - exp(-sigma_s * delta_s), T_0 = 1, T_{s+1} = T_s * (1 - alpha_s + 1e-10), w_s = alpha_s * T_s;
+ *     alpha is computed as -expm1f(-sigma * delta), which keeps the small weights of a nearly empty ray accurate.
+ *   Bins: the Nc-1 midpoints m_i = (z_i + z_{i+1}) / 2.  PDF: w_1 .. w_{Nc-2} (first and last dropped), each + 1e-5,
+ *     normalised; CDF c [Nc-1] = [0, cumsum(pdf)] (c[Nc-2] = 1; kept non-decreasing in fp32 by a running max).
+ *   Fine positions u_k, k < Nf: u_table [Nf] (deterministic: torch.linspace(0, 1, Nf), built on the host), or
+ *     u_k = (k + U[r,k]) / Nf from u_jitter U [B,Nf] in [0,1) (stratified).  Exactly one of the two must be given.
+ *   Inverse CDF: i = searchsorted(c, u, right=True), below = max(i-1, 0), above = min(i, Nc-2),
+ *     denom = c[above] - c[below] (1 if < 1e-5), t = (u - c[below]) / denom,
+ *     z_fine[r,k] = m[below] + t * (m[above] - m[below]), clamped to [m[below], m[above]] (which only absorbs rounding).
+ *     Every index is clamped: no input, a non-finite sigma included, reads out of range.  u non-decreasing in k makes
+ *     z_fine non-decreasing in k, inside [m_0, m_{Nc-2}].
+ *   Merge: z_merged [B,Nc+Nf] = the coarse and fine depths merged, non-decreasing, coarse before fine on ties;
+ *     merge_src [B,Nc+Nf] int32 = the source of each slot: s for coarse slot s, Nc + k for fine slot k.  z_merged is
+ *     bitwise the source value.
+ * Limits: Nc >= 3, Nf >= 1, Nc + Nf <= 1024 (b2n_composite_*'s limit); refused before any launch.  One kernel, one warp
+ * per ray, no atomics, no host synchronisation (capturable in a CUDA graph), deterministic.  Reads 8*Nc bytes per ray
+ * (+ 4*Nf with u_jitter), writes 4*Nf + 8*(Nc + Nf). */
+int b2n_importance_sample(const float* sigma, const float* z, const float* rays_d, const float* u_table,
+                          const float* u_jitter, int64_t B, int Nc, int Nf, float* z_fine, float* z_merged,
+                          int32_t* merge_src, b2n_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb2nerf.so")
 
-ABI_VERSION = 18
+ABI_VERSION = 19
 
 P, L, I, F = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
 
@@ -77,6 +77,7 @@ SIGNATURES = {
     "b2n_render_emit": [P, P, P, P, P, L, I, P, P, L, I, P, P, P, P, P, P, P],
     "b2n_render_composite": [P, P, P, P, L, I, F, P, P, L, P, P, P, P, P],
     "b2n_render_finish": [P, L, P, I, P, P, P, P],
+    "b2n_importance_sample": [P, P, P, P, P, L, I, I, P, P, P, P],
 }
 # development / measurement entry points (include/b2nerf_debug.h): bound like the rest, never called by a product path
 DEBUG_SIGNATURES = {

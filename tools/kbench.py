@@ -349,6 +349,147 @@ def render(H=800, N=128, chunk=2 ** 16, checkpoints=(300, 2000)):
         br.WAVE_POINTS = default
 
 
+def _device_line():
+    import subprocess
+    try:
+        smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,power.max_limit", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=60).stdout.strip().splitlines()[0]
+    except Exception as e:                                # noqa: BLE001 -- the measurement stands without it
+        smi = f"nvidia-smi unavailable ({e})"
+    print(f"device: {torch.cuda.get_device_name()} | nvidia-smi name, power.limit, power.max_limit: {smi}")
+
+
+def _torch_importance(sigma, z, rd, Nf, U):
+    """the rule of b2n_importance_sample as torch ops (cumprod, cumsum, searchsorted, gather, stable sort)"""
+    B, Nc = z.shape
+    delta = torch.cat([z[:, 1:] - z[:, :-1], torch.full_like(z[:, :1], 1e10)], -1) * rd.norm(dim=-1, keepdim=True)
+    alpha = -torch.expm1(-sigma * delta)
+    w = alpha * torch.cumprod(torch.cat([torch.ones_like(alpha[:, :1]), 1.0 - alpha[:, :-1] + 1e-10], -1), -1)
+    mids = 0.5 * (z[:, 1:] + z[:, :-1])
+    wi = w[:, 1:-1] + 1e-5
+    cdf = torch.cat([torch.zeros_like(wi[:, :1]), torch.cumsum(wi / wi.sum(-1, keepdim=True), -1)], -1)
+    u = (torch.arange(Nf, device=z.device) + U) / Nf
+    i = torch.searchsorted(cdf, u, right=True)
+    below, above = (i - 1).clamp_min(0), i.clamp_max(Nc - 2)
+    cb, ca = torch.gather(cdf, 1, below), torch.gather(cdf, 1, above)
+    mb, ma = torch.gather(mids, 1, below), torch.gather(mids, 1, above)
+    denom = ca - cb
+    denom = torch.where(denom < 1e-5, torch.ones_like(denom), denom)
+    zf = mb + (u - cb) / denom * (ma - mb)
+    zm, src = torch.sort(torch.cat([z, zf], -1), dim=-1, stable=True)
+    return zf, zm, src
+
+
+def importance(Nc=64, Nf=128, quality_steps=1000):
+    """Hierarchical sampling (b2n.importance, DESIGN.md §5h): (1) the sampler kernel against the same rule as torch ops
+    at the C1 batch (B = 4096, L2-resident) and one 800^2 view (640 000 rays), in HBM bytes/s of the algorithmic
+    traffic; (2) a C1 training step (vanilla model, bf16, B = 4096) with 64 + 128 hierarchical samples against
+    stratified N = 64 and N = 192, and the cost of the merged-order gather inside it; (3) held-out PSNR on the analytic
+    spheres of tests/test_gpu_training.py after a fixed number of steps: hierarchical 64 + 128 against stratified
+    N = 192 (as many composited samples) and N = 256 (NeRF's evaluation count)."""
+    from b2n import march, synthetic
+    from b2n.importance import _gather, importance_sample, render_rays_hierarchical
+    from src.renderer import render_rays
+    _device_line()
+    torch.manual_seed(0)
+    # (1) the sampler
+    for B in (4096, 640_000):
+        ro, rd, _ = (t.cuda() for t in synthetic.random_rays(B, seed=1))
+        z = march.march(ro, rd, 2.0, 6.0, Nc, torch.rand(B, Nc, device="cuda")).z
+        sigma = torch.rand(B, Nc, device="cuda") * 4 * (torch.rand(B, Nc, device="cuda") < 0.5)
+        U = torch.rand(B, Nf, device="cuda")
+        nbytes = B * (8.0 * Nc + 12 + 4.0 * Nf + 4.0 * Nf + 8.0 * (Nc + Nf))
+        ours = importance_sample(sigma, z, rd, Nf, U)
+        ref = _torch_importance(sigma, z, rd, Nf, U)
+        dz = float((ours[0] - ref[0]).abs().max())
+        same_src = float((ours[2].long() == ref[2]).float().mean())
+        for name, fn in (("b2n_importance_sample", lambda: importance_sample(sigma, z, rd, Nf, U)),
+                         ("torch ops", lambda: _torch_importance(sigma, z, rd, Nf, U))):
+            med, best = timeit(fn, n=20, warm=3)
+            print(f"sampler B={B} {Nc}+{Nf} [{name}]: median {med:.4f} ms (best {best:.4f}), "
+                  f"{nbytes / med / 1e6:.0f} GB/s of the kernel's {nbytes / B:.0f} B/ray")
+        print(f"  kernel vs torch ops: max |dz_fine| {dz:.2e}, merge sources equal for {100 * same_src:.3f} % of slots")
+    # (2) the C1 step
+    b2n.set_mlp_precision("bf16")
+    B = 4096
+    ro, rd, _ = (t.cuda() for t in synthetic.random_rays(B, seed=1))
+    for leg in ("stratified N=64", "stratified N=192", f"hierarchical {Nc}+{Nf}"):
+        torch.manual_seed(0)
+        model = NeuralField(dict(mode="part2_nerf", L_embed=10, L_embed_dir=4)).cuda().train()
+        opt = torch.optim.Adam(model.parameters(), lr=5e-4)
+        tgt = torch.rand(B, 3, device="cuda")
+
+        def step():
+            if leg.startswith("hier"):
+                out = render_rays_hierarchical(model, ro, rd, 2.0, 6.0, Nc, Nf, True)
+                loss = torch.nn.functional.mse_loss(out.color, tgt) + torch.nn.functional.mse_loss(out.coarse_color, tgt)
+            else:
+                pred = render_rays(model, ro, rd, 2.0, 6.0, int(leg.split("=")[1]), True, white_bkgd=True)[0]
+                loss = torch.nn.functional.mse_loss(pred, tgt)
+            opt.zero_grad()
+            loss.backward()
+            opt.step()
+        med, best = timeit(step, n=20, warm=3)
+        print(f"C1 train step [bf16] B={B} {leg}: median {med:.3f} ms (best {best:.3f})")
+    M = Nc + Nf
+    idx = torch.sort(torch.rand(B, M, device="cuda"), -1).indices
+    rgb_c = torch.rand(B * Nc, 3, device="cuda", requires_grad=True)
+    rgb_f = torch.rand(B * Nf, 3, device="cuda", requires_grad=True)
+    s_c = torch.rand(B * Nc, 1, device="cuda", requires_grad=True)
+    s_f = torch.rand(B * Nf, 1, device="cuda", requires_grad=True)
+
+    def gather():
+        out = _gather(rgb_c, rgb_f, idx).sum() + _gather(s_c, s_f, idx).sum()
+        torch.autograd.grad(out, [rgb_c, rgb_f, s_c, s_f])
+    med, best = timeit(gather, n=20, warm=3)
+    print(f"merged-order gather of rgb + sigma, forward + backward, B={B} {Nc}+{Nf}: median {med:.3f} ms")
+    # (3) quality at a fixed step budget
+    for radius, lr in ((0.6, 5e-4), (1.2, 1e-3)):
+        def sphere(o, d):
+            b = (o * d).sum(-1)
+            disc = b * b - ((o * o).sum(-1) - radius ** 2)
+            n = (o + d * (-b - torch.sqrt(disc.clamp_min(0)))[:, None]) / radius
+            col = torch.stack([0.5 + 0.5 * n[:, 2], 0.2 + 0.0 * n[:, 0], 0.5 - 0.5 * n[:, 2]], -1)
+            return torch.where((disc > 0)[:, None], col, torch.ones_like(col))
+        held_o, held_d, _ = (t.cuda() for t in synthetic.random_rays(16384, seed=9999))
+        held_t = sphere(held_o, held_d)
+        for leg in (f"hierarchical {Nc}+{Nf}", "stratified N=192", "stratified N=256"):
+            torch.manual_seed(0)
+            model = NeuralField(dict(mode="part2_nerf", L_embed=10, L_embed_dir=4)).cuda().train()
+            opt = torch.optim.Adam(model.parameters(), lr=lr)
+            hier = leg.startswith("hier")
+            torch.cuda.synchronize()
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            for step in range(1, quality_steps + 1):
+                o, d, _ = (t.cuda() for t in synthetic.random_rays(2048, seed=step))
+                tgt = sphere(o, d)
+                if hier:
+                    out = render_rays_hierarchical(model, o, d, 2.0, 6.0, Nc, Nf, True)
+                    loss = torch.nn.functional.mse_loss(out.color, tgt) + torch.nn.functional.mse_loss(out.coarse_color, tgt)
+                else:
+                    pred = render_rays(model, o, d, 2.0, 6.0, int(leg.split("=")[1]), True, white_bkgd=True)[0]
+                    loss = torch.nn.functional.mse_loss(pred, tgt)
+                opt.zero_grad()
+                loss.backward()
+                opt.step()
+            e1.record()
+            torch.cuda.synchronize()
+            model.eval()
+            with torch.no_grad():
+                if hier:
+                    out = render_rays_hierarchical(model, held_o, held_d, 2.0, 6.0, Nc, Nf, False)
+                    pred, coarse = out.color, out.coarse_color
+                else:
+                    pred = render_rays(model, held_o, held_d, 2.0, 6.0, int(leg.split("=")[1]), False)[0]
+                    coarse = None
+            psnr = -10 * torch.log10(((pred - held_t) ** 2).mean()).item()
+            extra = "" if coarse is None else f" (its coarse pass alone: {-10 * torch.log10(((coarse - held_t) ** 2).mean()).item():.2f} dB)"
+            print(f"sphere r={radius}, {quality_steps} steps of 2048 rays, Adam lr={lr}, {leg}: held-out PSNR {psnr:.2f} dB"
+                  f"{extra}, training {e0.elapsed_time(e1) / quality_steps:.3f} ms/step")
+    b2n.check_errors()
+
+
 def c1_step(P_rays=4096, N=64):
     """C1: vanilla NeRF training step (render_rays + MSE + backward + Adam), B=4096, N=64."""
     from b2n import synthetic
@@ -664,6 +805,8 @@ if __name__ == "__main__":
         mesh()
     elif what == "render":
         render()
+    elif what == "importance":
+        importance()
     elif what == "hashsort":
         hash_sorted()
     elif what == "hash":
