@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 19
+#define B2N_ABI_VERSION 20
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -511,6 +511,53 @@ int b2n_render_finish(const void* state, int64_t B, const float* bg, int bg_per_
 int b2n_importance_sample(const float* sigma, const float* z, const float* rays_d, const float* u_table,
                           const float* u_jitter, int64_t B, int Nc, int Nf, float* z_fine, float* z_merged,
                           int32_t* merge_src, b2n_stream_t stream);
+
+/* ------------------------------------------------------------------------
+ * Error-map ray sampling (b2n.errormap; DESIGN.md §5i): Instant-NGP's error map -- training pixels drawn in proportion
+ * to a coarse per-view map of recent loss, mixed with a uniform share.  Not part of the reference, whose rays are drawn
+ * uniformly (sample_random_rays, which is unchanged); an extension that is off unless asked for.
+ *   Map: V views of H x W pixels, each split into Hm x Wm cells, 1 <= Hm <= H, 1 <= Wm <= W, n = V*Hm*Wm < 2^31.
+ *     Pixel (v, y, x) lies in cell c = (v*Hm + floor(y*Hm/H))*Wm + floor(x*Wm/W) (integer arithmetic); cell row i covers
+ *     the pixel rows [ceil(i*H/Hm), ceil((i+1)*H/Hm)), n_y of them (neighbours differ by at most one); columns alike.
+ *     e [n] fp32, -1 = never observed (the caller's initial value).  Accumulators acc_sum [n] uint64, acc_cnt [n] uint32,
+ *     zero between updates (the caller zeroes them once; b2n_errormap_apply leaves them zero).
+ *   b2n_errormap_accumulate: for each ray r < B (B < 2^31), the pick (img_idx, pix_y, pix_x)[r] (int64, each clamped
+ *     into [0, V-1] x [0, H-1] x [0, W-1]) and err[r] fp32: s = isfinite(err) ? min(max(err, 0), 1) : 0,
+ *     q = rint(s * 2^24) (exact), acc_sum[c] += q, acc_cnt[c] += 1 with integer atomics: the sums do not depend on the
+ *     order of the rays, nor on how a batch is split across calls or ranks.  Over all calls between two applies the
+ *     rays of one cell must number < 2^32.  One kernel.
+ *   b2n_errormap_apply: for every cell with acc_cnt > 0: m = (float)((double)acc_sum * 2^-24 / acc_cnt),
+ *     e = e < 0 ? m : (1 - beta) * e + beta * m (fp32, each operation rounded separately), then acc_sum = acc_cnt = 0.
+ *     Cells with acc_cnt == 0 are not touched.  0 <= beta <= 1.  One kernel.
+ *   b2n_errormap_cdf: w_c = max(e_c, 0) (a NaN cell weighs 0), cdf [n] fp64 = the inclusive prefix of w in a fixed
+ *     association: a running sum over each run of 16 cells; the runs of a 4096-cell block chained in order (each run's
+ *     offset = the previous offset + the previous run's sum); the blocks chained the same way; cdf = block offset +
+ *     (run offset + running sum).  Every addition is an fp64 add rounded to nearest, so the CDF is non-decreasing and a
+ *     cell of weight 0 has cdf[c] == cdf[c-1] exactly.  S = cdf[n-1].  scratch: b2n_errormap_scratch(V, Hm, Wm) bytes
+ *     (0 for an invalid map).  Three kernels.
+ *   b2n_errormap_sample: u [B,3] fp32 (drawn by the caller; never in the kernel), lam = uniform_frac in [0, 1], N = V*H*W.
+ *     The map is used iff lam < 1 and 0 < S < inf.  Not used, or u0 < lam: the pixel index k = floor(f * N), f = u0
+ *     (map not used) or u0 / lam, is split as k = (v*H + y)*W + x.  Otherwise the cell c = the number of cdf entries
+ *     <= t, t = (u0 - lam) / (1 - lam) * S (searchsorted(cdf, t, right=True)); t < S for every u0 < 1, and t >= S or
+ *     NaN takes the last cell of positive weight.  Inside the cell, y = y_lo + min(floor(u1 * n_y), n_y - 1), x alike
+ *     from u2.  All arithmetic on u is fp64 from the fp32 inputs; every floor is clamped into range and a NaN gives 0,
+ *     so any u (0, 1, NaN) and any map (inf, NaN) give in-range picks.  Outputs img_idx, pix_y, pix_x [B] int64 (the
+ *     inputs of b2n_sample_rays) and ratio [B] fp32 = 1 / (N * p(v,y,x)) with
+ *     p = lam / N + (1 - lam) * w_c / (S * n_y * n_x) when the map is used (ratio = 1 when it is not): the weight that
+ *     makes a per-ray loss unbiased when lam > 0 (with lam = 0 the pixels of weight-0 cells have p = 0 and are never
+ *     drawn).  It is only returned, never applied.  V*H*W < 2^53.  One kernel.
+ * Every argument is checked before any launch.  No float atomics, no host synchronisation (capturable in a CUDA graph),
+ * deterministic: two runs give the same bits. */
+size_t b2n_errormap_scratch(int V, int Hm, int Wm);
+int b2n_errormap_accumulate(const int64_t* img_idx, const int64_t* pix_y, const int64_t* pix_x, const float* err,
+                            int64_t B, int V, int H, int W, int Hm, int Wm, uint64_t* acc_sum, uint32_t* acc_cnt,
+                            b2n_stream_t stream);
+int b2n_errormap_apply(float* e, uint64_t* acc_sum, uint32_t* acc_cnt, int V, int Hm, int Wm, float beta,
+                       b2n_stream_t stream);
+int b2n_errormap_cdf(const float* e, int V, int Hm, int Wm, double* cdf, void* scratch, b2n_stream_t stream);
+int b2n_errormap_sample(const float* e, const double* cdf, const float* u, int64_t B, int V, int H, int W, int Hm,
+                        int Wm, float uniform_frac, int64_t* img_idx, int64_t* pix_y, int64_t* pix_x, float* ratio,
+                        b2n_stream_t stream);
 
 #ifdef __cplusplus
 }

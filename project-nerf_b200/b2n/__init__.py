@@ -7,6 +7,7 @@ from . import _lib  # noqa: F401  (fails loudly when the .so is missing)
 from .ops import (HashGeometry, check_errors, composite, fourier_encode, fused_mlp, hash_encode, instant_mlp, instant_sigma, linear,  # noqa: F401
                   mlp_precision,
                   set_mlp_precision, sigma_head)
-from . import checkpoint, graphs, importance, march, mesh, ops, optim, render  # noqa: F401
+from . import checkpoint, errormap, graphs, importance, march, mesh, ops, optim, render  # noqa: F401
+from .errormap import ErrorMap  # noqa: F401
 from .importance import Hierarchical, render_image_hierarchical, render_rays_hierarchical  # noqa: F401
 from .render import Rendered, render_image_fast, render_rays_fast  # noqa: F401

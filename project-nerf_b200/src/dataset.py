@@ -131,8 +131,10 @@ class BlenderDataset:
                  torch.randint(0, self.W, (batch_size,)))
         return picks
 
-    def _sample(self, batch_size, device, with_time):
-        img_idx, pix_y, pix_x = self._draw(batch_size, device)
+    def _sample(self, batch_size, device, with_time, picks=None):
+        """rays for ``picks`` = (img_idx, pix_y, pix_x) int64 [batch_size] (in range: b2n_sample_rays does not check
+        them), or for a fresh uniform draw when None"""
+        img_idx, pix_y, pix_x = self._draw(batch_size, device) if picks is None else picks
         dev = torch.device(device)
         if dev.type == "cuda":
             from b2n._lib import call, ptr, stream

@@ -490,6 +490,112 @@ def importance(Nc=64, Nf=128, quality_steps=1000):
     b2n.check_errors()
 
 
+def _band_scene(ro, rd, radius=0.6, band=0.25):
+    """the checker-band sphere of tests/test_gpu_errormap.py: a shaded sphere with a 24 x 6 black-and-white checker on
+    the latitude band |n_z| < band, white background; returns (colour [B,3], on-band mask [B])"""
+    b = (ro * rd).sum(-1)
+    disc = b * b - ((ro * ro).sum(-1) - radius ** 2)
+    hit = disc > 0
+    n = (ro + rd * (-b - torch.sqrt(disc.clamp_min(0)))[:, None]) / radius
+    col = torch.stack([0.5 + 0.5 * n[:, 2], 0.2 + 0.0 * n[:, 0], 0.5 - 0.5 * n[:, 2]], -1)
+    on = hit & (n[:, 2].abs() < band)
+    az = torch.atan2(n[:, 1], n[:, 0])
+    check = ((torch.floor(az * 24 / (2 * 3.141592653589793)) + torch.floor(n[:, 2] * 6 / (2 * band))) % 2)
+    col = torch.where(on[:, None], check[:, None].expand(-1, 3), col)
+    return torch.where(hit[:, None], col, torch.ones_like(col)), on
+
+
+def errormap(steps=2000, B_train=8192):
+    """Error-map sampling (b2n.errormap, DESIGN.md §5i): (1) sample + update at the C2 size (2^18 rays, 100 views of
+    800^2, 128^2 cells per view) against the 21.5 ms C2 step; (2) held-out PSNR after a fixed number of steps on the
+    checker-band sphere, Instant model, uniform picks against the error map at uniform_frac = 0.25 (unweighted loss,
+    as Instant-NGP), with the step time of each leg: PSNR over every training pixel (what the sampler spends its rays
+    on) and over held-out views."""
+    from b2n import synthetic
+    from b2n.errormap import ErrorMap
+    from src.renderer import render_rays
+    _device_line()
+    # (1) the sampler at C2 size, the map filled by a few updates first (an all-unobserved map samples uniformly)
+    V, H, W, B = 100, 800, 800, 2 ** 18
+    emap = ErrorMap(V, H, W)
+    gen = torch.Generator(device="cuda").manual_seed(0)
+    for _ in range(20):
+        picks, _ = emap.sample(B, generator=gen)
+        emap.update(picks, torch.rand(B, device="cuda", generator=gen))
+    picks, _ = emap.sample(B, generator=gen)
+    err = torch.rand(B, device="cuda", generator=gen)
+    n = emap.cdf.numel()
+    print(f"map {V} x {H} x {W}, cells {emap.Hm} x {emap.Wm} ({n} cells, CDF {n * 8 / 1e6:.1f} MB), B = {B}; "
+          f"{int((emap.e >= 0).sum())} cells observed")
+    t_s, b_s = timeit(lambda: emap.sample(B, generator=gen), n=50, warm=5)
+    t_u, b_u = timeit(lambda: emap.update(picks, err), n=50, warm=5)
+    t_c, _ = timeit(emap.rebuild_cdf, n=50, warm=5)
+
+    def both():
+        p, _ = emap.sample(B, generator=gen)
+        emap.update(p, err)
+    t_b, b_b = timeit(both, n=50, warm=5)
+    print(f"sample (torch.rand + 1 kernel): median {t_s:.4f} ms (best {b_s:.4f})")
+    print(f"update (accumulate + apply + CDF, 5 kernels): median {t_u:.4f} ms (best {b_u:.4f}); of it the CDF "
+          f"rebuild alone {t_c:.4f} ms ({n * 16 / t_c / 1e6:.0f} GB/s of its {n * 16 / 1e6:.1f} MB)")
+    print(f"sample + update: median {t_b:.4f} ms (best {b_b:.4f}) = {100 * t_b / 21.5:.2f} % of the 21.5 ms C2 step")
+    # (2) quality at a fixed step budget on the checker-band sphere
+    b2n.set_mlp_precision("bf16")
+    Vt, Ht = 100, 128
+    cfg = dict(mode="part2_instant", n_levels=12, n_features_per_level=2, log2_hashmap_size=17, base_resolution=16,
+               per_level_scale=1.5, scene_bound=1.5, L_embed_dir=4, hidden_dim=64)
+
+    def views(nv, seed):
+        poses = synthetic.hemisphere_poses(nv, seed=seed)
+        ro, rd = zip(*(synthetic.image_rays(p, H=Ht, W=Ht) for p in poses))
+        ro, rd = torch.stack(ro).cuda(), torch.stack(rd).cuda()
+        tgt, on = _band_scene(ro.reshape(-1, 3), rd.reshape(-1, 3))
+        return ro, rd, tgt.reshape(nv, Ht * Ht, 3), on
+    tr_o, tr_d, tr_t, tr_on = views(Vt, 21)
+    he_o, he_d, he_t, he_on = views(8, 22)
+    bg = torch.ones(3, device="cuda")
+
+    def psnr(model, o, d, t, on):
+        o, d, t = o.reshape(-1, 3), d.reshape(-1, 3), t.reshape(-1, 3)
+        with torch.no_grad():
+            pred = torch.cat([render_rays(model, o[i:i + 2 ** 15], d[i:i + 2 ** 15], 2.0, 6.0, 64, False,
+                                          bg_color=bg)[0] for i in range(0, o.shape[0], 2 ** 15)])
+        mse = ((pred - t) ** 2).mean(-1)
+        return -10 * torch.log10(mse.mean()).item(), -10 * torch.log10(mse[on].mean()).item()
+    for leg in ("uniform", "error map, uniform_frac=0.25"):
+        torch.manual_seed(0)
+        model = NeuralField(cfg).cuda().train()
+        opt = torch.optim.AdamW(model.parameters(), lr=1e-2, weight_decay=1e-5)
+        em = ErrorMap(Vt, Ht, Ht, cells=(32, 32), uniform_frac=0.25)
+        g = torch.Generator(device="cuda").manual_seed(1)
+        use_map = leg.startswith("error")
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(steps):
+            if use_map:
+                (v, y, x), _ = em.sample(B_train, generator=g)
+            else:
+                v, y, x = (torch.randint(0, k, (B_train,), device="cuda", generator=g) for k in (Vt, Ht, Ht))
+            k = y * Ht + x
+            pred = render_rays(model, tr_o[v, k], tr_d[v, k], 2.0, 6.0, 64, True, bg_color=bg)[0]
+            per_ray = ((pred - tr_t[v, k]) ** 2).mean(-1)
+            opt.zero_grad()
+            per_ray.mean().backward()
+            opt.step()
+            if use_map:
+                em.update((v, y, x), per_ray.detach())
+        e1.record()
+        torch.cuda.synchronize()
+        model.eval()
+        fit, fit_band = psnr(model, tr_o, tr_d, tr_t, tr_on)
+        held, held_band = psnr(model, he_o, he_d, he_t, he_on)
+        print(f"checker-band sphere, {Vt} views of {Ht}^2, {steps} steps of {B_train} rays, Instant model, {leg}: "
+              f"PSNR over all training pixels {fit:.2f} dB (band {fit_band:.2f}), held-out {held:.2f} dB "
+              f"(band {held_band:.2f}), {e0.elapsed_time(e1) / steps:.3f} ms/step")
+    b2n.check_errors()
+
+
 def c1_step(P_rays=4096, N=64):
     """C1: vanilla NeRF training step (render_rays + MSE + backward + Adam), B=4096, N=64."""
     from b2n import synthetic
@@ -807,6 +913,8 @@ if __name__ == "__main__":
         render()
     elif what == "importance":
         importance()
+    elif what == "errormap":
+        errormap()
     elif what == "hashsort":
         hash_sorted()
     elif what == "hash":
