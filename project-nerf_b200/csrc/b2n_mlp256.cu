@@ -62,9 +62,12 @@
 #include <string.h>
 #include <cuda_bf16.h>
 #include "b2n_common.cuh"
+#include "b2n_tc.cuh"
 
 namespace b2n {
 namespace m256 {
+
+using namespace tc;
 
 constexpr int HID = 256;
 constexpr int KBLK_BYTES = 128 * 128;          // one k-block of one tile: 128 rows x 64 bf16
@@ -103,144 +106,6 @@ struct Plan {
   int n_steps;
   Step s[MAX_STEPS];
 };
-
-// ---------------------------------------------------------------------------------------- PTX
-__device__ __forceinline__ uint32_t s32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
-}
-// bounded wait: false = aborted (either this wait timed out or another role raised the flag)
-__device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity, volatile int* abort_flag, int* err, int code) {
-#pragma unroll 1
-  for (uint32_t it = 0; it < (1u << 22); ++it) {
-    if (mbar_try(bar, parity)) return true;
-    if ((it & 255) == 255 && *abort_flag) return false;
-  }
-  *abort_flag = 1;
-  atomicCAS(err, 0, code);
-  return false;
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-// one lane of a converged warp (warp-uniform control flow keeps descriptors in uniform registers)
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tc_mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc) : "memory");
-}
-// ---- CTA-pair (cta_group::2) variants: one MMA spans two SMs (M = 256: 128 rows per CTA; each CTA supplies half of B)
-__device__ __forceinline__ void tc_mma2(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(acc) : "memory");
-}
-// arrives on the barrier at the same shared-memory offset in BOTH CTAs of the pair once all prior MMAs are complete
-__device__ __forceinline__ void tc_commit2(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t cluster_idx() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%clusterid.x;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ uint32_t cluster_count() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%nclusterid.x;" : "=r"(r));
-  return r;
-}
-// shared::cluster address of `saddr` (a shared::cta address of this CTA) in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa(uint32_t saddr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// Remote arrive with the default (.release.cta) semantics, as CUTLASS's ClusterBarrier::arrive(cta_id) does.  What crosses
-// the CTA boundary here is shared memory only (the peer's activation tile, read by the leader's tensor core), which no
-// cache sits in front of; the explicit `.release.cluster` form compiles to MEMBAR.ALL.GPU and the matching
-// `try_wait.acquire.cluster` to CCTL.IVALL (an L1 flush) per wait -- together ~2000 cycles per tile and step (B2N_TRACE).
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA tile load issued by either CTA of a pair; the transaction bytes are credited to `mbar_cluster`, which may live in
-// the other CTA (the leader's "weights landed" barrier)
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const void* tmap, int x, int y, uint32_t mbar_cluster) {
-  asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               ::"r"(dst), "l"(tmap), "r"(x), "r"(y), "r"(mbar_cluster) : "memory");
-}
-__device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-        "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-        "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-        "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-      : "r"(taddr) : "memory");
-}
-// TMA tensor store of one swizzled [128 rows x 64 bf16] k-block: smem -> planes[slot][row0.., col0..col0+63]
-__device__ __forceinline__ void tma_store_3d(const void* tmap, uint32_t smem_src, int col0, int row0, int slot) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(tmap), "r"(smem_src), "r"(col0), "r"(row0), "r"(slot) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void tc_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// K-major SWIZZLE_128B shared-memory matrix descriptor: rows of 128 B, 8-row atoms 1024 B apart.
-__device__ __forceinline__ uint64_t umma_desc(uint32_t saddr) {
-  return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-         ((uint64_t)2 << 61);
-}
-// kind::f16 instruction descriptor: D = fp32, A = B = bf16, both K-major, M = 128 (256 for a CTA pair)
-__device__ __forceinline__ uint32_t umma_idesc(int n, int m = 128) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-// byte offset of 16-byte chunk c (0..7) of row r inside a swizzled 128-row x 128-byte block
-__device__ __forceinline__ uint32_t swz(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
 
 __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
@@ -355,22 +220,16 @@ __global__ void __launch_bounds__(N_THREADS, 1) k_mlp256(const __grid_constant__
       mbar_init(bar_tail + 8 * t, EPI_THREADS);
     }
     *abort_flag = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
   if (CTA2) {
     cluster_sync_all();                         // both CTAs resident, barriers initialised, before anything crosses over
-    if (warp == 1) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512));
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
-    }
+    if (warp == 1) tmem_alloc2(s32(tmem_slot), 512);
     tc_fence_before();
     cluster_sync_all();
     tc_fence_after();
   } else {
-    if (warp == 1) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512));
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
+    if (warp == 1) tmem_alloc(s32(tmem_slot), 512);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -450,7 +309,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) k_mlp256(const __grid_constant__
     // The whole warp walks the (warp-uniform) schedule; one elected lane issues the tcgen05 ops.
     {
       uint32_t use = 0, act_phase[2] = {0, 0};
-      const uint32_t idesc = umma_idesc(128);
+      const uint32_t idesc = umma_idesc(Fmt::BF16, Major::K, 128, 128);
       const uint32_t ring0 = s32(smem + RING), act0 = s32(smem + OFF_ACT), aux0 = s32(smem + OFF_AUX);
       for (int64_t pair = pair_first; pair < n_pairs; pair += pair_step) {
         for (int s = 0; s < plan.n_steps; ++s) {
@@ -471,7 +330,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) k_mlp256(const __grid_constant__
               // leader: one M = 256 x N = layer-width MMA per k16 over both CTAs' tiles; the peer's warp only does the
               // plane stores of its own tile
               if (rank == 0) {
-                const uint32_t idesc2 = umma_idesc(plan.s[s].n, 256);
+                const uint32_t idesc2 = umma_idesc(Fmt::BF16, Major::K, plan.s[s].n, 256);
                 const bool shared = nkc <= NST;      // both tiles read the same ring slots (see the producer)
                 const uint32_t use0 = use;
                 for (int c = 0; c < nkc; ++c) {
@@ -859,13 +718,11 @@ __global__ void __launch_bounds__(N_THREADS, 1) k_mlp256(const __grid_constant__
   if (CTA2) {
     tc_fence_before();
     cluster_sync_all();       // nothing of this CTA (barriers, TMEM, tiles) is touched by the peer after this point
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
+    if (warp == 1) tmem_dealloc2(tmem, 512);
     return;
   }
   __syncthreads();
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
-  }
+  if (warp == 1) tmem_dealloc(tmem, 512);
 }
 
 // ---------------------------------------------------------------------------------------- weight packing

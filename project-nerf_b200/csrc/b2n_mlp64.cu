@@ -284,15 +284,12 @@ k_instant_bwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
     reinterpret_cast<uint4*>(smem)[i] = make_uint4(0u, 0u, 0u, 0u);
   if (threadIdx.x == 0) {
     for (int i = 0; i < GROUPS; ++i) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s32(bars + i)), "r"(1));
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s32(bars + GROUPS + i)), "r"(MLP_THREADS));
+      mbar_init(s32(bars + i), 1);
+      mbar_init(s32(bars + GROUPS + i), MLP_THREADS);
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (threadIdx.x < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (threadIdx.x < 32) tmem_alloc(s32(tmem_slot), TMEM_COLS);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -304,13 +301,14 @@ k_instant_bwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
   // the 12 weight-gradient MMAs of one staged tile group + the commit that hands the slots back
   auto issue_wgrad = [&](int grp, uint32_t acc_first) {
     const uint32_t base = s32(smem) + grp * SL::N * SLOT;
+    const uint32_t id128 = umma_idesc(Fmt::F16, Major::MN, 128, 128), id64 = umma_idesc(Fmt::F16, Major::MN, 64, 128);
 #pragma unroll
     for (int kk = 0; kk < 4; ++kk) {
       const uint32_t o = base + kk * 2048;
       const uint32_t acc = (acc_first | (uint32_t)kk) ? 1u : 0u;
-      tc_mma(tmem + D1, umma_desc_mn(o + SL::DZ3 * SLOT, SLOT), umma_desc_mn(o + SL::C * SLOT, SLOT), umma_idesc_mn(128), acc);
-      tc_mma(tmem + D2, umma_desc_mn(o + SL::A2 * SLOT, SLOT), umma_desc_mn(o + SL::B2 * SLOT, SLOT), umma_idesc_mn(64), acc);
-      tc_mma(tmem + D3, umma_desc_mn(o + SL::A3 * SLOT, SLOT), umma_desc_mn(o + SL::B3 * SLOT, SLOT), umma_idesc_mn(64), acc);
+      tc_mma(tmem + D1, umma_desc_mn(o + SL::DZ3 * SLOT, SLOT), umma_desc_mn(o + SL::C * SLOT, SLOT), id128, acc);
+      tc_mma(tmem + D2, umma_desc_mn(o + SL::A2 * SLOT, SLOT), umma_desc_mn(o + SL::B2 * SLOT, SLOT), id64, acc);
+      tc_mma(tmem + D3, umma_desc_mn(o + SL::A3 * SLOT, SLOT), umma_desc_mn(o + SL::B3 * SLOT, SLOT), id64, acc);
     }
     tc_commit(s32(bars + grp));
   };
@@ -512,7 +510,7 @@ k_instant_bwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
           issue_wgrad(0, pending ? 1u : 0u);
         }
       } else {
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar_full) : "memory");      // release: the issuer acquires
+        mbar_arrive(bar_full);      // release: the issuer acquires
       }
       pending = true;
       if (g_x) {                   // d x_enc: registers + weights only, overlaps the MMAs
@@ -588,7 +586,7 @@ k_instant_bwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
   }
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
+  if (threadIdx.x < 32) tmem_dealloc(tmem, TMEM_COLS);
 }
 
 }  // namespace b2n

@@ -135,13 +135,10 @@ k_instant_fwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
     stage_weight(cp + 64 * 48 + 64 * 64, 16, 64, 16, smem + M::V3, false);
   }
   if (tid == 0) {
-    for (int s = 0; s < NS; ++s) asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s32(bars + s)), "r"(1));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    for (int s = 0; s < NS; ++s) mbar_init(s32(bars + s), 1);
+    mbar_init_fence();
   }
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(64 * NS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
+  if (warp == 0) tmem_alloc(s32(tmem_slot), 64 * NS);
   proxy_fence();
   tc_fence_before();
   __syncthreads();
@@ -199,7 +196,7 @@ k_instant_fwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
     const uint32_t a0 = a_base + s * M::SLOT, a1 = a0 + A_BYTES, acc = tmem + 64 * s;
     tc_fence_after();
     if (layer == 0) {            // sigma_net layer 1: split product, small terms first
-      const uint32_t id = umma_idesc(64);
+      const uint32_t id = umma_idesc(Fmt::F16, Major::K, 64, 128);
       // x_lo W_hi: the merged tile holds x_lo in its upper 32 columns, facing the second copy of W_hi
 #pragma unroll
       for (int k = 0; k < KS1; ++k)
@@ -211,7 +208,7 @@ k_instant_fwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
     } else {
       // 1: sigma_net layer 2 (64 -> 16)   2: color_net layer 1 (48 -> 64)   3: color_net layer 2   4: output layer (64 -> 3 of 16)
       const uint32_t w = layer == 1 ? w2 : (layer == 2 ? v1 : (layer == 3 ? v2 : v3));
-      const uint32_t id = umma_idesc((layer == 1 || layer == 4) ? 16 : 64);
+      const uint32_t id = umma_idesc(Fmt::F16, Major::K, (layer == 1 || layer == 4) ? 16 : 64, 128);
       const int ks = layer == 2 ? 3 : 4;
       for (int k = 0; k < ks; ++k) tc_mma(acc, umma_desc(a0) + 2 * k, umma_desc(w) + 2 * k, id, k > 0);
     }
@@ -329,7 +326,7 @@ k_instant_fwd_tc(const float* __restrict__ x, int ldx, int pos_dim, const float*
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(64 * NS));
+  if (warp == 0) tmem_dealloc(tmem, 64 * NS);
 }
 
 }  // namespace itc

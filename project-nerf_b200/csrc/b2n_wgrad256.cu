@@ -18,9 +18,12 @@
 #include <cuda_fp16.h>
 #include <string.h>
 #include "b2n_common.cuh"
+#include "b2n_tc.cuh"
 
 namespace b2n {
 namespace wg256 {
+
+using namespace tc;
 
 constexpr int TP = 64;                         // points per stage
 constexpr int BLK = TP * 128;                  // one 64-column operand block: 64 rows x 128 B
@@ -51,34 +54,6 @@ struct Args {
   const int* rows;          // optional device-side row count; rows up to the next multiple of 64 behind it are zero in the planes
 };
 
-__device__ __forceinline__ uint32_t s32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-               : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-  return ok != 0;
-}
-// bounded wait: a protocol bug must not hang the GPU
-__device__ __forceinline__ bool mbar_wait(uint32_t bar, uint32_t parity, volatile int* abort_flag, int* err, int code) {
-#pragma unroll 1
-  for (uint32_t it = 0; it < (1u << 24); ++it) {
-    if (mbar_try(bar, parity)) return true;
-    if ((it & 1023) == 1023 && *abort_flag) return false;
-  }
-  *abort_flag = 1;
-  atomicCAS(err, 0, code);
-  return false;
-}
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const void* tmap, int c0, int c1, int c2, uint32_t bar) {
-  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-               ::"r"(dst), "l"(tmap), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
-}
-// MN-major SWIZZLE_128B operand: 64-column blocks BLK bytes apart, 8-row groups 1024 B apart
-__device__ __forceinline__ uint64_t mn_desc(uint32_t saddr) {
-  return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((BLK >> 4) & 0x3FFF) << 16) | ((uint64_t)(1024 >> 4) << 32) |
-         ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
-}
-
 __global__ void __launch_bounds__(N_THREADS, 1)
 k_wgrad256(const Args a, const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUtensorMap tm1,
            const __grid_constant__ CUtensorMap tm2, const __grid_constant__ CUtensorMap tm3) {
@@ -99,20 +74,17 @@ k_wgrad256(const Args a, const __grid_constant__ CUtensorMap tm0, const __grid_c
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < N_STAGES; ++i) {
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar_full + 8 * i), "r"(1));
-      asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar_empty + 8 * i), "r"(gemm ? 9 : 8));
+      mbar_init(bar_full + 8 * i, 1);
+      mbar_init(bar_empty + 8 * i, gemm ? 9 : 8);
     }
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar_done), "r"(1));
+    mbar_init(bar_done, 1);
     *abort_flag = 0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_init_fence();
   }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(tmem_slot)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 1) tmem_alloc(s32(tmem_slot), 512);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem = *tmem_slot;
 
   if (warp == 0) {
@@ -122,7 +94,7 @@ k_wgrad256(const Args a, const __grid_constant__ CUtensorMap tm0, const __grid_c
         const int st = it % N_STAGES;
         if (!mbar_wait(bar_empty + 8 * st, ((it / N_STAGES) & 1) ^ 1, abort_flag, a.err, 1)) break;
         const uint32_t bytes = (uint32_t)(dz_blocks + in_blocks) * BLK;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar_full + 8 * st), "r"(bytes) : "memory");
+        mbar_expect_tx(bar_full + 8 * st, bytes);
         const int r0 = (int)(row_begin + (int64_t)it * TP);
         const uint32_t base = s32(smem + st * STAGE_BYTES);
         auto pick = [&](int i) { return i == 0 ? &tm0 : (i == 1 ? &tm1 : (i == 2 ? &tm2 : &tm3)); };
@@ -137,29 +109,23 @@ k_wgrad256(const Args a, const __grid_constant__ CUtensorMap tm0, const __grid_c
   } else if (warp == 1) {
     // ================================ MMA issuer ================================
     if (gemm) {
-      // instruction descriptor: D fp32, A = B = bf16, both MN-major, M = 128, N = n_cols
-      const uint32_t ab_fmt = a.fp16 ? 0u : ((1u << 7) | (1u << 10));      // a_format / b_format: 0 = f16, 1 = bf16
-      const uint32_t idesc = (1u << 4) | ab_fmt | (1u << 15) | (1u << 16) | ((uint32_t)(job.n_cols >> 3) << 17) |
-                             ((uint32_t)(128 >> 4) << 24);
+      const uint32_t idesc = umma_idesc(a.fp16 ? Fmt::F16 : Fmt::BF16, Major::MN, job.n_cols, 128);
       for (int it = 0; it < n_steps; ++it) {
         const int st = it % N_STAGES;
         if (!mbar_wait(bar_full + 8 * st, (it / N_STAGES) & 1, abort_flag, a.err, 2)) break;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (lane == 0) {
           const uint32_t base = s32(smem + st * STAGE_BYTES);
 #pragma unroll
           for (int kk = 0; kk < TP / 16; ++kk) {
             for (int mh = 0; mh < job.m_halves; ++mh) {
-              const uint64_t ad = mn_desc(base + mh * 2 * BLK + kk * 2048);      // dZ columns 128*mh .. +127
-              const uint64_t bd = mn_desc(base + 4 * BLK + kk * 2048);           // input columns 0 .. n_cols-1
-              const uint32_t acc = (it > 0 || kk > 0) ? 1u : 0u;
-              asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                           ::"r"(tmem + mh * 256), "l"(ad), "l"(bd), "r"(idesc), "r"(acc) : "memory");
+              const uint64_t ad = umma_desc_mn(base + mh * 2 * BLK + kk * 2048, BLK);      // dZ columns 128*mh .. +127
+              const uint64_t bd = umma_desc_mn(base + 4 * BLK + kk * 2048, BLK);           // input columns 0 .. n_cols-1
+              tc_mma(tmem + mh * 256, ad, bd, idesc, (it > 0 || kk > 0) ? 1u : 0u);
             }
           }
-          asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_empty + 8 * st) : "memory");
-          if (it + 1 == n_steps)
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_done) : "memory");
+          tc_commit(bar_empty + 8 * st);
+          if (it + 1 == n_steps) tc_commit(bar_done);
         }
         __syncwarp();
       }
@@ -188,27 +154,19 @@ k_wgrad256(const Args a, const __grid_constant__ CUtensorMap tm0, const __grid_c
         colsum += s;
       }
       __syncwarp();
-      if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar_empty + 8 * st) : "memory");
+      if (lane == 0) mbar_arrive(bar_empty + 8 * st);
     }
     if (job.db && n_steps > 0 && c < job.bias_cols) atomicAdd(job.db + c, colsum * inv_s);
     if (gemm && n_steps > 0 && mbar_wait(bar_done, 0, abort_flag, a.err, 4)) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const int q = warp & 3;                   // TMEM lane quarter this warp may read
       const int mh = (warp - 2) >> 2;           // which dZ column half (accumulator columns 256*mh ..)
       const int n = 128 * mh + 32 * q + lane;   // output neuron = dW row
       float* drow = job.dW + (size_t)n * job.n_cols;
       for (int c0 = 0; mh < job.m_halves && c0 < job.n_cols; c0 += 32) {
         uint32_t v[32];
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-            "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-            "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-              "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-              "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-              "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-            : "r"(tmem + ((uint32_t)(32 * q) << 16) + 256 * mh + c0) : "memory");
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tc_ld32(tmem + ((uint32_t)(32 * q) << 16) + 256 * mh + c0, v);
+        tc_ld_wait();
 #pragma unroll
         for (int j = 0; j < 32; j += 4)
           atomicAdd(reinterpret_cast<float4*>(drow + c0 + j),
@@ -217,9 +175,9 @@ k_wgrad256(const Args a, const __grid_constant__ CUtensorMap tm0, const __grid_c
       }
     }
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
+  if (warp == 1) tmem_dealloc(tmem, 512);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
