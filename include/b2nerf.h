@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define B2N_ABI_VERSION 20
+#define B2N_ABI_VERSION 21
 
 #define B2N_OK 0
 #define B2N_EINVAL (-1)  /* bad argument (null pointer, size, unsupported shape) */
@@ -43,7 +43,7 @@ const char* b2n_last_error(void);
  * behind an occupancy grid runs with fixed-capacity buffers and no device->host read of the active-sample count
  * (the reference reads it three times per call: src/renderer.py:309-323), which makes the step CUDA-graph capturable.
  * Honoured by: b2n_pe_*, b2n_hash_*, b2n_instant_mlp_*, b2n_fmlp_* (the saved planes get zero rows up to the next
- * multiple of 64 behind the count).  NOT honoured by the fp32 b2n_linear_* / b2n_sigma_head_* and the 256-wide
+ * multiple of 64 behind the count), b2n_distortion_*.  NOT honoured by the fp32 b2n_linear_* / b2n_sigma_head_* and the 256-wide
  * b2n_nerf_mlp_* entry points; b2n_composite_* / b2n_march_* index samples through ray offsets and do not need it. */
 int b2n_set_active_rows(const int* rows_device);
 
@@ -558,6 +558,35 @@ int b2n_errormap_cdf(const float* e, int V, int Hm, int Wm, double* cdf, void* s
 int b2n_errormap_sample(const float* e, const double* cdf, const float* u, int64_t B, int V, int H, int W, int Hm,
                         int Wm, float uniform_frac, int64_t* img_idx, int64_t* pix_y, int64_t* pix_x, float* ratio,
                         b2n_stream_t stream);
+
+/* ------------------------------------------------------------------------
+ * Distortion loss (b2n.distortion; DESIGN.md §5j): the regulariser of mip-NeRF 360 (Barron et al. 2022, eq. 15), which
+ * pulls the weights of a ray together into one compact interval.  Not part of the reference, which has no such term;
+ * an extension that is off unless asked for.
+ * Per ray r < B, with depths z [B,N] (non-decreasing, z[N-1] <= far, as b2n_march_mask and the importance merge give
+ * them), sigma in the sample layout of b2n_composite_* (dense [B*N], or compact through mask_words + ray_offset of
+ * b2n_march_mask / b2n_march_scan; an inactive sample has sigma = 0) and |d| = ||rays_d[r]||:
+ *   Weights, exactly those of b2n_composite_fwd: tau_i = (z_{i+1} - z_i) * |d| (1e10 * |d| for i = N-1),
+ *     alpha_i = 1 - exp(-sigma_i * tau_i), T_0 = 1, T_{i+1} = T_i * (1 - alpha_i + 1e-10), w_i = alpha_i * T_i.
+ *     (Unlike b2n_composite_fwd, N == 1 is not special: its one weight is alpha_0.)
+ *   Intervals in normalised distance s = (z - near) / (far - near): sample i owns [s_i, s_{i+1}] with s_N = 1 (z_N =
+ *     far), midpoint m_i = (s_i + s_{i+1}) / 2, width d_i = s_{i+1} - s_i.
+ *   loss[r] = sum_i sum_j w_i w_j |m_i - m_j| + 1/3 sum_i w_i^2 d_i, computed in the O(N) form
+ *     2 sum_i w_i (m_i W_{<i} - WM_{<i}) + 1/3 sum_i w_i^2 d_i (exclusive prefix sums W of w, WM of w * m).
+ *   Backward: g_sigma (same layout as sigma; only active samples are written) = g_loss[r] times the exact gradient
+ *     w.r.t. sigma: dL/dw_i = 2 (m_i W_{<i} - WM_{<i} + WM_{>i} - m_i W_{>i}) + 2/3 w_i d_i, taken through the weights
+ *     above (the 1e-10 included) by the reverse scan of b2n_composite_bwd.  z, rays_d, near and far get no gradient.
+ *     The weights are recomputed: nothing but the inputs is needed.
+ * Limits: B >= 0, 1 <= N <= 1024, near and far finite with near < far; refused before any launch.  A row at or behind
+ * the device-side row count (b2n_set_active_rows) counts as inactive and is not written.  One kernel each way, one warp
+ * per ray, fp32, no atomics, no host synchronisation (capturable in a CUDA graph), deterministic.  Reads 4 bytes of z and
+ * of sigma per sample (twice in the backward), writes 4 bytes per ray (forward) or per active sample (backward). */
+int b2n_distortion_fwd(const float* sigma, const float* z, const float* rays_d, const uint32_t* mask_words,
+                       const int32_t* ray_offset, int64_t B, int N, float near, float far, float* loss,
+                       b2n_stream_t stream);
+int b2n_distortion_bwd(const float* sigma, const float* z, const float* rays_d, const uint32_t* mask_words,
+                       const int32_t* ray_offset, int64_t B, int N, float near, float far, const float* g_loss,
+                       float* g_sigma, b2n_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -14,7 +14,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(os.path.dirname(_HERE), "lib", "libb2nerf.so")
 
-ABI_VERSION = 20
+ABI_VERSION = 21
 
 P, L, I, F = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int, ctypes.c_float
 
@@ -83,6 +83,8 @@ SIGNATURES = {
     "b2n_errormap_apply": [P, P, P, I, I, I, F, P],
     "b2n_errormap_cdf": [P, I, I, I, P, P, P],
     "b2n_errormap_sample": [P, P, P, L, I, I, I, I, I, F, P, P, P, P, P],
+    "b2n_distortion_fwd": [P, P, P, P, P, L, I, F, F, P, P],
+    "b2n_distortion_bwd": [P, P, P, P, P, L, I, F, F, P, P, P],
 }
 # development / measurement entry points (include/b2nerf_debug.h): bound like the rest, never called by a product path
 DEBUG_SIGNATURES = {

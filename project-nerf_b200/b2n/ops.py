@@ -419,6 +419,65 @@ def composite(rgb, sigma, z, rays_d, bg=None, dx=None, mask_words=None, ray_offs
     return color, depth, acc, (mdx if dx is not None else None)
 
 
+class _Distortion(torch.autograd.Function):
+    @staticmethod
+    @custom_fwd(device_type="cuda", cast_inputs=torch.float32)
+    def forward(ctx, sigma, z, rays_d, near, far, mask_words, ray_offset):
+        require_cuda(sigma, z, rays_d, mask_words, ray_offset)
+        ctx.rows = current_rows()
+        sigma, z, rays_d = _c(sigma), _c(z), _c(rays_d)
+        B, N = z.shape
+        loss = torch.empty(B, device=z.device)
+        call("b2n_distortion_fwd", ptr(sigma), ptr(z), ptr(rays_d), ptr(mask_words), ptr(ray_offset), B, N, near, far,
+             ptr(loss), stream(), work=(sigma.numel() * 4.0 + B * (4.0 * N + 20.0), 0.0))
+        ctx.save_for_backward(sigma, z, rays_d, mask_words, ray_offset)
+        ctx.near, ctx.far = near, far
+        return loss
+
+    @staticmethod
+    @custom_bwd(device_type="cuda")
+    @with_ctx_rows
+    def backward(ctx, g_loss):
+        sigma, z, rays_d, mask_words, ray_offset = ctx.saved_tensors
+        B, N = z.shape
+        g_sigma = _narrow_out(*sigma.shape, device=sigma.device)
+        call("b2n_distortion_bwd", ptr(sigma), ptr(z), ptr(rays_d), ptr(mask_words), ptr(ray_offset), B, N, ctx.near,
+             ctx.far, ptr(_c(g_loss)), ptr(g_sigma), stream(), work=(sigma.numel() * 8.0 + B * (4.0 * N + 20.0), 0.0))
+        return g_sigma, None, None, None, None, None, None
+
+
+def distortion(sigma, z, rays_d, near, far, mask_words=None, ray_offset=None):
+    """Distortion loss of mip-NeRF 360 per ray (b2n_distortion_fwd / _bwd; contract in include/b2nerf.h, DESIGN.md §5j).
+    sigma [P] (or [P,1]) in the layout of ``composite``: dense (P = B*N) or compact (mask_words [B, ceil(N/32)] and
+    ray_offset [B+1] of ``b2n.march.march``); z [B,N] non-decreasing depths in [near, far]; rays_d [B,3].  Returns
+    loss [B].  Differentiable w.r.t. sigma only; given the same sigma as ``composite``, autograd sums the two gradients."""
+    near, far = float(near), float(far)
+    if not (math.isfinite(near) and math.isfinite(far) and near < far):
+        raise ValueError(f"distortion: near and far must be finite with near < far, got {near}, {far}")
+    if not isinstance(z, torch.Tensor) or z.dim() != 2:
+        raise ValueError(f"distortion: z must be [B,N], got {getattr(z, 'shape', z)}")
+    B, N = z.shape
+    if not 1 <= N <= 1024:
+        raise ValueError(f"distortion: need 1 <= N <= 1024 samples per ray, got {N}")
+    if rays_d.shape != (B, 3):
+        raise ValueError(f"distortion: rays_d must be [B,3] = {(B, 3)}, got {tuple(rays_d.shape)}")
+    sigma = sigma.reshape(-1)
+    if (mask_words is None) != (ray_offset is None):
+        raise ValueError("distortion: the compact layout needs both mask_words and ray_offset")
+    if mask_words is None:
+        if sigma.numel() != B * N:
+            raise ValueError(f"distortion: dense sigma must have B*N = {B * N} entries, got {sigma.numel()}")
+    else:
+        W = (N + 31) // 32
+        if mask_words.dtype != torch.int32 or ray_offset.dtype != torch.int32:
+            raise ValueError("distortion: mask_words and ray_offset must be int32")
+        if mask_words.shape != (B, W) or ray_offset.shape != (B + 1,):
+            raise ValueError(f"distortion: need mask_words [B, {W}] and ray_offset [B+1], got "
+                             f"{tuple(mask_words.shape)} and {tuple(ray_offset.shape)}")
+        mask_words, ray_offset = mask_words.contiguous(), ray_offset.contiguous()
+    return _Distortion.apply(sigma, z, rays_d, near, far, mask_words, ray_offset)
+
+
 # ----------------------------------------------------------------------------
 # fused 64-wide Instant decoder (bf16 tensor cores)
 # ----------------------------------------------------------------------------

@@ -9,6 +9,9 @@ density_grid=grid)`` up to the order of the transmittance product; with ``t_min 
 ``t_min`` of that, depth within ``t_min * far``.  Each wave hands the next K active samples of every ray still alive to
 the model in one call, so a wave's buffers stay near ``WAVE_POINTS`` samples whatever the image size.  Every wave reads
 two 4-byte counts on the host, so a render cannot be captured into a CUDA graph.
+
+``render_rays_train`` is the training render itself (march -> model -> composite), the body that
+``src/renderer.py::render_rays`` and ``b2n.render_rays_distortion`` share.
 """
 from __future__ import annotations
 
@@ -18,8 +21,8 @@ import numpy as np
 import torch
 
 from . import march as _march
-from ._lib import call, lib, ptr, require_cuda, stream
-from .ops import check_errors
+from ._lib import active_rows, call, lib, ptr, require_cuda, stream
+from .ops import check_errors, composite, distortion
 
 MAX_SAMPLES = 1024
 WAVE_POINTS = 2 ** 21          # samples per model call, at most: the fastest in `tools/kbench.py render` (DESIGN.md §5g)
@@ -53,6 +56,56 @@ def _check_rays(rays_o, rays_d, n_samples, t_min):
     if not (0.0 <= t_min < 1.0):                   # NaN fails too
         raise ValueError(f"t_min must be finite with 0 <= t_min < 1, got {t_min}")
     return int(n_samples), t_min
+
+
+def render_rays_train(model, rays_o, rays_d, near, far, n_samples, perturb, density_grid=None, times=None,
+                      white_bkgd=True, bg_color=None, _jitter=None, with_distortion=False):
+    """The body of the training render (src/renderer.py::render_rays, and b2n.render_rays_distortion with
+    ``with_distortion``): march -> model -> composite, plus the per-ray distortion of the same samples when asked.
+    Returns (color, depth, acc, extras, dist): ``extras`` is the dict render_rays returns for a dynamic model given
+    ``times`` (else None), ``dist`` [B] the distortion (else None)."""
+    device = rays_o.device
+    n_rays = rays_o.shape[0]
+    mode = getattr(model, "mode", "unknown")
+    dynamic = mode in ("part3", "part4")
+    if bg_color is None:
+        bg_color = torch.ones(3, device=device) if white_bkgd else torch.zeros(3, device=device)
+    ray_times = None
+    if dynamic:
+        ray_times = times if times is not None else torch.zeros((n_rays, 1), device=device)
+        if ray_times.shape != (n_rays, 1):
+            raise ValueError("times must have shape [n_rays, 1]")
+    u = None
+    if perturb:
+        u = _jitter if _jitter is not None else torch.rand((n_rays, n_samples), device=device)
+
+    if density_grid is not None:
+        m = _march.march(rays_o, rays_d, near, far, n_samples, u, bits=density_grid.bits(),
+                         R=density_grid.resolution, bound=density_grid.bound, times=ray_times)
+    else:
+        m = _march.march(rays_o, rays_d, near, far, n_samples, u, times=ray_times)
+
+    # static mode (b2n.march.set_static_capacity): the number of valid rows of the compact buffers lives on the device
+    dist = None
+    with active_rows(m.n_dev):
+        if dynamic:
+            rgb, sigma, delta_x = model(m.pts, m.dirs, t=m.times)
+        else:
+            rgb, sigma = model(m.pts, m.dirs)
+            delta_x = None
+        want_dx = times is not None and dynamic and delta_x is not None
+        sigma = sigma.float()
+        color, depth, acc, mean_dx = composite(rgb.float(), sigma, m.z, rays_d, bg=bg_color,
+                                               dx=delta_x.float() if want_dx else None,
+                                               mask_words=m.mask_words, ray_offset=m.ray_offset)
+        if with_distortion:
+            dist = distortion(sigma, m.z, rays_d, near, far, mask_words=m.mask_words, ray_offset=m.ray_offset)
+    if times is None:
+        return color, depth, acc, None, dist
+    extras = {}
+    if want_dx:
+        extras["mean_delta_x"] = mean_dx
+    return color, depth, acc, extras, dist
 
 
 @torch.no_grad()

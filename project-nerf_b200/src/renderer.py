@@ -14,7 +14,7 @@ from torch import nn
 
 import b2n
 from b2n import march as _march
-from b2n._lib import active_rows, call, ptr, require_cuda, stream
+from b2n._lib import call, ptr, require_cuda, stream
 
 
 class DensityGrid(nn.Module):
@@ -159,43 +159,11 @@ def render_rays(model, rays_o, rays_d, near, far, n_samples, perturb, density_gr
                 white_bkgd=True, bg_color=None, _jitter=None):
     """``_jitter`` (private, tests only): a [n_rays, n_samples] U[0,1) tensor to use instead of drawing
     ``torch.rand`` -- lets parity tests feed the very jitter the CPU reference drew."""
-    device = rays_o.device
-    n_rays = rays_o.shape[0]
-    mode = getattr(model, "mode", "unknown")
-    dynamic = mode in ("part3", "part4")
-    if bg_color is None:
-        bg_color = torch.ones(3, device=device) if white_bkgd else torch.zeros(3, device=device)
-    ray_times = None
-    if dynamic:
-        ray_times = times if times is not None else torch.zeros((n_rays, 1), device=device)
-        if ray_times.shape != (n_rays, 1):
-            raise ValueError("times must have shape [n_rays, 1]")
-    u = None
-    if perturb:
-        u = _jitter if _jitter is not None else torch.rand((n_rays, n_samples), device=device)
-
-    if density_grid is not None:
-        m = _march.march(rays_o, rays_d, near, far, n_samples, u, bits=density_grid.bits(),
-                         R=density_grid.resolution, bound=density_grid.bound, times=ray_times)
-    else:
-        m = _march.march(rays_o, rays_d, near, far, n_samples, u, times=ray_times)
-
-    # static mode (b2n.march.set_static_capacity): the number of valid rows of the compact buffers lives on the device
-    with active_rows(m.n_dev):
-        if dynamic:
-            rgb, sigma, delta_x = model(m.pts, m.dirs, t=m.times)
-        else:
-            rgb, sigma = model(m.pts, m.dirs)
-            delta_x = None
-        want_dx = times is not None and dynamic and delta_x is not None
-        color, depth, acc, mean_dx = b2n.composite(rgb.float(), sigma.float(), m.z, rays_d, bg=bg_color,
-                                                   dx=delta_x.float() if want_dx else None,
-                                                   mask_words=m.mask_words, ray_offset=m.ray_offset)
+    color, depth, acc, extras, _ = b2n.render.render_rays_train(
+        model, rays_o, rays_d, near, far, n_samples, perturb, density_grid=density_grid, times=times,
+        white_bkgd=white_bkgd, bg_color=bg_color, _jitter=_jitter)
     if times is None:
         return color, depth, acc
-    extras = {}
-    if want_dx:
-        extras["mean_delta_x"] = mean_dx
     return color, depth, acc, extras
 
 
