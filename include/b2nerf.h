@@ -107,6 +107,16 @@ int b2n_march_compact(const float* rays_o, const float* rays_d, const float* tim
                       const uint32_t* mask_words, const int32_t* ray_offset, int64_t B, int N,
                       int32_t* sample_idx, float* pts, float* dirs, float* t_out, b2n_stream_t stream);
 
+/* Backward of the points of b2n_march_compact (pose refinement, DESIGN.md §5k): with pts = o + d*z,
+ *   g_rays_o[r] = sum_s g_pts[j(r,s)],  g_rays_d[r] = sum_s z[r,s] * g_pts[j(r,s)]
+ * over the ray's active samples s, where j(r,s) is the row b2n_march_compact wrote (r*N + s when mask_words == NULL;
+ * ray_offset[r] + the popcount of the ray's mask bits below s otherwise).  Both outputs [B,3] are overwritten.  Rows are
+ * reached only through ray_offset, so in the static-capacity layout rows at or behind the device-side count are never
+ * read.  One warp per ray, fp32 per-lane sums in sample order and a fixed butterfly: no atomics, deterministic, no host
+ * synchronisation.  Reads 12 bytes of g_pts and 4 of z per active sample.  Limits as b2n_march_compact. */
+int b2n_march_points_bwd(const float* z, const uint32_t* mask_words, const int32_t* ray_offset, const float* g_pts,
+                         int64_t B, int N, float* g_rays_o, float* g_rays_d, b2n_stream_t stream);
+
 /* ------------------------------------------------------------------------
  * Alpha compositing (volume_render, src/renderer.py:204-237; mean_delta_x,
  * src/renderer.py:363-380)
@@ -384,6 +394,23 @@ int b2n_sample_rays(const float* poses, const uint8_t* images_rgba8, const float
                     const int64_t* pix_y, const int64_t* pix_x, int64_t B, int V, int H, int W, float focal,
                     float scene_scale, float* rays_o, float* rays_d, float* target_rgba, float* t_out,
                     b2n_stream_t stream);
+
+/* Backward of b2n_sample_rays to the poses (pose refinement, b2n.PoseRefinement; DESIGN.md §5k).  Same poses / picks /
+ * H / W / focal / scene_scale as the forward, plus g_rays_o and g_rays_d [B,3] (the gradients w.r.t. its outputs).
+ * Per ray i of view v = img_idx[i], with the forward's camera direction c = ((x - W/2)/f, -(y - H/2)/f, -1),
+ * d = R_v c, n = |d|, dh = d / n:
+ *   g_R_v += ((g_dh - dh (dh . g_dh)) / n) (x) c,   g_t_v += scene_scale * g_o.
+ * g_poses [V,4,4] is overwritten: [:3,:3] = g_R, [:3,3] = g_t, bottom row 0, all zeros for a view without rays.
+ * The sum is deterministic without float atomics: a stable radix sort of (view, ray index) on ceil(log2(V+1)) bits,
+ * then one block per view sums its rays in sorted order in fp64 and combines its warps in a fixed order.  Two runs on
+ * the same picks give the same bits; reordered picks change only the order of the fp64 sum.  A view id outside [0, V)
+ * is sorted behind every view and never summed, so nothing is written outside g_poses.  No host synchronisation
+ * (capturable).  scratch: b2n_sample_rays_bwd_scratch(B, V) bytes (0 for a refused shape).  Limits: 0 <= B < 2^31,
+ * V, H, W >= 1, focal > 0; refused before any launch. */
+size_t b2n_sample_rays_bwd_scratch(int64_t B, int V);
+int b2n_sample_rays_bwd(const float* poses, const int64_t* img_idx, const int64_t* pix_y, const int64_t* pix_x,
+                        int64_t B, int V, int H, int W, float focal, float scene_scale, const float* g_rays_o,
+                        const float* g_rays_d, float* g_poses, void* scratch, b2n_stream_t stream);
 
 /* ------------------------------------------------------------------------
  * Per-step parameter update (SURVEY 8f-2): what run.py:611-630, :1112-1120 + :1167-1178, :1840-1859 + :1940-1949 do with

@@ -30,6 +30,7 @@ SIGNATURES = {
     "b2n_march_scan_scratch": [L],
     "b2n_march_scan": [P, P, I, L, P, P, P, P],
     "b2n_march_compact": [P, P, P, P, P, P, L, I, P, P, P, P, P],
+    "b2n_march_points_bwd": [P, P, P, P, L, I, P, P, P],
     "b2n_composite_fwd": [P, P, P, P, P, P, I, P, P, L, I, P, P, P, P, P],
     "b2n_composite_bwd": [P, P, P, P, P, P, I, P, P, L, I, P, P, P, P, P, P, P, P],
     "b2n_pe_fwd": [P, L, I, P, I, P, I, I, P],
@@ -66,6 +67,8 @@ SIGNATURES = {
     "b2n_opt_prepare": [P, I, P, P, P],
     "b2n_opt_adamw": [P, I, P, I, P, P, P, P, P],
     "b2n_sample_rays": [P, P, P, P, P, P, L, I, I, I, F, F, P, P, P, P, P],
+    "b2n_sample_rays_bwd_scratch": [L, I],
+    "b2n_sample_rays_bwd": [P, P, P, P, L, I, I, I, F, F, P, P, P, P, P],
     "b2n_nerf_mlp_packed_bwd_bytes": [],
     "b2n_nerf_mlp_pack_bwd": [P, P, P, I, I, P, P],
     "b2n_nerf_mlp_bwd": [P, P, P, P, P, P, P, P, L, P, P, P, P],
@@ -101,7 +104,7 @@ DEBUG_SIGNATURES = {
 }
 _RESTYPES = {"b2n_last_error": ctypes.c_char_p, "b2n_march_scan_scratch": ctypes.c_size_t, "b2n_hash_order_scratch": ctypes.c_size_t,
              "b2n_mesh_scratch": ctypes.c_size_t, "b2n_render_scratch": ctypes.c_size_t,
-             "b2n_errormap_scratch": ctypes.c_size_t,
+             "b2n_errormap_scratch": ctypes.c_size_t, "b2n_sample_rays_bwd_scratch": ctypes.c_size_t,
              "b2n_nerf_mlp_packed_bytes": ctypes.c_size_t, "b2n_nerf_mlp_packed_bwd_bytes": ctypes.c_size_t}
 
 
@@ -133,6 +136,9 @@ lib = _load()
 # number of kernels that entry point launches.
 LAUNCHES = {"count": 0}
 _KERNELS_PER_CALL = {"b2n_march_scan": 3, "b2n_hash_order": 5, "b2n_mesh_count": 2, "b2n_mesh_emit": 2, "b2n_render_begin": 3, "b2n_render_emit": 3, "b2n_render_composite": 3, "b2n_errormap_cdf": 3, "b2n_linear_wgrad": 2, "b2n_instant_mlp_bwd_tc": 2, "b2n_fmlp_bwd": 2}   # 16-bit MLP backwards: |g|-max pre-pass + kernel
+# an estimate: its 3 own kernels plus the CUB radix sort, which is 2 kernels (histogram + one onesweep pass) for up to
+# 255 views, 1 when the batch fits a single tile, and one more onesweep pass per further 8 bits of view id
+_KERNELS_PER_CALL["b2n_sample_rays_bwd"] = 5
 
 
 def ptr(t):

@@ -88,7 +88,11 @@ def march(rays_o: torch.Tensor, rays_d: torch.Tensor, near: float, far: float, n
 
     With ``bits`` the number of active samples is data dependent, so exactly one
     4-byte device->host read sizes the compact buffers (the reference syncs three
-    times per call: renderer.py:309,316,332)."""
+    times per call: renderer.py:309,316,332).
+
+    When ``rays_o`` or ``rays_d`` requires grad (and grad mode is on), ``pts`` is differentiable w.r.t. both
+    (b2n_march_points_bwd; pose refinement, DESIGN.md §5k) with the same values.  ``dirs``, ``times``, ``z`` and the
+    mask never carry a gradient."""
     require_cuda(rays_o, rays_d, u, bits, times)
     rays_o, rays_d = rays_o.float().contiguous(), rays_d.float().contiguous()
     B, N = rays_o.shape[0], int(n_samples)
@@ -130,13 +134,46 @@ def march(rays_o: torch.Tensor, rays_d: torch.Tensor, near: float, far: float, n
             m.n_active, m.n_dev = B * N, total     # fixed capacity, count stays on the device
         else:
             m.n_active = int(total.item())        # the one host sync of the masked path
-    Pn = m.n_active
-    m.pts = torch.empty(Pn, 3, device=dev)
+    if torch.is_grad_enabled() and (rays_o.requires_grad or rays_d.requires_grad):
+        m.pts = _Points.apply(rays_o, rays_d, times, m, want_idx)
+    else:
+        m.pts = _compact(rays_o, rays_d, times, m, want_idx)
+    return m
+
+
+def _compact(rays_o, rays_d, times, m, want_idx):
+    """b2n_march_compact: fills m.dirs, m.times, m.sample_idx (if asked) and returns the points"""
+    Pn, B, N, dev = m.n_active, m.B, m.N, rays_o.device
+    W = (N + 31) // 32
+    pts = torch.empty(Pn, 3, device=dev)
     m.dirs = torch.empty(Pn, 3, device=dev)
     m.times = torch.empty(Pn, 1, device=dev) if times is not None else None
     if want_idx:
         m.sample_idx = torch.empty(Pn, device=dev, dtype=torch.int32)
     call("b2n_march_compact", ptr(rays_o), ptr(rays_d), ptr(times), ptr(m.z), ptr(m.mask_words), ptr(m.ray_offset),
-         B, N, ptr(m.sample_idx), ptr(m.pts), ptr(m.dirs), ptr(m.times), stream(),
+         B, N, ptr(m.sample_idx), ptr(pts), ptr(m.dirs), ptr(m.times), stream(),
          work=(Pn * (4.0 + 24.0 + (4.0 if times is not None else 0.0)) + B * (24.0 + 4.0 * W + 4.0), 0.0))
-    return m
+    return pts
+
+
+class _Points(torch.autograd.Function):
+    """The points o + d * z of ``march`` as a function of the rays (pose refinement, DESIGN.md §5k): the forward is the
+    same b2n_march_compact call, the backward b2n_march_points_bwd.  dirs, times, z and the mask stay constants."""
+
+    @staticmethod
+    def forward(ctx, rays_o, rays_d, times, m, want_idx):
+        pts = _compact(rays_o, rays_d, times, m, want_idx)
+        ctx.save_for_backward(m.z, m.mask_words, m.ray_offset)
+        ctx.n_active = m.n_active
+        return pts
+
+    @staticmethod
+    def backward(ctx, g_pts):
+        z, words, offs = ctx.saved_tensors
+        B, N = z.shape
+        g_pts = g_pts.float().contiguous()
+        g_o = torch.empty(B, 3, device=g_pts.device)
+        g_d = torch.empty(B, 3, device=g_pts.device)
+        call("b2n_march_points_bwd", ptr(z), ptr(words), ptr(offs), ptr(g_pts), B, N, ptr(g_o), ptr(g_d), stream(),
+             work=(ctx.n_active * 12.0 + B * (4.0 * N + 4.0 * ((N + 31) // 32) + 28.0), 0.0))
+        return g_o, g_d, None, None, None

@@ -273,6 +273,51 @@ k_march_compact(const float* __restrict__ rays_o, const float* __restrict__ rays
   }
 }
 
+// Backward of the points of k_march_compact, pts = o + d * z: g_o = sum_s g_pts, g_d = sum_s z_s g_pts over the ray's
+// active samples.  One warp per ray, rows found as in k_march_compact (so rows behind a device-side count are never
+// reached); each lane sums its own samples in order, then a fixed xor-butterfly: deterministic without atomics.
+__global__ void __launch_bounds__(256)
+k_march_points_bwd(const float* __restrict__ z, const uint32_t* __restrict__ mask_words,
+                   const int32_t* __restrict__ ray_offset, const float* __restrict__ g_pts, int64_t B, int N,
+                   float* __restrict__ g_o, float* __restrict__ g_d) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+  const int W = (N + 31) >> 5;
+  for (int64_t r = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); r < B; r += warps) {
+    float so[3] = {0.f, 0.f, 0.f}, sd[3] = {0.f, 0.f, 0.f};
+    int64_t out = mask_words ? (int64_t)ray_offset[r] : r * N;
+    for (int k = 0; k < W; ++k) {
+      uint32_t w;
+      if (mask_words) {
+        w = mask_words[r * W + k];
+      } else {
+        const int rem = N - (k << 5);
+        w = rem >= 32 ? 0xffffffffu : ((1u << rem) - 1u);
+      }
+      if ((w >> lane) & 1u) {
+        const int64_t j = out + __popc(w & ((1u << lane) - 1u));
+        const float zz = __ldg(z + r * N + (k << 5) + lane);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const float g = __ldcs(g_pts + 3 * j + c);
+          so[c] += g;
+          sd[c] = fmaf(zz, g, sd[c]);
+        }
+      }
+      out += __popc(w);
+    }
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      so[c] = warp_sum(so[c]);
+      sd[c] = warp_sum(sd[c]);
+    }
+    if (lane < 3) {
+      g_o[3 * r + lane] = lane == 0 ? so[0] : (lane == 1 ? so[1] : so[2]);
+      g_d[3 * r + lane] = lane == 0 ? sd[0] : (lane == 1 ? sd[1] : sd[2]);
+    }
+  }
+}
+
 }  // namespace b2n
 
 using namespace b2n;
@@ -365,4 +410,17 @@ extern "C" int b2n_march_compact(const float* rays_o, const float* rays_d, const
   k_march_compact<<<ray_grid(B), 256, 0, (cudaStream_t)stream>>>(rays_o, rays_d, times, z, mask_words, ray_offset, B,
                                                                 N, sample_idx, pts, dirs, t_out);
   return check_launch("b2n_march_compact");
+}
+
+extern "C" int b2n_march_points_bwd(const float* z, const uint32_t* mask_words, const int32_t* ray_offset,
+                                    const float* g_pts, int64_t B, int N, float* g_rays_o, float* g_rays_d,
+                                    b2n_stream_t stream) {
+  B2N_REQUIRE(B >= 0 && N > 0 && N <= 4096, "bad B or N");
+  if (B == 0) return B2N_OK;
+  B2N_REQUIRE(z && g_pts && g_rays_o && g_rays_d, "null pointer");
+  B2N_REQUIRE(!mask_words || ray_offset, "compact mode needs ray_offset");
+  B2N_REQUIRE(B * (int64_t)N < (int64_t)1 << 31, "B*N must fit int32");
+  k_march_points_bwd<<<ray_grid(B), 256, 0, (cudaStream_t)stream>>>(z, mask_words, ray_offset, g_pts, B, N, g_rays_o,
+                                                                   g_rays_d);
+  return check_launch("b2n_march_points_bwd");
 }
