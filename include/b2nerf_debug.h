@@ -40,6 +40,11 @@ int b2n_debug_instant_bwd_groups(int groups);
 int b2n_debug_hash_variant(int variant, int merge_res);
 /* the current variant and merge threshold (host ints), so that a caller can restore what it found */
 int b2n_debug_hash_config(int* variant, int* merge_res);
+/* table gradient of the spatially ordered F = 2 hash grid (b2n_hash_bwd_ordered): dedup_res > 0 takes the corners by
+ * vertex parity and reduces equal table entries across the warp before the reductions on the levels with res <= dedup_res
+ * (default 122); 0 = run merging up to merge_res, as in ray order.  Same table gradient up to the order of the fp32 sums.
+ * dedup_res < 0 changes nothing.  Returns the previous value. */
+int b2n_debug_hash_dedup(int dedup_res);
 
 /* random 8-byte gathers over a float2[n_entries] table (n_entries = 2^k): the L2 gather peak the hash-grid kernels are
  * compared against (tools/kbench.py l2, bench.py hash_vs_l2) */

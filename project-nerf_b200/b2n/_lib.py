@@ -96,6 +96,7 @@ DEBUG_SIGNATURES = {
     "b2n_debug_mlp256_set_pair": [ctypes.c_int],
     "b2n_debug_hash_variant": [I, I],
     "b2n_debug_hash_config": [P, P],
+    "b2n_debug_hash_dedup": [I],
     "b2n_debug_instant_bwd_groups": [I],
     "b2n_debug_instant_fwd_slots": [I],
     "b2n_debug_gather_bench": [P, L, I, I, P, P],
@@ -218,6 +219,23 @@ class hash_variant:
 
     def __exit__(self, *exc):
         _raise_on("b2n_debug_hash_variant", lib.b2n_debug_hash_variant(*self.prev))
+        return False
+
+
+class hash_dedup:
+    """``with hash_dedup(dedup_res):`` -- the table gradient of the spatially ordered F = 2 hash grid merges equal table
+    entries of a warp on the levels with res <= dedup_res (0: the run merging of ray order) (b2n_debug_hash_dedup); the
+    value found on entry is restored on exit."""
+
+    def __init__(self, dedup_res):
+        self.res = dedup_res
+
+    def __enter__(self):
+        self.prev = lib.b2n_debug_hash_dedup(self.res)
+        return self
+
+    def __exit__(self, *exc):
+        lib.b2n_debug_hash_dedup(self.prev)
         return False
 
 

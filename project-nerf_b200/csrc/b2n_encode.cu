@@ -303,6 +303,24 @@ k_hash_bwd_table_dense(const float* __restrict__ x, int64_t P, float bound, floa
 // warp holds fall into a handful of cells that share their lines.  Level geometry comes from the constant bank.
 __device__ __forceinline__ float pair_sum(float v) { return v + __shfl_xor_sync(0xffffffffu, v, 1); }
 
+// Sum of (v0, v1) over the lanes of `peers` (the lanes of this one that hold the same key, __match_any_sync) in log2(|peers|)
+// rounds of a tree over the ranks inside the group; the lowest lane of the group ends with the sum and gets true.  All 32
+// lanes must call it.  (The warp-aggregation of E. Westphal, "Voting and Shuffling to Optimize Atomic Operations", 2015.)
+__device__ __forceinline__ bool reduce_peers(uint32_t peers, float& v0, float& v1) {
+  const int lane = threadIdx.x & 31;
+  uint32_t rank = __popc(peers & ((1u << lane) - 1u));
+  uint32_t above = peers & (0xfffffffeu << lane);              // the group's lanes above this one not yet summed
+  const bool leader = rank == 0;
+  while (__any_sync(0xffffffffu, above != 0u)) {
+    const int next = __ffs(above);                              // nearest lane above still holding a partial sum (1-based)
+    const float t0 = __shfl_sync(0xffffffffu, v0, next - 1), t1 = __shfl_sync(0xffffffffu, v1, next - 1);
+    if (next) v0 += t0, v1 += t1;
+    above &= __ballot_sync(0xffffffffu, !(rank & 1u));          // odd ranks have handed their partial sum down
+    rank >>= 1;
+  }
+  return leader;
+}
+
 // Spatial order (b2n_hash_order): in ray order the 16 points of a warp are 16 samples of one ray and share cells only at
 // the coarsest levels; in Morton order they share cells and table lines up to the middle levels.  The key is the Morton
 // code of the point's cell on a 2^7 lattice over the box; within a bucket points keep the order in which the counting
@@ -495,13 +513,18 @@ k_hash_fwd_pair(const float* __restrict__ x, int64_t P, float bound, float two_b
   }
 }
 
-// Table gradient with the same lane mapping.  A level whose resolution is <= merge_res is reduced across the run of
-// consecutive points (consecutive samples of a ray) that share a cell before the run head issues the red.global -- the
-// coarse levels would otherwise serialise millions of reductions on a few thousand addresses.
+// Table gradient with the same lane mapping.  Ray order (dedup_res == 0): a level whose resolution is <= merge_res is
+// reduced across the run of consecutive points (consecutive samples of a ray) that share a cell before the run head issues
+// the red.global -- the coarse levels would otherwise serialise millions of reductions on a few thousand addresses.
+// Spatial order (dedup_res > 0): the points of a warp are neighbours and reach the same vertices from different cells.  On a
+// level whose resolution is <= dedup_res, instruction slot k takes the corner whose vertex has (y, z) parity k, so every
+// occurrence of a vertex in the warp falls into the same slot; each slot is reduced over the lanes that hold the same
+// entry and one of them issues the red.global.  The finer levels scatter plainly: there the match, the reduction rounds
+// and the per-slot weights cost more issue slots than the fewer reductions save (DESIGN.md section 7b).
 __global__ void __launch_bounds__(256)
 k_hash_bwd_table_pair(const float* __restrict__ x, int64_t P, float bound, float two_bound, const Levels lv, int lbeg,
                       int nl, const float* __restrict__ g, int ld, int col0, float2* __restrict__ g_table,
-                      uint32_t merge_res, const int* __restrict__ order, const int* __restrict__ rows) {
+                      uint32_t merge_res, uint32_t dedup_res, const int* __restrict__ order, const int* __restrict__ rows) {
   P = clamp_rows(P, rows);
   // levels [lbeg, nl) of the table (lbeg a multiple of 4): a caller that overlaps the gradient all-reduce of the fine
   // levels with the scatter of the coarse ones launches this kernel once per level window.  order != NULL: x is in
@@ -541,7 +564,22 @@ k_hash_bwd_table_pair(const float* __restrict__ x, int64_t P, float bound, float
       const uint32_t cx = c.g[0] + (uint32_t)s;
       const float wx = s ? c.w[0] : 1.f - c.w[0];
       const float g0 = gv[2 * j], g1 = gv[2 * j + 1];
-      if (L.res > merge_res) {
+      if (L.res <= dedup_res) {
+        // samples that received no gradient (and lanes behind the row count) leave the match with a key no entry has
+        const bool act = live && (g0 != 0.f || g1 != 0.f);
+        const uint32_t py = c.g[1] & 1u, pz = c.g[2] & 1u;
+#pragma unroll 1
+        for (int k = 0; k < 4; ++k) {
+          const uint32_t dy = (k & 1) ^ py, dz = (k >> 1) ^ pz;
+          const float w = wx * (dy ? c.w[1] : 1.f - c.w[1]) * (dz ? c.w[2] : 1.f - c.w[2]);
+          const uint32_t e = corner_entry(L, cx, c.g[1] + dy, c.g[2] + dz);
+          float v0 = w * g0, v1 = w * g1;
+          if (reduce_peers(__match_any_sync(0xffffffffu, act ? e : 0xffffffffu), v0, v1) && act)
+            atomicAdd(g_table + e, make_float2(v0, v1));
+        }
+        continue;
+      }
+      if (dedup_res > 0 || L.res > merge_res) {
         if (live && (g0 != 0.f || g1 != 0.f)) {        // samples that received no gradient scatter nothing
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
@@ -801,9 +839,12 @@ k_hash_tri_bwd(const float* __restrict__ x, const float* __restrict__ tval, int6
 }
 
 // A/B switch of the F == 2 kernels (b2nerf_debug.h: b2n_debug_hash_variant): bit 0 = pair-lane forward, bit 1 = pair-lane
-// table gradient; g_merge_res = coarsest-level run merging threshold of the pair-lane table gradient.
+// table gradient; g_merge_res = coarsest-level run merging threshold of the pair-lane table gradient in ray order.
+// g_dedup_res (b2n_debug_hash_dedup): in spatial order the table gradient merges equal entries of a warp on the levels with
+// res <= g_dedup_res; 0 = run merging up to g_merge_res, as in ray order.
 static int g_hash_variant = 3;
 static uint32_t g_merge_res = 128;      // measured on the C2 sample set: 64 -> 7.59 ms, 128 -> 7.49, 200 -> 7.44 (T = 2^20: 128 best)
+static uint32_t g_dedup_res = 122;      // levels 0-5 of the C2 geometry: DESIGN.md section 7b
 
 static int fill_levels(const b2n_hash_level* h, int L, Levels* out) {
   if (!h || L <= 0 || L > B2N_MAX_LEVELS) return -1;
@@ -889,12 +930,15 @@ static int hash_bwd(const float* x, const int* order, int64_t P, float bound, co
               "table / g_table must be 16-byte aligned (vector reductions)");
   B2N_REQUIRE(!order || (!g_x && F == 2 && ((g_hash_variant & 2) || windowed)),
               "an order needs F = 2, the pair-lane table gradient and no input gradient");
+  // the entry merge of the ordered scatter keys idle lanes with 0xffffffff, which no entry of the table may be
+  B2N_REQUIRE(!order || (uint64_t)lv.l[L - 1].offset + lv.l[L - 1].size < 0xffffffffull, "table too large for the entry merge");
   const float tb = 2.0f * bound;
   cudaStream_t st = (cudaStream_t)stream;
   if (g_table && F == 2 && ((g_hash_variant & 2) || windowed)) {
     if (level_begin < level_end)
       k_hash_bwd_table_pair<<<pair_grid(P, order), 256, 0, st>>>(x, P, bound, tb, lv, level_begin, level_end, g_out, ld_g,
-                                                               col0, reinterpret_cast<float2*>(g_table), g_merge_res, order,
+                                                               col0, reinterpret_cast<float2*>(g_table), g_merge_res,
+                                                               order ? g_dedup_res : 0u, order,
                                                                g_active_rows);
   } else if (g_table) {
     int n_dense = 0;                      // leading run of un-hashed levels
@@ -1019,4 +1063,10 @@ extern "C" int b2n_debug_hash_config(int* variant, int* merge_res) {
   *variant = g_hash_variant;
   *merge_res = (int)g_merge_res;
   return B2N_OK;
+}
+
+extern "C" int b2n_debug_hash_dedup(int dedup_res) {
+  const int prev = (int)g_dedup_res;
+  if (dedup_res >= 0) g_dedup_res = (uint32_t)dedup_res;
+  return prev;
 }

@@ -659,61 +659,67 @@ def hash_levels(P=24_000_000):
 
 
 def hash_sorted():
-    """What spatial order buys the shipped pair-lane hash-grid kernels (variant 3) on the C2 sample set (dense occupancy,
-    2^18 rays x 128 samples, L = 16, T = 2^19): ray order against the same points ordered by a Morton key of their cell on
-    a 2^k lattice over the box (torch.argsort, stable, so a cell keeps its points in ray order), and against the k = 10 order
-    with its 128-point blocks interleaved over the curve, with the run-merging threshold merge_res swept.  Per entry: median
-    and best of 10 calls (CUDA events of b2n._lib.Profiler).  Result: profiles/hashsort_b200.txt, DESIGN.md section 7b."""
+    """The spatially ordered hash-grid path of the C2 step (dense occupancy, 2^18 rays x 128 samples, L = 16, F = 2,
+    T = 2^19): hash_encode forward + backward as the C2 step runs it (b2n_hash_order, b2n_hash_fwd_ordered,
+    b2n_hash_bwd_ordered), with the table gradient's warp-level entry merge on the levels with res <= dedup_res
+    (b2n_debug_hash_dedup; 0 = run merging up to res 128), the settings alternated; then the table-gradient scatter
+    alone per 4-level window [lbeg, lbeg + 4) for each setting.  Per entry: median (best) of 10 calls, CUDA events.
+    Result: profiles/hashdedup_b200.txt, DESIGN.md section 7b."""
     from b2n import synthetic, march
-    hash_variant = b2n._lib.hash_variant
+    _device_line()
     torch.manual_seed(0)
     ro, rd, _ = (t.cuda() for t in synthetic.random_rays(2 ** 18, seed=1))
     u = torch.rand(2 ** 18, 128, device="cuda")
     occ = torch.ones(128, 128, 128, dtype=torch.bool, device="cuda")
     x = march.march(ro, rd, 2.0, 6.0, 128, u, bits=march.pack_occupancy(occ), R=128, bound=1.5).pts
-    print("points", x.shape[0], "|", torch.cuda.get_device_name())
-
-    def spread(v):                                   # 10 bits -> every third bit
-        v = (v | (v << 16)) & 0x030000FF
-        v = (v | (v << 8)) & 0x0300F00F
-        v = (v | (v << 4)) & 0x030C30C3
-        return (v | (v << 2)) & 0x09249249
-
-    def morton(p, k):
-        q = ((p + 1.5) / 3.0 * (1 << k)).clamp(0, (1 << k) - 1).to(torch.int64)
-        return spread(q[:, 0]) | (spread(q[:, 1]) << 1) | (spread(q[:, 2]) << 2)
-
-    def interleave(xs, S=2048):
-        # the sorted set in chunks of 128 points (one block of the pair-lane kernels), chunk i of a group of S at curve
-        # position i * (n_chunks / S): consecutive blocks -- the ones resident at the same time -- sit far apart on the curve
-        nc = xs.shape[0] // 128 // S * S
-        head = xs[: nc * 128].view(S, nc // S, 128, 3).transpose(0, 1).reshape(-1, 3)
-        return torch.cat([head, xs[nc * 128:]]).contiguous()
-
-    sets = [("ray order", x)]
-    for k in (8, 10):
-        t_sort, _ = timeit(lambda: x[torch.argsort(morton(x, k), stable=True)], n=5, warm=2)
-        sets.append((f"morton k={k}", x[torch.argsort(morton(x, k), stable=True)].contiguous()))
-        print(f"morton key (k={k}) + torch.argsort + gather: {t_sort:.3f} ms")
-    sets.append(("morton k=10, blocks interleaved", interleave(sets[-1][1])))
+    P = x.shape[0]
     geom = b2n.HashGeometry(16, 16, 1.5, 19, 2)
+    print("points", P, "| level res:", " ".join(str(lv[1]) for lv in geom.levels))
     table = (torch.randn(geom.n_params, device="cuda") * 0.1).requires_grad_(True)
-    keys = ("b2n_hash_fwd", "b2n_hash_bwd")
-    for name, pts in sets:
-        for merge in (128, 200, 300, 400):
-            with hash_variant(3, merge):
-                y = b2n.hash_encode(pts, table, geom, 1.5)
-                g = torch.randn_like(y)
-                b2n._lib.PROFILER = prof = b2n._lib.Profiler()
-                for _ in range(10):
-                    y = b2n.hash_encode(pts, table, geom, 1.5)
-                    y.backward(g)
+    settings = (0, 54, 81, 122, 183, 274, 616, 1 << 20)
+    keys = ("b2n_hash_order", "b2n_hash_fwd", "b2n_hash_bwd")
+    g = None
+    times = {d: {k: [] for k in keys} for d in settings}
+    for rep in range(10):
+        for d in settings:                                    # alternated: each setting sees the same clocks
+            with _lib.hash_dedup(d):
+                y = b2n.hash_encode(x, table, geom, 1.5)
+                if g is None:
+                    g = torch.randn_like(y)
+                table.grad = None
                 torch.cuda.synchronize()
-                b2n._lib.PROFILER = None
-            ts = {k: sorted(e0.elapsed_time(e1) for n_, _, _, e0, e1 in prof.records if n_ == k) for k in keys}
-            med = {k: v[len(v) // 2] for k, v in ts.items()}
-            print(f"{name:31s} merge_res={merge:3d}: " + ", ".join(f"{k} {med[k]:.3f} (best {ts[k][0]:.3f}) ms" for k in keys)
-                  + f", fwd+bwd {sum(med.values()):.3f} ms")
+                _lib.PROFILER = prof = _lib.Profiler()
+                y = b2n.hash_encode(x, table, geom, 1.5)
+                y.backward(g)
+                torch.cuda.synchronize()
+                _lib.PROFILER = None
+            for n_, _, _, e0, e1 in prof.records:
+                if n_ in times[d]:
+                    times[d][n_].append(e0.elapsed_time(e1))
+    for d in settings:
+        ts = {k: sorted(v) for k, v in times[d].items()}
+        med = {k: v[len(v) // 2] for k, v in ts.items()}
+        print(f"hash_encode fwd+bwd dedup_res={d:7d}: " + ", ".join(f"{k} {med[k]:.3f} ({ts[k][0]:.3f})" for k in keys)
+              + f" ms, sum {sum(med.values()):.3f} ms")
+
+    order = torch.empty(P, dtype=torch.int32, device="cuda")
+    xs = torch.empty_like(x)
+    scratch = torch.empty(_lib.lib.b2n_hash_order_scratch(P) // 4, dtype=torch.int32, device="cuda")
+    _lib.call("b2n_hash_order", _lib.ptr(x), P, 1.5, _lib.ptr(order), _lib.ptr(xs), _lib.ptr(scratch), _lib.stream())
+    G = torch.zeros(geom.n_params, device="cuda")
+    L = geom.n_levels
+    for lbeg in range(0, L, 4):
+        def scatter():
+            _lib.call("b2n_hash_bwd_ordered", _lib.ptr(xs), _lib.ptr(order), P, 1.5, _lib.ptr(table), geom.c_levels, L, 2,
+                      _lib.ptr(g), 2 * L, 0, _lib.ptr(G), lbeg, lbeg + 4, _lib.stream())
+        res = [geom.levels[l][1] for l in range(lbeg, lbeg + 4)]
+        ts = {d: [] for d in settings}
+        for rep in range(10):
+            for d in settings:
+                with _lib.hash_dedup(d):
+                    ts[d].append(timeit(scatter, n=1, warm=1)[0])
+        print(f"scatter levels [{lbeg:2d}, {lbeg + 4:2d}) res {res}: " +
+              ", ".join(f"dedup_res={d} {sorted(v)[len(v) // 2]:.3f} ({min(v):.3f})" for d, v in ts.items()) + " ms")
 
 
 def hash_variants():
